@@ -13,6 +13,9 @@ A *step* is one pass of the hot path over one batch of synthetic QPs:
                         primary line when the batch kernels are not built.
 `value` is whole-job throughput with all inputs resident in HBM (CUDA-event time on the launching stream, max over
 ranks); `e2e` goes through the public C API with host buffers (setup/H2D + solve + D2H inside the timed region).
+`--dump-outputs DIR` writes, after the timed steps, what the last step computed (rank 0's x, y and info fields per QP) as
+DIR/<name>.npy, so that two builds can be compared output for output: the inputs are seeded, the same arguments give the
+same inputs.
 """
 from __future__ import annotations
 
@@ -98,6 +101,31 @@ def get_stats(lib, solver) -> abi.QPALMB200Stats:
     st = abi.QPALMB200Stats()
     lib.qpalm_b200_get_stats(solver._work, C.byref(st))
     return st
+
+
+DUMP_BYTES = 60_000_000     # --dump-outputs: data bytes in all (64 MB less room for the .npy headers)
+
+
+def solve_outputs(prefix, x, y, infos):
+    """What a caller of the timed path receives: x, y and the info fields, one row per QP."""
+    out = {prefix + "x": x, prefix + "y": y}
+    out.update({prefix + k: [i[k] for i in infos] for k in ("status_val", "iter", "iter_out", "objective")})
+    return out
+
+
+def dump_outputs(out_dir, outputs):
+    """Every array of `outputs` as <out_dir>/<name>.npy in float64.  When they come to more than DUMP_BYTES, every array
+    keeps the same fixed, seeded fraction of its rows (axis 0), whose indices go to <name>_rows.npy."""
+    arrays = {k: np.atleast_1d(np.asarray(v, dtype=np.float64)) for k, v in outputs.items()}
+    data = sum(a.nbytes for a in arrays.values())
+    with_rows = data + sum(8 * len(a) for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if data > DUMP_BYTES:
+            rows = np.sort(np.random.default_rng(0).choice(len(a), max(1, len(a) * DUMP_BYTES // with_rows), replace=False))
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -266,7 +294,7 @@ def bench_dense(args, lib, steps, warmup, sample_clocks=True):
                                + (st1.inner_iterations - st0.inner_iterations))) / steps,      # minus update sweeps (2 k n^2) and solves (2 n^2)
         updown_rank_sum=int(st1.updown_rank_sum - st0.updown_rank_sum) // steps,
         sigma_update_calls=int(st1.sigma_update_calls - st0.sigma_update_calls) // steps, alg_bytes=(st1.algorithmic_bytes - st0.algorithmic_bytes) / steps,
-        clocks=clocks, h2d=h2d, d2h=d2h, x=res.x, y=res.y, objective=res.objective)
+        clocks=clocks, h2d=h2d, d2h=d2h, x=res.x, y=res.y, objective=res.objective, status_val=res.status_val)
     s.cleanup()
     # e2e: setup (H2D + Ruiz) + solve + solution read-back through the public API, host buffers (pageable, as the caller's CSC
     # arrays are; pinning the 1.28 GB of matrix values made qpalm_setup slower on the box: 0.63 s against 0.21 s)
@@ -513,7 +541,10 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-dense", action="store_true", help="skip the dense time-to-solution block")
     ap.add_argument("--sweep-total", type=int, default=4096, help="N = 1: also run the whole sweep on the one GPU (0 to skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     rank, world, local = dist_env()
     steps, warmup = max(1, args.steps), max(3, args.warmup) if args.impl == "b200" else max(0, args.warmup)
 
@@ -580,6 +611,7 @@ def main():
             "dtype": "f64", "data": "synthetic"}
     if workload == "mpc_batch":
         r = bench_batch(args, steps, warmup, rank, world)
+        outputs = solve_outputs("", r["x"], r["y"], r["infos"])
         t = torch.tensor([r["dev_ms"], r["e2e_s"]], device="cuda", dtype=torch.float64)
         if world > 1:
             torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
@@ -624,6 +656,7 @@ def main():
             rowshard.init(rank, world, torch.device("cuda", local))
             line["scaling"] = "strong"
         dense, p = bench_dense(args, lib, steps, warmup)
+        outputs = solve_outputs("", dense["x"], dense["y"], [dense])
         t = torch.tensor([dense["ms_per_solve"], dense["e2e_s"]], device="cuda", dtype=torch.float64)
         if world > 1:
             torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
@@ -653,6 +686,7 @@ def main():
     # the dense time-to-solution block rides along on the batch line at N = 1
     if workload == "mpc_batch" and world == 1 and not args.no_dense:
         dense, p = bench_dense(args, lib, 1, 1, sample_clocks=False)
+        outputs.update(solve_outputs("dense_", dense["x"], dense["y"], [dense]))
         line["time_to_solution"] = {"workload": f"dense random convex QP n={args.n} m={args.m} eps 1e-6",
                                     "seconds": dense["ms_per_solve"] * 1e-3, "e2e_seconds": dense["e2e_s"], "setup_seconds": dense["setup_warm_s"], "setup_seconds_first_call": dense["setup_s"],
                                     "status": dense["status"], "iter": dense["iter"], "iter_out": dense["iter_out"],
@@ -694,6 +728,8 @@ def main():
         torch.distributed.barrier()
         torch.distributed.destroy_process_group()
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
 
 
