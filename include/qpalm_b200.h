@@ -356,7 +356,27 @@ int  qpalm_b200_batch_stats(QPALMB200Batch *batch, c_int nb, double *out8);
 /* persistent engine, QPALM_B200_BATCH_PROF=1 at setup: per-instance SM-clock totals of 16 phases of the last solve */
 int  qpalm_b200_batch_phase_profile(QPALMB200Batch *batch, c_int nb, long long *out);
 long long qpalm_b200_batch_last_launches(const QPALMB200Batch *batch);   /* kernels launched by the last solve */
+/* engine and CTA shape of the last solve: 0 lock-step, 3 or 4 persistent (the build with 3 or 4 CTAs per SM) */
+int  qpalm_b200_batch_last_shape(const QPALMB200Batch *batch);
 void qpalm_b200_batch_cleanup(QPALMB200Batch *batch);
+
+/* Test probes of the persistent engine's in-CTA building blocks, run by separate kernels of the same build (shape 3: the
+ * default build, shape 4: the 4-CTAs-per-SM build) with its CTA size, shared-memory plan and persistent work queue.
+ * Newton-step probe, per instance b < nb (matrices n x n column-major, lower triangle used; 1 <= n <= 240):
+ *   H = src + sum_{pos} w^2 a a' - sum_{neg} w^2 a a', src = H0[b] (H0: nb x n x n), or with from_q the one shared matrix
+ *       H0 scaled by sscale (the solver's path without active rows; then npos = nneg = 0 and the factor reads H0 itself)
+ *   L = chol(H + beta I), d_fused = (L L')^{-1} rhs[b] with the forward substitution fused into the factorisation
+ *   then, nup > 0: rank update of L by the rows upd[0 .. nup), the first kpos entering (+), the rest leaving (-), in sweeps of 8
+ *   d_after = (L L')^{-1} rhs[b] with the final L (separate forward and backward substitutions)
+ * a = wts entry * column list entry of At (n x m, shared).  cnt: nb x 4 {npos, nneg, nup, kpos}; lists, wts: nb x 3m, per
+ * instance the pos rows at [0, m), the neg rows at [m, 2m), the update rows at [2m, 3m).  Outputs H_out, L_out (nb x n x n,
+ * lower triangles, zero above), d_fused, d_after (nb x n) and info (bit 0: a sweep lost definiteness, bit 1: the
+ * factorisation met a non-positive pivot).  Returns 0, 1 for invalid arguments, < 0 for a CUDA error. */
+int qpalm_b200_batchp_probe_newton(c_int shape, c_int nb, c_int n, c_int m, const c_float *At, const c_float *H0, c_int from_q,
+        c_float sscale, const c_int *cnt, const c_int *lists, const c_float *wts, c_float beta, const c_float *rhs,
+        c_float *H_out, c_float *L_out, c_float *d_fused, c_float *d_after, c_int *info);
+/* the line search's stable radix sort on nb independent arrays of N <= 2048 (key, val) pairs (nb x N each), in place */
+int qpalm_b200_batchp_probe_sort(c_int shape, c_int nb, c_int N, unsigned long long *keys, unsigned int *vals);
 
 #ifdef __cplusplus
 }

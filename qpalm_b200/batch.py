@@ -26,6 +26,8 @@ def _lib():
         lib.qpalm_b200_batch_download.restype = C.c_int
         lib.qpalm_b200_batch_last_launches.argtypes = [C.c_void_p]
         lib.qpalm_b200_batch_last_launches.restype = C.c_longlong
+        lib.qpalm_b200_batch_last_shape.argtypes = [C.c_void_p]
+        lib.qpalm_b200_batch_last_shape.restype = C.c_int
         lib.qpalm_b200_batch_stats.argtypes = [C.c_void_p, abi.c_int, c_float_p]
         lib.qpalm_b200_batch_stats.restype = C.c_int
         lib.qpalm_b200_batch_cleanup.argtypes = [C.c_void_p]
@@ -107,6 +109,10 @@ class Batch:
 
     def last_launches(self):
         return int(self.lib.qpalm_b200_batch_last_launches(self.h))
+
+    def last_shape(self):
+        """Engine of the last solve: 0 lock-step, 3 or 4 persistent with 3 or 4 CTAs per SM."""
+        return int(self.lib.qpalm_b200_batch_last_shape(self.h))
 
     def cleanup(self):
         if self.h:

@@ -936,10 +936,12 @@ extern "C" int qpalm_b200_batch_solve_resident(QPALMB200Batch *B, c_int nb_, dou
     if (device_ms) *device_ms = msp;
     B->launches_last = g_kernel_launches - launches0;
     B->last_engine = 2;
+    B->last_shape = four ? 4 : 3;
     QB_CUDA_TRY(cudaGetLastError());
     return 0;
   }
   B->last_engine = 1;
+  B->last_shape = 0;
   QB_CUDA_TRY(cudaEventRecord(B->ev0, s));
   QB_LAUNCH(kb_init, nb, 256, 0, s, n, m, st, e->D, e->E, B->q_raw, B->bmin_raw, B->bmax_raw, B->q, B->bmin, B->bmax, B->x, B->y, B->Ax,
             B->Qx, B->Aty, B->x_prev, B->x0, B->sigma, B->sigma_inv, B->sqrt_sigma, B->Qd, B->Ad, B->d, B->pri_res_in, B->active,
@@ -1065,6 +1067,104 @@ extern "C" int qpalm_b200_batch_phase_profile(QPALMB200Batch *B, c_int nb, long 
 }
 
 extern "C" long long qpalm_b200_batch_last_launches(const QPALMB200Batch *B) { return B ? B->launches_last : 0; }
+
+extern "C" int qpalm_b200_batch_last_shape(const QPALMB200Batch *B) { return B ? B->last_shape : 0; }
+
+// ------------------------------------------------------------------------------------------------
+// test probes of the persistent engine's in-CTA building blocks (batchp.cu kbp_probe_*): host buffers in and out, like the
+// operator ABI of Part 2.  shape picks the build: 3 the default one, 4 the -DQB_BP_VARIANT4 one.
+// ------------------------------------------------------------------------------------------------
+namespace {
+struct ProbeBufs {   // device buffers of one probe call, freed on every return path
+  std::vector<void *> p;
+  bool failed = false;
+  template <typename T> T *get(size_t count) {
+    void *q = nullptr;
+    if (dev_alloc(&q, sizeof(T) * (count ? count : 1))) { failed = true; return nullptr; }
+    p.push_back(q);
+    return static_cast<T *>(q);
+  }
+  ~ProbeBufs() { for (void *q : p) cudaFree(q); }
+};
+}  // namespace
+
+extern "C" int qpalm_b200_batchp_probe_newton(c_int shape, c_int nb_, c_int n_, c_int m_, const c_float *At, const c_float *H0, c_int from_q,
+                                              c_float sscale, const c_int *cnt, const c_int *lists, const c_float *wts, c_float beta,
+                                              const c_float *rhs, c_float *H_out, c_float *L_out, c_float *d_fused, c_float *d_after,
+                                              c_int *info) {
+  if ((shape != 3 && shape != 4) || nb_ < 1 || n_ < 1 || m_ < 1) return 1;
+  const int nb = (int)nb_, n = (int)n_, m = (int)m_, ld = round_up(n, kPanel);
+  const size_t NB = nb, N = n, M = m, LL = (size_t)ld * ld;
+  std::vector<int> cnt_i(NB * 4), lists_i(NB * 3 * M, 0);
+  for (size_t b = 0; b < NB; b++) {
+    const c_int *c = cnt + 4 * b;
+    if (c[0] < 0 || c[0] > m || c[1] < 0 || c[1] > m || c[2] < 0 || c[2] > m || c[3] < 0 || c[3] > c[2]) return 1;
+    if (from_q && (c[0] || c[1])) return 1;   // the f.fq path factors the shared matrix itself: no SYRK lists
+    for (int k = 0; k < 4; k++) cnt_i[4 * b + k] = (int)c[k];
+    for (int seg = 0; seg < 3; seg++)
+      for (c_int q = 0; q < c[seg]; q++) {
+        const size_t at = (b * 3 + seg) * M + q;
+        if (lists[at] < 0 || lists[at] >= m) return 1;
+        lists_i[at] = (int)lists[at];
+      }
+  }
+  ProbeBufs d;
+  BpProbeArgs P;
+  memset(&P, 0, sizeof(P));
+  P.nb = nb; P.n = n; P.m = m; P.ld = ld; P.from_q = from_q != 0; P.sscale = sscale; P.beta = beta;
+  double *dAt = d.get<double>(N * M), *dH0 = d.get<double>(from_q ? N * N : NB * N * N), *dw = d.get<double>(NB * 3 * M);
+  double *drhs = d.get<double>(NB * N);
+  int *dcnt = d.get<int>(NB * 4), *dl = d.get<int>(NB * 3 * M);
+  P.H = d.get<double>(NB * LL); P.L = d.get<double>(NB * LL); P.rdiag = d.get<double>(NB * ld);
+  P.d_fused = d.get<double>(NB * N); P.d_after = d.get<double>(NB * N);
+  P.info = d.get<int>(NB); P.queue = d.get<int>(1);
+  if (d.failed) return 2;
+  P.At = dAt; P.H0 = dH0; P.wts = dw; P.rhs = drhs; P.cnt = dcnt; P.lists = dl;
+  const cudaStream_t s = 0;
+  QB_CUDA_TRY(cudaMemcpyAsync(dAt, At, sizeof(double) * N * M, cudaMemcpyHostToDevice, s));
+  QB_CUDA_TRY(cudaMemcpyAsync(dH0, H0, sizeof(double) * (from_q ? N * N : NB * N * N), cudaMemcpyHostToDevice, s));
+  QB_CUDA_TRY(cudaMemcpyAsync(dw, wts, sizeof(double) * NB * 3 * M, cudaMemcpyHostToDevice, s));
+  QB_CUDA_TRY(cudaMemcpyAsync(drhs, rhs, sizeof(double) * NB * N, cudaMemcpyHostToDevice, s));
+  QB_CUDA_TRY(cudaMemcpyAsync(dcnt, cnt_i.data(), sizeof(int) * NB * 4, cudaMemcpyHostToDevice, s));
+  QB_CUDA_TRY(cudaMemcpyAsync(dl, lists_i.data(), sizeof(int) * NB * 3 * M, cudaMemcpyHostToDevice, s));
+  if (int r = shape == 4 ? batchp4_probe_newton(P, s) : batchp_probe_newton(P, s)) return r;
+  std::vector<double> hH(NB * LL), hL(NB * LL);
+  std::vector<int> hinfo(NB);
+  QB_CUDA_TRY(cudaMemcpyAsync(hH.data(), P.H, sizeof(double) * NB * LL, cudaMemcpyDeviceToHost, s));
+  QB_CUDA_TRY(cudaMemcpyAsync(hL.data(), P.L, sizeof(double) * NB * LL, cudaMemcpyDeviceToHost, s));
+  QB_CUDA_TRY(cudaMemcpyAsync(d_fused, P.d_fused, sizeof(double) * NB * N, cudaMemcpyDeviceToHost, s));
+  QB_CUDA_TRY(cudaMemcpyAsync(d_after, P.d_after, sizeof(double) * NB * N, cudaMemcpyDeviceToHost, s));
+  QB_CUDA_TRY(cudaMemcpyAsync(hinfo.data(), P.info, sizeof(int) * NB, cudaMemcpyDeviceToHost, s));
+  QB_CUDA_TRY(cudaStreamSynchronize(s));
+  for (size_t b = 0; b < NB; b++) {   // lower triangles, n x n column-major
+    info[b] = hinfo[b];
+    for (size_t j = 0; j < N; j++)
+      for (size_t i = 0; i < N; i++) {
+        H_out[b * N * N + i + N * j] = (i >= j) ? hH[b * LL + i + ld * j] : 0.0;
+        L_out[b * N * N + i + N * j] = (i >= j) ? hL[b * LL + i + ld * j] : 0.0;
+      }
+  }
+  return 0;
+}
+
+extern "C" int qpalm_b200_batchp_probe_sort(c_int shape, c_int nb_, c_int N_, unsigned long long *keys, unsigned int *vals) {
+  if ((shape != 3 && shape != 4) || nb_ < 1 || N_ < 1) return 1;
+  const int nb = (int)nb_, N = (int)N_;
+  const size_t T = (size_t)nb * N;
+  ProbeBufs d;
+  unsigned long long *dk = d.get<unsigned long long>(T);
+  unsigned int *dv = d.get<unsigned int>(T);
+  int *dq = d.get<int>(1);
+  if (d.failed) return 2;
+  const cudaStream_t s = 0;
+  QB_CUDA_TRY(cudaMemcpyAsync(dk, keys, sizeof(unsigned long long) * T, cudaMemcpyHostToDevice, s));
+  QB_CUDA_TRY(cudaMemcpyAsync(dv, vals, sizeof(unsigned int) * T, cudaMemcpyHostToDevice, s));
+  if (int r = shape == 4 ? batchp4_probe_sort(nb, N, dk, dv, dq, s) : batchp_probe_sort(nb, N, dk, dv, dq, s)) return r;
+  QB_CUDA_TRY(cudaMemcpyAsync(keys, dk, sizeof(unsigned long long) * T, cudaMemcpyDeviceToHost, s));
+  QB_CUDA_TRY(cudaMemcpyAsync(vals, dv, sizeof(unsigned int) * T, cudaMemcpyDeviceToHost, s));
+  QB_CUDA_TRY(cudaStreamSynchronize(s));
+  return 0;
+}
 
 extern "C" void qpalm_b200_batch_cleanup(QPALMB200Batch *B) {
   if (!B) return;

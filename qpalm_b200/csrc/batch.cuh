@@ -61,6 +61,7 @@ struct QPALMB200Batch {
   int *queue = nullptr;        // persistent engine: work-queue counter
   int engine = 0;              // 0 auto, 1 lock-step, 2 persistent (QPALM_B200_BATCH_ENGINE)
   int last_engine = 0;
+  int last_shape = 0;          // CTA shape of the last solve: 0 lock-step, 3 or 4 persistent (CTAs per SM)
   long long *prof = nullptr;   // persistent engine: optional per-phase clock totals [nb][16]
 };
 
@@ -71,4 +72,21 @@ int batchp_solve(QPALMB200Batch *B, int nb);
 // the same engine compiled in its 4-CTAs-per-SM shape (batchp.cu with -DQB_BP_VARIANT4)
 bool batchp4_supported(int n, int m);
 int batchp4_solve(QPALMB200Batch *B, int nb);
+
+// test probes of the persistent engine's in-CTA building blocks (device pointers; qpalm_b200_batchp_probe_* in batch.cu).
+// Per instance b: H0 is n x n (lds = n) at H0 + b n n, or with from_q the one shared matrix H0 scaled by sscale; cnt[4 b ..] =
+// {npos, nneg, nup, kpos}; lists / wts hold 3 m entries per instance: SYRK + rows at [0, m), SYRK - rows at [m, 2 m), update rows
+// at [2 m, 3 m).  H, L: ld x ld per instance, rdiag: ld per instance.
+struct BpProbeArgs {
+  int nb, n, m, ld, from_q;
+  double sscale, beta;
+  const double *At, *H0, *wts, *rhs;
+  const int *cnt, *lists;
+  double *H, *L, *rdiag, *d_fused, *d_after;
+  int *info, *queue;
+};
+int batchp_probe_newton(const BpProbeArgs &P, cudaStream_t s);
+int batchp4_probe_newton(const BpProbeArgs &P, cudaStream_t s);
+int batchp_probe_sort(int nb, int N, unsigned long long *keys, unsigned int *vals, int *queue, cudaStream_t s);
+int batchp4_probe_sort(int nb, int N, unsigned long long *keys, unsigned int *vals, int *queue, cudaStream_t s);
 }  // namespace qb

@@ -31,7 +31,8 @@
 
 using namespace qb;
 
-// Build-time shape of a CTA; this file is compiled twice (build.sh):
+// Build-time shape of a CTA; this file is compiled twice (build.sh), and each shape once more with -DQB_BP_PROBE, which
+// replaces the solver kernel by the test probes of its building blocks (see kbp_probe_newton):
 //   default            8 warps, 32-column panel (16-wide sub-panels), both sort buffers in shared memory: 80 registers x 256
 //                      threads, 72 KB -> 3 CTAs / SM (444 slots on a B200).  Best per-wave throughput: 444 instances in
 //                      57.9 ms (7675 solves/s), 4096 instances in 488 ms (8396 solves/s) at the end of round 2.
@@ -48,6 +49,8 @@ using namespace qb;
 #define QB_BP_NAMESPACE bp4
 #define QB_BP_SUPPORTED batchp4_supported
 #define QB_BP_SOLVE batchp4_solve
+#define QB_BP_PROBE_NEWTON batchp4_probe_newton
+#define QB_BP_PROBE_SORT batchp4_probe_sort
 #ifndef QB_BP_NT
 #define QB_BP_NT 256
 #endif
@@ -60,6 +63,16 @@ using namespace qb;
 #define QB_BP_NAMESPACE bp
 #define QB_BP_SUPPORTED batchp_supported
 #define QB_BP_SOLVE batchp_solve
+#define QB_BP_PROBE_NEWTON batchp_probe_newton
+#define QB_BP_PROBE_SORT batchp_probe_sort
+#endif
+#ifdef QB_BP_PROBE   // the probe objects carry their own copy of the device code: keep its (host-stub) symbols apart
+#undef QB_BP_NAMESPACE
+#ifdef QB_BP_VARIANT4
+#define QB_BP_NAMESPACE bp4_probe
+#else
+#define QB_BP_NAMESPACE bp_probe
+#endif
 #endif
 #ifndef QB_BP_NT
 #define QB_BP_NT 256
@@ -1544,6 +1557,7 @@ __device__ __noinline__ void p_store(const Args &P, int b, double *scratch) {
 #ifndef QB_BP_MINB
 #define QB_BP_MINB (QB_BP_NT <= 192 ? 4 : 3)
 #endif
+#ifndef QB_BP_PROBE
 __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_solve(const Args P) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ double scratch[32];
@@ -1692,7 +1706,124 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_solve(const Args P) {
   }
 }
 
+#else   // QB_BP_PROBE
+// ------------------------------------------------------------------------------------------------
+// test probes: the Newton-step building blocks and the line-search sort on caller data, run the way kbp_solve runs them
+// (same CTA shape, launch bounds, shared-memory carving, per-column mbarriers whose phase carries across the sweeps and the
+// instances of a CTA, persistent CTAs on an atomic queue), so that a test checks the code the solver executes.
+// They are built from this file in objects of their own (build.sh, -DQB_BP_PROBE): with a second caller in the same
+// translation unit, the __noinline__ building blocks (cta_updown_sweep, warp_factor_diag16) would no longer see kbp_solve's
+// __shared__ mbarrier and info addresses as constants, and kbp_solve would be compiled differently (more spills).
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ Smem probe_smem(unsigned char *smem_raw) {
+  Smem S;
+  S.u = smem_raw;
+  S.panel = reinterpret_cast<double *>(smem_raw);
+  S.vs = reinterpret_cast<double *>(smem_raw + kUnionBytes);
+  S.v = S.vs + VS_LEN;
+  S.rd = S.v + NMAX + 16;
+  return S;
+}
+
+// per instance b (batch.cuh, BpProbeArgs): H <- src, H += / -= the SYRK lists, L <- chol(H + beta I) with the fused forward
+// substitution, d_fused <- (L L')^{-1} rhs; then the rank update of L by the rows upd[0 .. nup) in sweeps of KU (kbp_solve's
+// update branch) and d_after <- (L L')^{-1} rhs with the final L and rdiag.  info[b]: bit 0 a sweep lost definiteness, bit 1
+// the factorisation met a non-positive pivot.
+__global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_probe_newton(const BpProbeArgs P) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  __shared__ int s_b;
+  __shared__ int s_info;
+  __shared__ __align__(8) unsigned long long s_udbar[UW];
+  unsigned ud_phase = 0;
+  if (threadIdx.x == 0) {
+    for (int j = 0; j < UW; j++) ud_mbar_init(s_udbar + j, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  __syncthreads();
+  const Smem S = probe_smem(smem_raw);
+  const int tid = threadIdx.x, n = P.n, m = P.m, ld = P.ld;
+  for (;;) {
+    __syncthreads();
+    if (tid == 0) s_b = atomicAdd(P.queue, 1);
+    __syncthreads();
+    const int b = s_b;
+    if (b >= P.nb) return;
+    const size_t on = (size_t)b * n, sLL = (size_t)ld * ld;
+    double *Hb = P.H + (size_t)b * sLL, *Lb = P.L + (size_t)b * sLL, *rdg = P.rdiag + (size_t)b * ld;
+    const int npos = P.cnt[4 * b], nneg = P.cnt[4 * b + 1], nup = P.cnt[4 * b + 2], kpos = P.cnt[4 * b + 3];
+    const int *lst = P.lists + (size_t)b * 3 * m;
+    const double *wt = P.wts + (size_t)b * 3 * m;
+    const double *src = P.from_q ? P.H0 : P.H0 + (size_t)b * n * n;
+    const double sc = P.from_q ? P.sscale : 1.0;
+    for (int i = tid; i < n; i += NT) {   // H <- sc * src (lower), kbp_solve's scratch copy of c Q
+      for (int j0 = 0; j0 <= i; j0 += 8) {
+        double v[8];
+#pragma unroll
+        for (int u = 0; u < 8; u++) v[u] = (j0 + u <= i) ? src[(size_t)i + (size_t)n * (j0 + u)] : 0.0;
+#pragma unroll
+        for (int u = 0; u < 8; u++) if (j0 + u <= i) Hb[(size_t)i + (size_t)ld * (j0 + u)] = v[u] * sc;
+      }
+    }
+    __syncthreads();
+    for (int pass = 0; pass < 2; pass++)
+      cta_syrk_list(Hb, ld, n, P.At, lst + pass * m, wt + pass * m, pass ? nneg : npos, pass ? -1.0 : 1.0, S);
+    for (int i = tid; i < n; i += NT) S.v[i] = P.rhs[on + i];
+    __syncthreads();
+    if (tid == 0) s_info = 0;
+    // from_q: the f.fq path, the factor reads the shared source (lds = n) directly; else the refactorisation of H (lds = ld)
+    cta_potrf(Lb, ld, P.from_q ? P.H0 : Hb, P.from_q ? n : ld, sc, P.beta, n, rdg, S, &s_info, true, nullptr);
+    cta_chol_solve(Lb, ld, n, rdg, S, true);
+    for (int i = tid; i < n; i += NT) P.d_fused[on + i] = S.v[i];
+    __syncthreads();
+    const int finfo = s_info;
+    __syncthreads();
+    if (tid == 0) s_info = 0;
+    __syncthreads();
+    for (int off = 0; off < nup; off += KU) {
+      const int k = (nup - off < KU) ? nup - off : KU;
+      const int kp = (kpos - off < 0) ? 0 : ((kpos - off < k) ? kpos - off : k);
+      cta_updown_sweep(Lb, ld, n, rdg, P.At, lst + 2 * m + off, wt + 2 * m + off, k, kp, S, &s_info, s_udbar, ud_phase, nullptr);
+    }
+    __syncthreads();
+    if (tid == 0) P.info[b] = (s_info ? 1 : 0) | (finfo ? 2 : 0);
+    for (int i = tid; i < n; i += NT) S.v[i] = P.rhs[on + i];
+    __syncthreads();
+    cta_chol_solve(Lb, ld, n, rdg, S, false);
+    for (int i = tid; i < n; i += NT) P.d_after[on + i] = S.v[i];
+  }
+}
+
+// p_sort on instance b's N (key, val) pairs at keys + b N, vals + b N, in place
+__global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_probe_sort(int nb, int N, unsigned long long *keys, unsigned int *vals, int *queue) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  __shared__ int s_b;
+  const Smem S = probe_smem(smem_raw);
+  for (;;) {
+    __syncthreads();
+    if (threadIdx.x == 0) s_b = atomicAdd(queue, 1);
+    __syncthreads();
+    const int b = s_b;
+    if (b >= nb) return;
+    p_sort(N, keys + (size_t)b * N, vals + (size_t)b * N, S);
+  }
+}
+
+// occupancy x SMs capped at nb: the grid QB_BP_SOLVE gives kbp_solve
+static int probe_grid(const void *kernel, int nb, int *grid) {
+  QB_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
+  int per_sm = 0, dev = 0, sms = 0;
+  QB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, NT, kSmemBytes));
+  QB_CUDA_TRY(cudaGetDevice(&dev));
+  QB_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  *grid = (per_sm < 1 ? 1 : per_sm) * sms;
+  if (*grid > nb) *grid = nb;
+  return 0;
+}
+#endif  // QB_BP_PROBE
+
 }  // namespace QB_BP_NAMESPACE (bp / bp4)
+
+#ifndef QB_BP_PROBE
 
 bool QB_BP_SUPPORTED(int n, int m) {
   return n >= 1 && n <= QB_BP_NAMESPACE::NMAX && m >= 1 && 2 * m <= QB_BP_NAMESPACE::SORT_MAX && m <= QB_BP_NAMESPACE::VS_LEN;
@@ -1732,5 +1863,29 @@ int QB_BP_SOLVE(QPALMB200Batch *B, int nb) {
   QB_CUDA_TRY(cudaGetLastError());
   return 0;
 }
+#else   // QB_BP_PROBE
+
+int QB_BP_PROBE_NEWTON(const BpProbeArgs &P, cudaStream_t s) {
+  using namespace QB_BP_NAMESPACE;
+  if (P.nb < 1 || P.n < 1 || P.n > NMAX || P.m < 1) return 1;
+  int grid = 0;
+  if (int r = probe_grid((const void *)kbp_probe_newton, P.nb, &grid)) return r;
+  QB_CUDA_TRY(cudaMemsetAsync(P.queue, 0, sizeof(int), s));
+  QB_LAUNCH(kbp_probe_newton, grid, NT, kSmemBytes, s, P);
+  QB_CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+
+int QB_BP_PROBE_SORT(int nb, int N, unsigned long long *keys, unsigned int *vals, int *queue, cudaStream_t s) {
+  using namespace QB_BP_NAMESPACE;
+  if (nb < 1 || N < 1 || N > SORT_MAX) return 1;
+  int grid = 0;
+  if (int r = probe_grid((const void *)kbp_probe_sort, nb, &grid)) return r;
+  QB_CUDA_TRY(cudaMemsetAsync(queue, 0, sizeof(int), s));
+  QB_LAUNCH(kbp_probe_sort, grid, NT, kSmemBytes, s, nb, N, keys, vals, queue);
+  QB_CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+#endif  // QB_BP_PROBE
 
 }  // namespace qb

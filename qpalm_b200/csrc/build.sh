@@ -18,6 +18,14 @@ if [ ! -f build/batchp4.o ] || [ batchp.cu -nt build/batchp4.o ] || [ batch.cuh 
   $NVCC $FLAGS -DQB_BP_VARIANT4 ${QB_BP4_FLAGS:--DQB_BP_SW=8} -c batchp.cu -o build/batchp4.o &
   pids+=($!)
 fi
+# and both shapes once more with the test probes of its building blocks instead of the solver kernel (-DQB_BP_PROBE)
+for v in batchp_probe batchp4_probe; do
+  if [ ! -f build/$v.o ] || [ batchp.cu -nt build/$v.o ] || [ batch.cuh -nt build/$v.o ] || [ common.cuh -nt build/$v.o ] || [ engine.cuh -nt build/$v.o ] || [ chol32.cuh -nt build/$v.o ] || [ ../../include/qpalm_b200.h -nt build/$v.o ]; then
+    if [ $v = batchp4_probe ]; then VF="-DQB_BP_VARIANT4 ${QB_BP4_FLAGS:--DQB_BP_SW=8}"; else VF=""; fi
+    $NVCC $FLAGS $VF -DQB_BP_PROBE -c batchp.cu -o build/$v.o &
+    pids+=($!)
+  fi
+done
 for p in "${pids[@]}"; do wait $p; done
-$NVCC -shared -o ../libqpalm_b200.so build/dense.o build/updown_flow.o build/updown_gen.o build/kernels.o build/api.o build/ops.o build/compat.o build/kkt.o build/batch.o build/batchp.o build/batchp4.o build/prof.o build/shard.o build/sparse.o build/sparse_sym.o build/qps.o -lcudart -ldl
+$NVCC -shared -o ../libqpalm_b200.so build/dense.o build/updown_flow.o build/updown_gen.o build/kernels.o build/api.o build/ops.o build/compat.o build/kkt.o build/batch.o build/batchp.o build/batchp4.o build/batchp_probe.o build/batchp4_probe.o build/prof.o build/shard.o build/sparse.o build/sparse_sym.o build/qps.o -lcudart -ldl
 echo "built $(cd .. && pwd)/libqpalm_b200.so"

@@ -24,6 +24,12 @@ def engine(request, monkeypatch):
 
 def _check_batch(b, idx, tol=1e-7):
     xs, ys, infos = qb.solve_batch(b)
+    _check_instances(b, idx, xs, ys, infos, tol)
+    return xs, ys, infos
+
+
+def _check_instances(b, idx, xs, ys, infos, tol=1e-7):
+    """Instances idx of a solved batch against the oracle: status, iteration counts, x, y and objective."""
     for k in idx:
         q = b.instance(k)
         o = solve_qp("oracle", q.Q.copy(), q.A.copy(), q.q, q.bmin, q.bmax, **q.settings)
@@ -35,7 +41,6 @@ def _check_batch(b, idx, tol=1e-7):
             assert _rel(xs[k], o.x) < tol, (k, _rel(xs[k], o.x))
             assert _rel(ys[k], o.y) < tol, (k, _rel(ys[k], o.y))
             assert abs(g["objective"] - o.objective) <= 1e-7 * max(1.0, abs(o.objective))
-    return xs, ys, infos
 
 
 def test_batch_small_chain80w_settings():
