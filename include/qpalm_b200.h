@@ -365,7 +365,7 @@ void qpalm_b200_batch_cleanup(QPALMB200Batch *batch);
  * Newton-step probe, per instance b < nb (matrices n x n column-major, lower triangle used; 1 <= n <= 240):
  *   H = src + sum_{pos} w^2 a a' - sum_{neg} w^2 a a', src = H0[b] (H0: nb x n x n), or with from_q the one shared matrix
  *       H0 scaled by sscale (the solver's path without active rows; then npos = nneg = 0 and the factor reads H0 itself)
- *   L = chol(H + beta I), d_fused = (L L')^{-1} rhs[b] with the forward substitution fused into the factorisation
+ *   L = chol(H + beta I), d_fused = (L L')^{-1} rhs[b] right after the factorisation
  *   then, nup > 0: rank update of L by the rows upd[0 .. nup), the first kpos entering (+), the rest leaving (-), in sweeps of 8
  *   d_after = (L L')^{-1} rhs[b] with the final L (separate forward and backward substitutions)
  * a = wts entry * column list entry of At (n x m, shared).  cnt: nb x 4 {npos, nneg, nup, kpos}; lists, wts: nb x 3m, per
@@ -375,6 +375,12 @@ void qpalm_b200_batch_cleanup(QPALMB200Batch *batch);
 int qpalm_b200_batchp_probe_newton(c_int shape, c_int nb, c_int n, c_int m, const c_float *At, const c_float *H0, c_int from_q,
         c_float sscale, const c_int *cnt, const c_int *lists, const c_float *wts, c_float beta, const c_float *rhs,
         c_float *H_out, c_float *L_out, c_float *d_fused, c_float *d_after, c_int *info);
+/* The Newton-step probe, then 2 rounds more triangular solves per instance, so that the solves' mbarrier phase carries across
+ * update sweeps, solves and instances: round r < rounds first updates L by the rows upd[0 .. nup), all entering (+) for even r and
+ * all leaving (-) for odd r; every round r < 2 rounds then writes (L L')^{-1} ((r + 1) rhs[b]) to d_rounds (nb x 2 rounds x n). */
+int qpalm_b200_batchp_probe_solves(c_int shape, c_int nb, c_int n, c_int m, const c_float *At, const c_float *H0, c_int from_q,
+        c_float sscale, const c_int *cnt, const c_int *lists, const c_float *wts, c_float beta, const c_float *rhs,
+        c_float *H_out, c_float *L_out, c_float *d_fused, c_float *d_after, c_int *info, c_int rounds, c_float *d_rounds);
 /* the line search's stable radix sort on nb independent arrays of N <= 2048 (key, val) pairs (nb x N each), in place */
 int qpalm_b200_batchp_probe_sort(c_int shape, c_int nb, c_int N, unsigned long long *keys, unsigned int *vals);
 

@@ -1088,11 +1088,10 @@ struct ProbeBufs {   // device buffers of one probe call, freed on every return 
 };
 }  // namespace
 
-extern "C" int qpalm_b200_batchp_probe_newton(c_int shape, c_int nb_, c_int n_, c_int m_, const c_float *At, const c_float *H0, c_int from_q,
-                                              c_float sscale, const c_int *cnt, const c_int *lists, const c_float *wts, c_float beta,
-                                              const c_float *rhs, c_float *H_out, c_float *L_out, c_float *d_fused, c_float *d_after,
-                                              c_int *info) {
-  if ((shape != 3 && shape != 4) || nb_ < 1 || n_ < 1 || m_ < 1) return 1;
+static int probe_newton(c_int shape, c_int nb_, c_int n_, c_int m_, const c_float *At, const c_float *H0, c_int from_q, c_float sscale,
+                        const c_int *cnt, const c_int *lists, const c_float *wts, c_float beta, const c_float *rhs, c_float *H_out,
+                        c_float *L_out, c_float *d_fused, c_float *d_after, c_int *info, c_int rounds, c_float *d_rounds) {
+  if ((shape != 3 && shape != 4) || nb_ < 1 || n_ < 1 || m_ < 1 || rounds < 0) return 1;
   const int nb = (int)nb_, n = (int)n_, m = (int)m_, ld = round_up(n, kPanel);
   const size_t NB = nb, N = n, M = m, LL = (size_t)ld * ld;
   std::vector<int> cnt_i(NB * 4), lists_i(NB * 3 * M, 0);
@@ -1117,6 +1116,7 @@ extern "C" int qpalm_b200_batchp_probe_newton(c_int shape, c_int nb_, c_int n_, 
   int *dcnt = d.get<int>(NB * 4), *dl = d.get<int>(NB * 3 * M);
   P.H = d.get<double>(NB * LL); P.L = d.get<double>(NB * LL); P.rdiag = d.get<double>(NB * ld);
   P.d_fused = d.get<double>(NB * N); P.d_after = d.get<double>(NB * N);
+  P.rounds = (int)rounds; P.d_rounds = d.get<double>(NB * 2 * (size_t)rounds * N + 1);
   P.info = d.get<int>(NB); P.queue = d.get<int>(1);
   if (d.failed) return 2;
   P.At = dAt; P.H0 = dH0; P.wts = dw; P.rhs = drhs; P.cnt = dcnt; P.lists = dl;
@@ -1135,6 +1135,7 @@ extern "C" int qpalm_b200_batchp_probe_newton(c_int shape, c_int nb_, c_int n_, 
   QB_CUDA_TRY(cudaMemcpyAsync(d_fused, P.d_fused, sizeof(double) * NB * N, cudaMemcpyDeviceToHost, s));
   QB_CUDA_TRY(cudaMemcpyAsync(d_after, P.d_after, sizeof(double) * NB * N, cudaMemcpyDeviceToHost, s));
   QB_CUDA_TRY(cudaMemcpyAsync(hinfo.data(), P.info, sizeof(int) * NB, cudaMemcpyDeviceToHost, s));
+  if (rounds) QB_CUDA_TRY(cudaMemcpyAsync(d_rounds, P.d_rounds, sizeof(double) * NB * 2 * (size_t)rounds * N, cudaMemcpyDeviceToHost, s));
   QB_CUDA_TRY(cudaStreamSynchronize(s));
   for (size_t b = 0; b < NB; b++) {   // lower triangles, n x n column-major
     info[b] = hinfo[b];
@@ -1145,6 +1146,21 @@ extern "C" int qpalm_b200_batchp_probe_newton(c_int shape, c_int nb_, c_int n_, 
       }
   }
   return 0;
+}
+
+extern "C" int qpalm_b200_batchp_probe_newton(c_int shape, c_int nb, c_int n, c_int m, const c_float *At, const c_float *H0, c_int from_q,
+                                              c_float sscale, const c_int *cnt, const c_int *lists, const c_float *wts, c_float beta,
+                                              const c_float *rhs, c_float *H_out, c_float *L_out, c_float *d_fused, c_float *d_after,
+                                              c_int *info) {
+  return probe_newton(shape, nb, n, m, At, H0, from_q, sscale, cnt, lists, wts, beta, rhs, H_out, L_out, d_fused, d_after, info, 0, nullptr);
+}
+
+extern "C" int qpalm_b200_batchp_probe_solves(c_int shape, c_int nb, c_int n, c_int m, const c_float *At, const c_float *H0, c_int from_q,
+                                              c_float sscale, const c_int *cnt, const c_int *lists, const c_float *wts, c_float beta,
+                                              const c_float *rhs, c_float *H_out, c_float *L_out, c_float *d_fused, c_float *d_after,
+                                              c_int *info, c_int rounds, c_float *d_rounds) {
+  return probe_newton(shape, nb, n, m, At, H0, from_q, sscale, cnt, lists, wts, beta, rhs, H_out, L_out, d_fused, d_after, info, rounds,
+                      d_rounds);
 }
 
 extern "C" int qpalm_b200_batchp_probe_sort(c_int shape, c_int nb_, c_int N_, unsigned long long *keys, unsigned int *vals) {

@@ -76,13 +76,14 @@ int batchp4_solve(QPALMB200Batch *B, int nb);
 // test probes of the persistent engine's in-CTA building blocks (device pointers; qpalm_b200_batchp_probe_* in batch.cu).
 // Per instance b: H0 is n x n (lds = n) at H0 + b n n, or with from_q the one shared matrix H0 scaled by sscale; cnt[4 b ..] =
 // {npos, nneg, nup, kpos}; lists / wts hold 3 m entries per instance: SYRK + rows at [0, m), SYRK - rows at [m, 2 m), update rows
-// at [2 m, 3 m).  H, L: ld x ld per instance, rdiag: ld per instance.
+// at [2 m, 3 m).  H, L: ld x ld per instance, rdiag: ld per instance.  rounds > 0: then 2 rounds more solves per instance into
+// d_rounds (nb x 2 rounds x n), see qpalm_b200_batchp_probe_solves.
 struct BpProbeArgs {
-  int nb, n, m, ld, from_q;
+  int nb, n, m, ld, from_q, rounds;
   double sscale, beta;
   const double *At, *H0, *wts, *rhs;
   const int *cnt, *lists;
-  double *H, *L, *rdiag, *d_fused, *d_after;
+  double *H, *L, *rdiag, *d_fused, *d_after, *d_rounds;
   int *info, *queue;
 };
 int batchp_probe_newton(const BpProbeArgs &P, cudaStream_t s);

@@ -745,34 +745,8 @@ __device__ __forceinline__ void panel_update16(double *Pn, int c0, int w, int ro
 }
 
 // L <- chol(sscale * src + beta I) (lower, n x n), right-looking with PW-column panels.  rdiag_g[j] = 1 / l_jj.
-// forward substitution step of one resident panel: z_k = L_kk^{-1} v_k (warp 0), v_below -= L_below,k z_k (all threads)
-__device__ __forceinline__ void panel_forward(const double *Pn, double *v, const double *rdv, int k0, int w, int rows) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (warp == 0) {
-    double vl = (lane < w) ? v[k0 + lane] : 0.0;
-    const double rd = (lane < w) ? rdv[lane] : 1.0;
-    __syncwarp();   // re-join the warp: a split warp pays the slow collective path on every shuffle
-    for (int j = 0; j < w; j++) {
-      const double zj = __shfl_sync(0xffffffffu, vl, j) * __shfl_sync(0xffffffffu, rd, j);
-      if (lane == j) vl = zj;
-      else if (lane > j && lane < w) vl = fma(-Pn[j * LDP + lane], zj, vl);
-    }
-    if (lane < w) v[k0 + lane] = vl;
-  }
-  __syncthreads();
-  for (int r = w + tid; r < rows; r += NT) {
-    double s0 = 0.0, s1 = 0.0;
-    int t = 0;
-    for (; t + 1 < w; t += 2) { s0 = fma(Pn[t * LDP + r], v[k0 + t], s0); s1 = fma(Pn[(t + 1) * LDP + r], v[k0 + t + 1], s1); }
-    if (t < w) s0 = fma(Pn[t * LDP + r], v[k0 + t], s0);
-    v[k0 + r] -= (s0 + s1);
-  }
-  __syncthreads();
-}
-
-// fwd: additionally run the forward substitution L z = v on S.v while each panel is resident (saves re-reading L).
 __device__ __forceinline__ void cta_potrf(double *L, int ld, const double *src, int lds, double sscale, double beta, int n, double *rdiag_g,
-                          const Smem &S, int *info, bool fwd, long long *pf) {
+                          const Smem &S, int *info, long long *pf) {
   const int tid = threadIdx.x;
   double *Pn = S.panel;
   long long tq = clock64();
@@ -812,9 +786,6 @@ __device__ __forceinline__ void cta_potrf(double *L, int ld, const double *src, 
       if (r >= t) L[(size_t)(k0 + r) + (size_t)ld * (k0 + t)] = Pn[t * LDP + r];
     }
     if (tid < w) rdiag_g[k0 + tid] = S.rd[tid];
-    if (fwd) {
-      panel_forward(Pn, S.v, S.rd, k0, w, rows);   // ends with a barrier; only reads the panel
-    }
     PQ(20);
     if (w & 3) {   // ragged last panel: zero the pad columns the DMMA product loop reads (no trailing matrix then, but keep it defined)
       for (int idx = tid; idx < (((w + 3) & ~3) - w) * rows; idx += NT) { const int t = w + idx / rows, r = idx - (t - w) * rows; Pn[t * LDP + r] = 0.0; }
@@ -825,48 +796,6 @@ __device__ __forceinline__ void cta_potrf(double *L, int ld, const double *src, 
     PQ(21);
   }
 #undef PQ
-}
-
-// v <- (L L')^{-1} v, v in shared memory (S.v), L n x n lower in global memory, rdiag_g = 1 / diag(L).
-// skip_forward: the forward substitution was already done inside cta_potrf.
-__device__ __forceinline__ void cta_chol_solve(const double *L, int ld, int n, const double *rdiag_g, const Smem &S, bool skip_forward) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  double *Pn = S.panel, *v = S.v;
-  if (!skip_forward) {
-    for (int k0 = 0; k0 < n; k0 += PW) {   // forward: L z = v
-      const int w = (n - k0 < PW) ? n - k0 : PW, rows = n - k0;
-      panel_load_async(Pn, L, ld, k0, w, rows);
-      if (tid < w) S.rd[tid] = rdiag_g[k0 + tid];
-      __syncthreads();
-      panel_forward(Pn, v, S.rd, k0, w, rows);
-    }
-  }
-  // backward: L' d = z
-  const int last = ((n - 1) / PW) * PW;
-  for (int k0 = last; k0 >= 0; k0 -= PW) {
-    const int w = (n - k0 < PW) ? n - k0 : PW, rows = n - k0;
-    panel_load_async(Pn, L, ld, k0, w, rows);
-    __syncthreads();
-    for (int t = warp; t < w; t += NW) {   // v[k0 + t] -= sum_{r >= w} L(k0 + r, k0 + t) d(k0 + r)
-      double s = 0.0;
-      for (int r = w + lane; r < rows; r += 32) s = fma(Pn[t * LDP + r], v[k0 + r], s);
-      s = warp_sum(s);
-      if (lane == 0) S.rd[PW + t] = s;
-    }
-    __syncthreads();
-    if (warp == 0) {
-      double vl = (lane < w) ? v[k0 + lane] - S.rd[PW + lane] : 0.0;
-      const double rd = (lane < w) ? rdiag_g[k0 + lane] : 1.0;
-      __syncwarp();
-      for (int j = w - 1; j >= 0; j--) {
-        const double dj = __shfl_sync(0xffffffffu, vl, j) * __shfl_sync(0xffffffffu, rd, j);
-        if (lane == j) vl = dj;
-        else if (lane < j) vl = fma(-Pn[lane * LDP + j], dj, vl);   // L(k0 + j, k0 + lane)
-      }
-      if (lane < w) v[k0 + lane] = vl;
-    }
-    __syncthreads();
-  }
 }
 
 // dst(lower) += sign * sum_{c < cnt} (wgt[c] A'[:, list[c]]) (...)'   in chunks of PW list entries staged in the panel
@@ -1179,6 +1108,177 @@ __device__ __noinline__ void cta_updown_sweep(double *L, int ld, int n, double *
   __syncthreads();
   PQ(24);
 #undef PQ
+}
+
+// ------------------------------------------------------------------------------------------------
+// v <- (L L')^{-1} v: the two triangular solves of the Newton step, as the dataflow of the update sweep.  v is S.v, L the
+// instance's factor in global memory (n x n lower), rdiag_g = 1 / diag(L).  Both directions walk 16-column blocks:
+//   * the CHAIN WARP (warp 0) holds the 32-entry window of v at the block (the 16 block entries and 16 look-ahead entries) in
+//     registers and the window's entries of L in a shared buffer requested one block ahead (cp.async, warp 1); per column it
+//     forms the next solution entry, publishes it in S.v, arrives on that column's mbarrier and applies it to its window;
+//   * every other thread owns one entry of v outside the window -- forward: row t (thread t), backward: column t - 32 --, keeps it
+//     in a register, streams its entries of the block's L through a private cp.async ring (LVW ahead of use, as the sweep's row
+//     owners) and applies each column as soon as its mbarrier completes;
+//   * at a block's end the entries that enter the next window are handed to the chain through S.v (named barrier 1).
+// The panel-staged form it replaces paid, per 24 / 32-column panel, a full load of the panel, a wait and three barriers with
+// seven warps parked behind one warp's chain (13 us per panel at 512 instances, profiles/r03a_batch_phase_clocks_parent_solve_split.txt).
+// Rounding: every entry is updated by one fma per column in column order (forward: ascending j, z_j = v_j / l_jj as v_j * rdiag;
+// backward: descending i, d_j likewise), whoever holds it, so the result does not depend on the CTA shape.  This is the only
+// forward substitution of the engine: the factorisation no longer runs one while its panels are resident.
+// ------------------------------------------------------------------------------------------------
+constexpr int SV_SLOT = UW * PBL + UW;   // one window block: 16 x 32 entries of L at [c * PBL + lane] and the block's 16 1 / l_jj
+constexpr int SV_NWIN = 3;               // window blocks: in use by the chain / requested one and two blocks ahead
+constexpr int SV_G = 4;                  // owners: columns applied per mbarrier wait
+static_assert((SV_NWIN * SV_SLOT * sizeof(double)) % 16 == 0 && (SV_NWIN * SV_SLOT + UW * NT) * sizeof(double) <= kUnionBytes,
+              "the window blocks + the owners' staging ring of the triangular solves must fit the union region");
+
+// The owners poll with test_wait.  A thread suspended in try_wait (ud_mbar_wait) resumed too late for a chain step of ~180 clocks:
+// at 512 instances the chain then spent 2.6 us per block end waiting for the owners' last columns (4.9 of the solve's 8.4 ms per
+// instance); polling took the launch from 78.4 to 76.1 ms.  The sweep keeps try_wait: its owners have eight ranks of work per column.
+__device__ __forceinline__ void sv_mbar_wait_spin(unsigned long long *bar, unsigned parity) {
+  const unsigned a = (unsigned)__cvta_generic_to_shared(bar);
+  asm volatile("{\n.reg .pred p;\nWAIT_%=:\nmbarrier.test_wait.parity.shared::cta.b64 p, [%0], %1;\n@!p bra WAIT_%=;\n}\n" ::"r"(a), "r"(parity) : "memory");
+}
+
+// 16-byte cp.async that bypasses L1 (.cg has no 8-byte form)
+__device__ __forceinline__ void bp_cp_async16_cg(void *smem_dst, const double *gsrc) {
+  const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gsrc) : "memory");
+}
+
+// request window block k0: forward rows k0 + lane, columns k0 + c (c <= lane); backward rows k0 + c, columns k0 - 16 + lane
+// (lower triangle only, zeros elsewhere); 1 / l_jj of columns k0 .. k0 + 15 behind them.  Called by the chain warp.
+template <bool fwd>
+__device__ __forceinline__ void sv_block_prefetch(double *Pb, const double *L, int ld, const double *rdiag_g, int k0, int n, int lane) {
+#pragma unroll
+  for (int c = 0; c < UW; c++) {
+    const int row = fwd ? k0 + lane : k0 + c, col = fwd ? k0 + c : k0 - UW + lane;
+    if (row < n && col >= 0 && col <= row) bp_cp_async8(&Pb[c * PBL + lane], L + (size_t)row + (size_t)ld * col);
+    else Pb[c * PBL + lane] = 0.0;
+  }
+  if (lane < UW && k0 + lane < n) bp_cp_async8(&Pb[UW * PBL + lane], rdiag_g + k0 + lane);
+  bp_cp_async_commit();
+}
+
+// chain warp.  fwd: lane = row k0 + lane; block columns ascending.  bwd: lane = column k0 - 16 + lane; block rows descending.
+// It requests its own window blocks, two ahead, so a block's L is in flight for two blocks' worth of chain.
+// Slots pf[0] / pf[1]: the column loops / the block-end rendezvous and window waits (clock of lane 31).
+template <bool fwd>
+__device__ __forceinline__ void sv_chain_role(const double *L, int ld, int n, const double *rdiag_g, double *v, double *Pb0, unsigned long long *bars,
+                                              long long *pf) {
+  const int lane = threadIdx.x & 31;
+  long long tq = clock64();
+#define PC(k) do { if (pf) { const long long t_ = clock64(); if (lane == 31) atomicAdd(reinterpret_cast<unsigned long long *>(pf + (k)), (unsigned long long)(t_ - tq)); tq = t_; } } while (0)
+  const int nblk = (n + UW - 1) / UW;
+  auto blk_k0 = [&](int blk) { return fwd ? blk * UW : (nblk - 1 - blk) * UW; };
+#pragma unroll 1
+  for (int blk = 0; blk < 2; blk++) {
+    if (blk < nblk) sv_block_prefetch<fwd>(Pb0 + blk * SV_SLOT, L, ld, rdiag_g, blk_k0(blk), n, lane);
+    else bp_cp_async_commit();
+  }
+  for (int blk = 0; blk < nblk; blk++) {
+    const int k0 = blk_k0(blk), w = (n - k0 < UW) ? n - k0 : UW;
+    if (blk + 2 < nblk) sv_block_prefetch<fwd>(Pb0 + ((blk + 2) % SV_NWIN) * SV_SLOT, L, ld, rdiag_g, blk_k0(blk + 2), n, lane);
+    else bp_cp_async_commit();   // an empty group: "all but the two newest groups" stays "this block's window"
+    bp_cp_async_wait_group<2>();
+    __syncwarp();
+    PC(1);
+    const double *Pb = Pb0 + (blk % SV_NWIN) * SV_SLOT, *rd = Pb + UW * PBL;
+    const int e = fwd ? k0 + lane : k0 - UW + lane;   // this lane's entry of v
+    const bool valid = e >= 0 && e < n;
+    double x = valid ? v[e] : 0.0;
+    for (int jj = 0; jj < w; jj++) {
+      const int j = fwd ? jj : w - 1 - jj, src = fwd ? j : UW + j;   // column (fwd) / row (bwd) k0 + j, held by lane src
+      const double a = Pb[j * PBL + lane], r = rd[j];
+      const double z = __shfl_sync(0xffffffffu, x, src) * r;
+      if (lane == 0) v[k0 + j] = z;
+      ud_mbar_arrive_lane0(bars + j, lane);   // entry k0 + j is final: the owners may apply it
+      const bool after = fwd ? lane > src : lane < src;
+      x = (lane == src) ? z : (after ? fma(-a, z, x) : x);
+    }
+    PC(0);
+    for (int j = w; j < UW; j++) ud_mbar_arrive_lane0(bars + j, lane);   // ragged block: every barrier completes one phase per block
+    if ((fwd ? lane >= UW : lane < UW) && valid) v[e] = x;              // the look-ahead entries: the next block's window
+    ud_block_barrier();
+  }
+  PC(1);
+#undef PC
+}
+
+// an owner (threads >= 32).  fwd: row t = thread t, below the window (t >= k0 + 32); bwd: column t - 32, left of the window
+// (t - 32 < k0 - 16).  Its entries of L arrive through a private ring in shared memory, a whole block (16 entries) ahead of use:
+// fwd 16 slots of 8 bytes, L(e, col), one per column (neighbouring threads read neighbouring rows: whole sectors per warp);
+// bwd 8 slots of 16 bytes, L(r, e) L(r + 1, e) with r even, one per two rows (a column segment, read in whole 16-byte pieces
+// past L1: the 8-byte form would allocate an L1 line per thread that the co-resident CTAs need for their own working sets).
+template <bool fwd>
+__device__ __forceinline__ void sv_owner_role(const double *L, int ld, int n, double *v, double2 *R, unsigned long long *bars, unsigned phase) {
+  const int t = threadIdx.x, e = fwd ? t : t - WIN;
+  const int nblk = (n + UW - 1) / UW, last = (nblk - 1) * UW;
+  double *R8 = reinterpret_cast<double *>(R);
+  double x = (e < n) ? v[e] : 0.0;
+  if (fwd ? (e >= WIN && e < n) : (e < last - UW)) {
+#pragma unroll
+    for (int q = 0; q < (fwd ? UW : UW / 2); q++) {   // fwd: columns 0 .. 15; bwd: rows last + 14 - 2 q, + 1
+      if (fwd) { if (q < n) bp_cp_async8(&R8[q * NT + t], L + (size_t)e + (size_t)ld * q); }
+      else if (last + UW - 2 - 2 * q < n) bp_cp_async16_cg(&R[q * NT + t], L + (size_t)ld * e + (last + UW - 2 - 2 * q));
+      bp_cp_async_commit();
+    }
+  }
+  for (int blk = 0; blk < nblk; blk++) {
+    const int k0 = fwd ? blk * UW : last - blk * UW, w = (n - k0 < UW) ? n - k0 : UW;
+    const unsigned par = (phase + blk) & 1u;
+    const bool own = fwd ? (e >= k0 + WIN && e < n) : (e < k0 - UW);
+    const bool own_next = fwd ? (e >= k0 + UW + WIN && e < n) : (e < k0 - 2 * UW);
+    if (own) {
+#pragma unroll 1
+      for (int p = 0; p < UW; p++) {   // rolled: sixteen copies of the wait loops cost instruction-cache misses in every other phase
+        const int j = fwd ? p : UW - 1 - p;
+        if (j < w) {
+          if (fwd) bp_cp_async_wait_group<UW - 1>();   // this slot has landed (the later ones may be in flight)
+          else bp_cp_async_wait_group<UW / 2 - 1>();
+          // one wait per group of SV_G columns, on the group's last column in chain order (the chain publishes in order): a woken
+          // owner then applies SV_G columns, where one wait per column cost more than the chain's step and left the owners a
+          // block's worth of wake-ups behind it at every block end
+          if (fwd ? (j % SV_G == 0) : (j % SV_G == SV_G - 1 || j == w - 1))
+            sv_mbar_wait_spin(bars + (fwd ? min(j | (SV_G - 1), w - 1) : (j & ~(SV_G - 1))), par);
+          double l;
+          if (fwd) l = R8[p * NT + t];
+          else { const double2 l2 = R[(p >> 1) * NT + t]; l = (p & 1) ? l2.x : l2.y; }
+          x = fma(-l, v[k0 + j], x);
+        }
+        // the slot is used up: refill it with the same slot of the next block
+        if (fwd) {
+          if (own_next && k0 + UW + p < n) bp_cp_async8(&R8[p * NT + t], L + (size_t)e + (size_t)ld * (k0 + UW + p));
+          bp_cp_async_commit();
+        } else if (p & 1) {
+          if (own_next) bp_cp_async16_cg(&R[(p >> 1) * NT + t], L + (size_t)ld * e + (k0 - 1 - p));
+          bp_cp_async_commit();
+        }
+      }
+      if (!own_next) v[e] = x;   // this entry enters the chain warp's window with the next block
+    }
+    ud_block_barrier();
+  }
+}
+
+// one direction (nblk blocks, mbarrier phases phase .. phase + nblk - 1)
+template <bool fwd>
+__device__ __forceinline__ void sv_direction(const double *L, int ld, int n, const double *rdiag_g, const Smem &S, unsigned long long *bars,
+                                             unsigned phase, long long *pf) {
+  double *Pb0 = S.panel;
+  double2 *R = reinterpret_cast<double2 *>(S.panel + SV_NWIN * SV_SLOT);
+  if (threadIdx.x < 32) sv_chain_role<fwd>(L, ld, n, rdiag_g, S.v, Pb0, bars, pf);
+  else sv_owner_role<fwd>(L, ld, n, S.v, R, bars, phase);
+  __syncthreads();
+}
+// bars / phase: the update sweep's per-column mbarriers and their phase count (each direction completes one phase of each barrier
+// per block).  pf: the instance's phase-clock row (slots 28 .. 31), or null.
+__device__ __noinline__ void cta_chol_solve(const double *L, int ld, int n, const double *rdiag_g, const Smem &S, unsigned long long *bars,
+                                            unsigned &phase, long long *pf) {
+  const unsigned nblk = (unsigned)((n + UW - 1) / UW), ph = phase;   // phase lives in the caller's frame: read and written once
+  sv_direction<true>(L, ld, n, rdiag_g, S, bars, ph, pf ? pf + 28 : nullptr);           // L z = v
+  sv_direction<false>(L, ld, n, rdiag_g, S, bars, ph + nblk, pf ? pf + 30 : nullptr);   // L' d = z
+  phase = ph + 2 * nblk;
 }
 
 // ordered lists of the entering (candidate active, not in the factor) and leaving rows, entering first, weights sqrt(sigma):
@@ -1664,11 +1764,11 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_solve(const Args P) {
         if (factor) {
           const double beta = P.ctl[b].beta;
           if (tid == 0) s_info = 0;
-          cta_potrf(Lb, ld, f.fq ? P.Qs : Hb, f.fq ? n : ld, f.fq ? P.ctl[b].c : 1.0, beta, n, rdg, S, &s_info, true,
+          cta_potrf(Lb, ld, f.fq ? P.Qs : Hb, f.fq ? n : ld, f.fq ? P.ctl[b].c : 1.0, beta, n, rdg, S, &s_info,
                     P.prof ? P.prof + (size_t)b * 32 : nullptr);
         }
         PH(7);
-        cta_chol_solve(Lb, ld, n, rdg, S, factor != 0);
+        cta_chol_solve(Lb, ld, n, rdg, S, s_udbar, ud_phase, P.prof ? P.prof + (size_t)b * 32 : nullptr);
         for (int i = tid; i < n; i += NT) P.d[on + i] = S.v[i];
         for (int i = tid; i < m; i += NT) P.active_old[om + i] = P.active[om + i];
         __syncthreads();
@@ -1725,9 +1825,9 @@ __device__ __forceinline__ Smem probe_smem(unsigned char *smem_raw) {
   return S;
 }
 
-// per instance b (batch.cuh, BpProbeArgs): H <- src, H += / -= the SYRK lists, L <- chol(H + beta I) with the fused forward
-// substitution, d_fused <- (L L')^{-1} rhs; then the rank update of L by the rows upd[0 .. nup) in sweeps of KU (kbp_solve's
-// update branch) and d_after <- (L L')^{-1} rhs with the final L and rdiag.  info[b]: bit 0 a sweep lost definiteness, bit 1
+// per instance b (batch.cuh, BpProbeArgs): H <- src, H += / -= the SYRK lists, L <- chol(H + beta I), d_fused <- (L L')^{-1} rhs;
+// then the rank update of L by the rows upd[0 .. nup) in sweeps of KU (kbp_solve's update branch) and d_after <- (L L')^{-1} rhs
+// with the final L and rdiag; then P.rounds rounds of {+ or - the update rows, solve} and P.rounds rounds of {solve}.  info[b]: bit 0 a sweep lost definiteness, bit 1
 // the factorisation met a non-positive pivot.
 __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_probe_newton(const BpProbeArgs P) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -1771,8 +1871,8 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_probe_newton(const BpProbe
     __syncthreads();
     if (tid == 0) s_info = 0;
     // from_q: the f.fq path, the factor reads the shared source (lds = n) directly; else the refactorisation of H (lds = ld)
-    cta_potrf(Lb, ld, P.from_q ? P.H0 : Hb, P.from_q ? n : ld, sc, P.beta, n, rdg, S, &s_info, true, nullptr);
-    cta_chol_solve(Lb, ld, n, rdg, S, true);
+    cta_potrf(Lb, ld, P.from_q ? P.H0 : Hb, P.from_q ? n : ld, sc, P.beta, n, rdg, S, &s_info, nullptr);
+    cta_chol_solve(Lb, ld, n, rdg, S, s_udbar, ud_phase, nullptr);
     for (int i = tid; i < n; i += NT) P.d_fused[on + i] = S.v[i];
     __syncthreads();
     const int finfo = s_info;
@@ -1788,8 +1888,21 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_probe_newton(const BpProbe
     if (tid == 0) P.info[b] = (s_info ? 1 : 0) | (finfo ? 2 : 0);
     for (int i = tid; i < n; i += NT) S.v[i] = P.rhs[on + i];
     __syncthreads();
-    cta_chol_solve(Lb, ld, n, rdg, S, false);
+    cta_chol_solve(Lb, ld, n, rdg, S, s_udbar, ud_phase, nullptr);
     for (int i = tid; i < n; i += NT) P.d_after[on + i] = S.v[i];
+    for (int r = 0; r < 2 * P.rounds; r++) {   // rounds x {update sweeps, solve}, then rounds x {solve}
+      __syncthreads();
+      if (r < P.rounds) {   // the update rows, all entering in even rounds and all leaving in odd ones
+        for (int off = 0; off < nup; off += KU) {
+          const int k = (nup - off < KU) ? nup - off : KU;
+          cta_updown_sweep(Lb, ld, n, rdg, P.At, lst + 2 * m + off, wt + 2 * m + off, k, (r & 1) ? 0 : k, S, &s_info, s_udbar, ud_phase, nullptr);
+        }
+      }
+      for (int i = tid; i < n; i += NT) S.v[i] = P.rhs[on + i] * (double)(r + 1);
+      __syncthreads();
+      cta_chol_solve(Lb, ld, n, rdg, S, s_udbar, ud_phase, nullptr);
+      for (int i = tid; i < n; i += NT) P.d_rounds[((size_t)b * 2 * P.rounds + r) * n + i] = S.v[i];
+    }
   }
 }
 
