@@ -337,7 +337,9 @@ int  qpalm_b200_qps_solve(const char *qps_path, const char *settings_path, QPALM
 /* ------------------------------------------------------------------------------------------------
  * Part 3 -- batch entry point (additive).  `nb` QPs sharing Q, A (values and pattern) and settings
  * but with their own q, bmin, bmax.  Each instance's result equals what qpalm_setup + qpalm_solve
- * return for that instance alone.  q: nb x n, bmin/bmax: nb x m (row-major, one instance per row).
+ * return for that instance alone; after qpalm_b200_batch_warm_start, what qpalm_setup +
+ * qpalm_warm_start(x_ws[k], y_ws[k]) + qpalm_solve return for instance k alone.
+ * q: nb x n, bmin/bmax: nb x m (row-major, one instance per row).
  * Outputs (host): x: nb x n, y: nb x m, info: nb entries.  One persistent CTA per instance in flight.
  * ---------------------------------------------------------------------------------------------- */
 typedef struct QPALMB200Batch QPALMB200Batch;
@@ -349,6 +351,12 @@ int  qpalm_b200_batch_solve(QPALMB200Batch *batch, c_int nb, const c_float *q, c
 int  qpalm_b200_batch_upload(QPALMB200Batch *batch, c_int nb, const c_float *q, const c_float *bmin, const c_float *bmax);
 int  qpalm_b200_batch_solve_resident(QPALMB200Batch *batch, c_int nb, double *device_ms);
 int  qpalm_b200_batch_download(QPALMB200Batch *batch, c_int nb, c_float *x, c_float *y, QPALMInfo *info);
+/* Warm start of the NEXT batch solve, per instance (qpalm_warm_start, qpalm.c:322-399): x_ws nb x n, y_ws nb x m, host,
+ * row-major, unscaled (what a solve returns).  Either may be NULL: that part starts cold.  Instances k < nb start from
+ * row k; instances >= nb of the next solve start cold.  Consumed by the next qpalm_b200_batch_solve / _solve_resident,
+ * like qpalm_solve resets `initialized`; (NULL, NULL) clears a pending warm start (nb is not read).  Returns 0, 1 for
+ * invalid arguments (pending state unchanged), < 0 for a CUDA error (no warm start pending). */
+int  qpalm_b200_batch_warm_start(QPALMB200Batch *batch, c_int nb, const c_float *x_ws, const c_float *y_ws);
 /* totals of the last solve over instances 0..nb-1: out8 = {inner iterations, outer iterations, refactorisations,
  * sum of |J| over the refactorisations, engine (1 lock-step, 2 persistent), rank-k update sweeps, sum of their ranks,
  * downdates that lost definiteness (followed by a refactorisation)} -- inputs of the SURVEY 8(d) byte model */

@@ -24,6 +24,8 @@ def _lib():
         lib.qpalm_b200_batch_solve_resident.restype = C.c_int
         lib.qpalm_b200_batch_download.argtypes = [C.c_void_p, abi.c_int, c_float_p, c_float_p, C.POINTER(QPALMInfo)]
         lib.qpalm_b200_batch_download.restype = C.c_int
+        lib.qpalm_b200_batch_warm_start.argtypes = [C.c_void_p, abi.c_int, c_float_p, c_float_p]
+        lib.qpalm_b200_batch_warm_start.restype = C.c_int
         lib.qpalm_b200_batch_last_launches.argtypes = [C.c_void_p]
         lib.qpalm_b200_batch_last_launches.restype = C.c_longlong
         lib.qpalm_b200_batch_last_shape.argtypes = [C.c_void_p]
@@ -61,10 +63,33 @@ class Batch:
     def ok(self):
         return bool(self.h)
 
-    def solve(self, q, bmin, bmax, x=None, y=None, info=None, raw_info=False):
+    def warm_start(self, x=None, y=None):
+        """Warm start of the next solve (qpalm_warm_start per instance): x is nb' x n, y is nb' x m, unscaled, as a solve
+        returns them; instances k < nb' start from row k, the others cold.  Either may be None: that part starts cold.
+        warm_start() with neither clears a pending warm start."""
+        x = None if x is None else np.ascontiguousarray(x, dtype=np.float64)
+        y = None if y is None else np.ascontiguousarray(y, dtype=np.float64)
+        rows = None
+        for name, a, cols in (("x", x, self.n), ("y", y, self.m)):
+            if a is None:
+                continue
+            if a.ndim != 2 or a.shape[1] != cols:
+                raise ValueError(f"warm start {name}: expected nb x {cols}, got shape {a.shape}")
+            if rows is not None and a.shape[0] != rows:
+                raise ValueError(f"warm start x and y have different row counts ({rows} and {a.shape[0]})")
+            rows = a.shape[0]
+        if rows is not None and not 1 <= rows <= self.nb_max:
+            raise ValueError(f"warm start of {rows} instances: expected 1 to nb_max = {self.nb_max}")
+        rc = self.lib.qpalm_b200_batch_warm_start(self.h, rows or 0, None if x is None else fptr(x), None if y is None else fptr(y))
+        if rc:
+            raise RuntimeError(f"qpalm_b200_batch_warm_start failed: {rc}")
+
+    def solve(self, q, bmin, bmax, x=None, y=None, info=None, raw_info=False, x_ws=None, y_ws=None):
         """One call of the batch entry point with HOST buffers (H2D of q / bmin / bmax, solve, D2H of x / y / info).
         x, y, info: optional caller-owned result buffers (e.g. pinned memory) reused across calls; raw_info=True returns the
-        QPALMInfo array itself instead of a list of dicts."""
+        QPALMInfo array itself instead of a list of dicts.  x_ws, y_ws: warm start of this solve (see warm_start)."""
+        if x_ws is not None or y_ws is not None:
+            self.warm_start(x_ws, y_ws)
         nb = q.shape[0]
         q, bmin, bmax = (np.ascontiguousarray(a, dtype=np.float64) for a in (q, bmin, bmax))
         if x is None:
@@ -139,10 +164,11 @@ def available() -> bool:
         return False
 
 
-def solve_batch(b, nb_max=None):
+def solve_batch(b, nb_max=None, x_ws=None, y_ws=None):
     h = Batch(b.Q, b.A, b.settings, nb_max or b.q.shape[0])
     if not h.ok:
         raise RuntimeError("batch setup failed")
-    out = h.solve(b.q, b.bmin, b.bmax)
-    h.cleanup()
-    return out
+    try:
+        return h.solve(b.q, b.bmin, b.bmax, x_ws=x_ws, y_ws=y_ws)
+    finally:
+        h.cleanup()

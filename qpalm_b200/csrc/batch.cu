@@ -79,6 +79,68 @@ kb_init(int n, int m, BSet st, const double *__restrict__ D, const double *__res
 }
 
 // ------------------------------------------------------------------------------------------------
+// warm start of instances b < grid after kb_init (qpalm_warm_start, qpalm.c:322-399): x = Dinv x_ws (x0 = x_prev = x),
+// y = c Einv y_ws; with x, kb_gemv_rows / kb_gemv_cols then form Qd = c (D Q D) x and Ad = A x, and kb_warm_sigma finishes.
+// A null x_ws or y_ws leaves that part cold.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+kb_warm_set(int n, int m, BSet st, const double *__restrict__ Dinv, const double *__restrict__ Einv, const double *__restrict__ x_ws,
+            const double *__restrict__ y_ws, const BCtl *__restrict__ ctl, double *x, double *x0, double *x_prev, double *y) {
+  const int b = blockIdx.x;
+  const size_t on = (size_t)b * n, om = (size_t)b * m;
+  if (x_ws)
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+      double v = x_ws[on + i];
+      if (st.scaling) v = v * Dinv[i];
+      x[on + i] = v; x0[on + i] = v; x_prev[on + i] = v;
+    }
+  if (y_ws) {
+    const double cc = ctl[b].c;
+    for (int i = threadIdx.x; i < m; i += blockDim.x) {
+      double v = y_ws[om + i];
+      if (st.scaling) { v = v * Einv[i]; v = v * cc; }
+      y[om + i] = v;
+    }
+  }
+}
+// Qx = Qd (+ x / gamma_init), Ax = Ad, sigma = clamp(sigma_init max(1, |f|) / max(1, dist2 / 2)) with f = x'Qx / 2 + q'x and
+// dist2 = |Ax - clip(Ax)|^2 (initialize_sigma, iteration.c:50-84)
+__global__ void __launch_bounds__(256)
+kb_warm_sigma(int n, int m, BSet st, const double *__restrict__ x, const double *__restrict__ q, const double *__restrict__ Qd,
+              const double *__restrict__ Ad, const double *__restrict__ bmin, const double *__restrict__ bmax, double *Qx, double *Ax,
+              double *sigma, double *sigma_inv, double *sqrt_sigma) {
+  __shared__ double scratch[32];
+  __shared__ double sig_s;
+  const int b = blockIdx.x, tid = threadIdx.x;
+  const size_t on = (size_t)b * n, om = (size_t)b * m;
+  const double inv_g = 1 / st.gamma_init;
+  double xqx = 0.0, qtx = 0.0, dist2 = 0.0;
+  for (int i = tid; i < n; i += blockDim.x) {
+    const double xi = x[on + i];
+    double qx = Qd[on + i];
+    if (st.proximal) qx = qx + inv_g * xi;
+    Qx[on + i] = qx;
+    xqx += xi * qx; qtx += q[on + i] * xi;
+  }
+  for (int i = tid; i < m; i += blockDim.x) {
+    const double ax = Ad[om + i];
+    Ax[om + i] = ax;
+    const double t = ax - fmax(bmin[om + i], fmin(ax, bmax[om + i]));
+    dist2 += t * t;
+  }
+  xqx = block_red<RED_SUM>(xqx, scratch);
+  qtx = block_red<RED_SUM>(qtx, scratch);
+  dist2 = block_red<RED_SUM>(dist2, scratch);
+  if (tid == 0) {
+    const double f = 0.5 * xqx + qtx;
+    sig_s = fmax(1e-4, fmin(st.sigma_init * fmax(1.0, fabs(f)) / fmax(1.0, 0.5 * dist2), 1e4));
+  }
+  __syncthreads();
+  const double s = sig_s;
+  for (int i = tid; i < m; i += blockDim.x) { sigma[om + i] = s; sigma_inv[om + i] = 1.0 / s; sqrt_sigma[om + i] = sqrt(s); }
+}
+
+// ------------------------------------------------------------------------------------------------
 // residual step (compute_residuals + candidate active set + termination reductions), one CTA per instance
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
@@ -882,6 +944,7 @@ extern "C" QPALMB200Batch *qpalm_b200_batch_setup(const QPALMData *shared, const
     rc |= iv(p, NB);
   rc |= iv(&B->ndone, 4);
   rc |= iv(&B->queue, 4);
+  rc |= dv(&B->x_ws, NB * N); rc |= dv(&B->y_ws, NB * M);
   if (getenv("QPALM_B200_BATCH_PROF")) rc |= dev_alloc((void **)&B->prof, sizeof(long long) * 32 * NB);
   if (const char *env = getenv("QPALM_B200_BATCH_ENGINE")) {   // tests / profiling: force one engine
     if (!strcmp(env, "lockstep")) B->engine = 1; else if (!strcmp(env, "persistent")) B->engine = 2;
@@ -905,6 +968,19 @@ extern "C" int qpalm_b200_batch_upload(QPALMB200Batch *B, c_int nb_, const c_flo
   return 0;
 }
 
+extern "C" int qpalm_b200_batch_warm_start(QPALMB200Batch *B, c_int nb_, const c_float *x_ws, const c_float *y_ws) {
+  if (!B) return 1;
+  if (!x_ws && !y_ws) { B->ws_nb = 0; B->ws_x = 0; B->ws_y = 0; return 0; }
+  const int nb = (int)nb_;
+  if (nb <= 0 || nb > B->nb_max) return 1;
+  B->ws_nb = 0; B->ws_x = 0; B->ws_y = 0;   // the buffers are being overwritten: no half-copied warm start stays pending
+  if (x_ws) QB_CUDA_TRY(cudaMemcpyAsync(B->x_ws, x_ws, sizeof(double) * (size_t)nb * B->n, cudaMemcpyHostToDevice, B->stream));
+  if (y_ws && B->m > 0) QB_CUDA_TRY(cudaMemcpyAsync(B->y_ws, y_ws, sizeof(double) * (size_t)nb * B->m, cudaMemcpyHostToDevice, B->stream));
+  QB_CUDA_TRY(cudaStreamSynchronize(B->stream));
+  B->ws_nb = nb; B->ws_x = x_ws != nullptr; B->ws_y = y_ws != nullptr;
+  return 0;
+}
+
 extern "C" int qpalm_b200_batch_solve_resident(QPALMB200Batch *B, c_int nb_, double *device_ms) {
   const int nb = (int)nb_;
   if (!B || nb <= 0 || nb > B->nb_max) return 1;
@@ -915,6 +991,9 @@ extern "C" int qpalm_b200_batch_solve_resident(QPALMB200Batch *B, c_int nb_, dou
   const long long sLL = (long long)ld * npad, sX = (long long)npad * kPanel, sW = (long long)ld * B->wcols;
   const long long launches0 = g_kernel_launches;
   const int gnb = cdiv(nb, 128);
+  // a pending warm start is consumed by this solve (qpalm_solve resets `initialized` the same way)
+  const int nwarm = B->ws_nb < nb ? B->ws_nb : nb, wx = B->ws_x, wy = B->ws_y;
+  B->ws_nb = 0; B->ws_x = 0; B->ws_y = 0;
   // engine choice: the persistent one-CTA-per-instance kernel (batchp.cu) when the shapes fit its shared-memory plan,
   // else the lock-step engine below
   const bool persistent = (B->engine == 2) || (B->engine == 0 && batchp_supported(n, m));
@@ -929,7 +1008,7 @@ extern "C" int qpalm_b200_batch_solve_resident(QPALMB200Batch *B, c_int nb_, dou
     if (shape_env && shape_env[0] == '3') four = false;
     if (shape_env && shape_env[0] == '4') four = true;
     if (four && !batchp4_supported(n, m)) four = false;
-    if (int r = four ? batchp4_solve(B, nb) : batchp_solve(B, nb)) return r;
+    if (int r = four ? batchp4_solve(B, nb, nwarm, wx, wy) : batchp_solve(B, nb, nwarm, wx, wy)) return r;
     QB_CUDA_TRY(cudaEventRecord(B->ev1, s));
     QB_CUDA_TRY(cudaEventSynchronize(B->ev1));
     float msp = 0; cudaEventElapsedTime(&msp, B->ev0, B->ev1);
@@ -946,6 +1025,18 @@ extern "C" int qpalm_b200_batch_solve_resident(QPALMB200Batch *B, c_int nb_, dou
   QB_LAUNCH(kb_init, nb, 256, 0, s, n, m, st, e->D, e->E, B->q_raw, B->bmin_raw, B->bmax_raw, B->q, B->bmin, B->bmax, B->x, B->y, B->Ax,
             B->Qx, B->Aty, B->x_prev, B->x0, B->sigma, B->sigma_inv, B->sqrt_sigma, B->Qd, B->Ad, B->d, B->pri_res_in, B->active,
             B->active_old, B->activeH, B->scal, B->ctl);
+  if (nwarm && (wx || wy)) {
+    QB_LAUNCH(kb_warm_set, nwarm, 256, 0, s, n, m, st, e->Dinv, e->Einv, wx ? B->x_ws : nullptr, wy ? B->y_ws : nullptr, B->ctl,
+              B->x, B->x0, B->x_prev, B->y);
+    if (wx) {
+      QB_LAUNCH(kb_gemv_rows, dim3(cdiv(n, 256), nwarm), 256, sizeof(double) * n, s, n, n, n, B->Qs, B->x, (long long)n, B->Qd,
+                (long long)n, B->ctl, (const int *)nullptr, 1);
+      if (m > 0) QB_LAUNCH(kb_gemv_cols, dim3(cdiv(m, 8), nwarm), 256, sizeof(double) * n, s, n, m, n, e->At, B->x, (long long)n, B->Ad,
+                           (long long)m, B->ctl, (const int *)nullptr);
+      QB_LAUNCH(kb_warm_sigma, nwarm, 256, 0, s, n, m, st, B->x, B->q, B->Qd, B->Ad, B->bmin, B->bmax, B->Qx, B->Ax, B->sigma,
+                B->sigma_inv, B->sqrt_sigma);
+    }
+  }
   const dim3 tri_grid(cdiv(npad, 256), npad, nb);
   for (int it = 0; it <= st.max_iter; it++) {
     // ---- residuals + termination scalars ----
@@ -1189,7 +1280,7 @@ extern "C" void qpalm_b200_batch_cleanup(QPALMB200Batch *B) {
                   B->Qd, B->Ad, B->vpad, B->active, B->active_old, B->active_cand, B->activeH, B->list_pos, B->list_neg, B->sigmaH, B->w_pos,
                   B->w_neg, B->Kpos, B->Kneg, B->H, B->L, B->invdiag, B->W, B->keys, B->vals, B->ls_da, B->ls_db, B->scal, B->ctl,
                   B->mask_outer, B->mask_sigma, B->mask_inner, B->mask_refac, B->mask_factor, B->mask_scratch, B->mask_fq, B->mask_boost,
-                  B->ndone, B->info, B->queue, B->prof, B->Am};
+                  B->ndone, B->info, B->queue, B->prof, B->Am, B->x_ws, B->y_ws};
   for (void *p : ptrs) if (p) cudaFree(p);
   if (B->ndone_host) cudaFreeHost(B->ndone_host);
   if (B->ev0) cudaEventDestroy(B->ev0);

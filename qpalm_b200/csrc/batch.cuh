@@ -63,15 +63,20 @@ struct QPALMB200Batch {
   int last_engine = 0;
   int last_shape = 0;          // CTA shape of the last solve: 0 lock-step, 3 or 4 persistent (CTAs per SM)
   long long *prof = nullptr;   // persistent engine: optional per-phase clock totals [nb][16]
+  // pending warm start of the next solve (qpalm_b200_batch_warm_start): unscaled rows [nb_max][n] / [nb_max][m]; instances
+  // b < ws_nb start from them, the part whose flag is 0 starts cold
+  double *x_ws = nullptr, *y_ws = nullptr;
+  int ws_nb = 0, ws_x = 0, ws_y = 0;
 };
 
 namespace qb {
 // persistent engine (batchp.cu): true when the shapes fit its shared-memory plan
 bool batchp_supported(int n, int m);
-int batchp_solve(QPALMB200Batch *B, int nb);
+// nwarm: instances b < nwarm start from B->x_ws (when wx) / B->y_ws (when wy), the others cold
+int batchp_solve(QPALMB200Batch *B, int nb, int nwarm, int wx, int wy);
 // the same engine compiled in its 4-CTAs-per-SM shape (batchp.cu with -DQB_BP_VARIANT4)
 bool batchp4_supported(int n, int m);
-int batchp4_solve(QPALMB200Batch *B, int nb);
+int batchp4_solve(QPALMB200Batch *B, int nb, int nwarm, int wx, int wy);
 
 // test probes of the persistent engine's in-CTA building blocks (device pointers; qpalm_b200_batchp_probe_* in batch.cu).
 // Per instance b: H0 is n x n (lds = n) at H0 + b n n, or with from_q the one shared matrix H0 scaled by sscale; cnt[4 b ..] =

@@ -117,6 +117,8 @@ struct Args {
   BCtl *ctl;
   int *queue;
   long long *prof;   // optional [nb][16] per-phase clock64 totals (QPALM_B200_BATCH_PROF=1)
+  int nwarm;                         // instances b < nwarm start from the rows of x_ws / y_ws (either may be null: that part cold)
+  const double *x_ws, *y_ws;         // unscaled, [nb][n] / [nb][m]
 };
 
 struct Flags { int outer, sigma, inner, refac, factor, fq, boost, done, updown; };
@@ -373,6 +375,60 @@ __device__ __forceinline__ void p_gemv_cols(int len, int ncols, int ld, const do
       if (lane == 0 && col0 + u < ncols) out[col0 + u] = r;
     }
   }
+}
+
+// warm start of instance b after p_init's cold start (qpalm_warm_start, qpalm.c:322-399, then initialize_sigma,
+// iteration.c:50-84), in the engine's scaled storage: x = Dinv x_ws, y = c Einv y_ws, Qd = c (D Q D) x, Qx = Qd (+ x / gamma_init),
+// Ad = Ax = A x, sigma from f = x'Qx / 2 + q'x and the bound distance of Ax.  Aty, d, the active sets and the control state
+// keep their cold values, as a fresh setup leaves them.  Without x, Qx = Ax = 0 and the cold sigma stands.
+__device__ __noinline__ void p_warm(const Args &P, int b, double *scratch, const Smem &S) {
+  __shared__ double sig_s;
+  const int n = P.n, m = P.m, tid = threadIdx.x;
+  const BSet &st = P.st;
+  const size_t on = (size_t)b * n, om = (size_t)b * m;
+  const double cc = P.ctl[b].c;
+  if (P.y_ws)
+    for (int i = tid; i < m; i += NT) {
+      double v = P.y_ws[om + i];
+      if (st.scaling) { v = v * P.Einv[i]; v = v * cc; }
+      P.y[om + i] = v;
+    }
+  if (!P.x_ws) return;
+  for (int i = tid; i < n; i += NT) {
+    double v = P.x_ws[on + i];
+    if (st.scaling) v = v * P.Dinv[i];
+    P.x[on + i] = v; P.x0[on + i] = v; P.x_prev[on + i] = v;
+  }
+  __syncthreads();
+  p_gemv_rows(n, n, n, P.Qs, P.x + on, P.Qd + on, cc, S);
+  __syncthreads();
+  p_gemv_rows(m, n, m, P.Am, P.x + on, P.Ad + om, 1.0, S);
+  __syncthreads();
+  const double inv_g = 1 / st.gamma_init;
+  double xqx = 0.0, qtx = 0.0, dist2 = 0.0;
+  for (int i = tid; i < n; i += NT) {
+    const double xi = P.x[on + i];
+    double qx = P.Qd[on + i];
+    if (st.proximal) qx = qx + inv_g * xi;
+    P.Qx[on + i] = qx;
+    xqx += xi * qx; qtx += P.q[on + i] * xi;
+  }
+  for (int i = tid; i < m; i += NT) {
+    const double ax = P.Ad[om + i];
+    P.Ax[om + i] = ax;
+    const double t = ax - fmax(P.bmin[om + i], fmin(ax, P.bmax[om + i]));
+    dist2 += t * t;
+  }
+  xqx = block_red<RED_SUM>(xqx, scratch);
+  qtx = block_red<RED_SUM>(qtx, scratch);
+  dist2 = block_red<RED_SUM>(dist2, scratch);
+  if (tid == 0) {
+    const double f = 0.5 * xqx + qtx;
+    sig_s = fmax(1e-4, fmin(st.sigma_init * fmax(1.0, fabs(f)) / fmax(1.0, 0.5 * dist2), 1e4));
+  }
+  __syncthreads();
+  const double s = sig_s;
+  for (int i = tid; i < m; i += NT) { P.sigma[om + i] = s; P.sigma_inv[om + i] = 1.0 / s; P.sqrt_sigma[om + i] = sqrt(s); }
 }
 
 __device__ __noinline__ void p_res_n(const Args &P, int b, double *part) {
@@ -1691,6 +1747,7 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_solve(const Args P) {
     if (P.prof && tid == 0) for (int k = 0; k < 32; k++) P.prof[(size_t)b * 32 + k] = 0;
     p_init(P, b, scratch);
     __syncthreads();
+    if (b < P.nwarm) { p_warm(P, b, scratch, S); __syncthreads(); }
     PH(0);
     for (;;) {
       // ---- residuals + termination scalars ----
@@ -1942,7 +1999,7 @@ bool QB_BP_SUPPORTED(int n, int m) {
   return n >= 1 && n <= QB_BP_NAMESPACE::NMAX && m >= 1 && 2 * m <= QB_BP_NAMESPACE::SORT_MAX && m <= QB_BP_NAMESPACE::VS_LEN;
 }
 
-int QB_BP_SOLVE(QPALMB200Batch *B, int nb) {
+int QB_BP_SOLVE(QPALMB200Batch *B, int nb, int nwarm, int wx, int wy) {
   using namespace QB_BP_NAMESPACE;
   Engine *e = B->shared;
   Args P;
@@ -1959,6 +2016,7 @@ int QB_BP_SOLVE(QPALMB200Batch *B, int nb) {
   P.H = B->H; P.L = B->L; P.rdiag = B->invdiag;
   P.sLL = (long long)B->ld * B->npad; P.sR = (long long)B->npad * kPanel;
   P.prof = B->prof;
+  P.nwarm = nwarm; P.x_ws = wx ? B->x_ws : nullptr; P.y_ws = wy ? B->y_ws : nullptr;
   P.keys = B->keys; P.vals = B->vals; P.ls_da = B->ls_da; P.ls_db = B->ls_db; P.scal = B->scal; P.ctl = B->ctl; P.queue = B->queue;
   static int ctas_per_sm = 0, num_sms = 0;
   if (!ctas_per_sm) {

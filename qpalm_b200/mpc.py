@@ -30,6 +30,22 @@ def mpc_sequence(steps: int, n: int = 240, m0: int = 709, seed: int = 0, drift: 
     return b, seq
 
 
+def batch_sequence(nb: int, steps: int, n: int = 240, m0: int = 709, seed: int = 0, drift: float = 0.01):
+    """The batch form of mpc_sequence: a chain80w-sized BatchQP of nb instances and, per step, the (q, bmin, bmax) arrays
+    (nb x n, nb x m, nb x m) of all instances.  Every instance drifts as mpc_sequence's does, from its own PRNG stream."""
+    b = problems.mpc_batch(nb, n=n, m0=m0, seed=seed)
+    rngs = [np.random.default_rng([seed + 12345, k]) for k in range(nb)]
+    q, lo, hi = b.q.copy(), b.bmin.copy(), b.bmax.copy()
+    seq = []
+    for _ in range(steps):
+        for k, rng in enumerate(rngs):
+            q[k] = q[k] + drift * rng.standard_normal(q.shape[1])
+            shift = drift * rng.standard_normal(lo.shape[1])
+            lo[k], hi[k] = lo[k] + shift, hi[k] + shift
+        seq.append((q.copy(), lo.copy(), hi.copy()))
+    return b, seq
+
+
 def run_sequence(impl: str, b, seq, warm: bool = True, **settings):
     """Returns (results, seconds per step) of the warm-started loop on one workspace."""
     s = Qpalm(impl)
