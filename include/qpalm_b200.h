@@ -361,6 +361,9 @@ int  qpalm_b200_batch_warm_start(QPALMB200Batch *batch, c_int nb, const c_float 
  * sum of |J| over the refactorisations, engine (1 lock-step, 2 persistent), rank-k update sweeps, sum of their ranks,
  * downdates that lost definiteness (followed by a refactorisation)} -- inputs of the SURVEY 8(d) byte model */
 int  qpalm_b200_batch_stats(QPALMB200Batch *batch, c_int nb, double *out8);
+/* persistent engine, totals of the last solve over instances 0..nb-1: out2 = {rows of A streamed through the H SYRK, summed
+ * over the refactorisations; refactorisations that rebuilt H from c Q} (zeros after a lock-step solve) */
+int  qpalm_b200_batch_syrk_stats(QPALMB200Batch *batch, c_int nb, double *out2);
 /* persistent engine, QPALM_B200_BATCH_PROF=1 at setup: per-instance SM-clock totals of 16 phases of the last solve */
 int  qpalm_b200_batch_phase_profile(QPALMB200Batch *batch, c_int nb, long long *out);
 long long qpalm_b200_batch_last_launches(const QPALMB200Batch *batch);   /* kernels launched by the last solve */

@@ -32,6 +32,8 @@ def _lib():
         lib.qpalm_b200_batch_last_shape.restype = C.c_int
         lib.qpalm_b200_batch_stats.argtypes = [C.c_void_p, abi.c_int, c_float_p]
         lib.qpalm_b200_batch_stats.restype = C.c_int
+        lib.qpalm_b200_batch_syrk_stats.argtypes = [C.c_void_p, abi.c_int, c_float_p]
+        lib.qpalm_b200_batch_syrk_stats.restype = C.c_int
         lib.qpalm_b200_batch_cleanup.argtypes = [C.c_void_p]
         lib.qpalm_b200_batch_cleanup.restype = None
         lib._batch_typed = True
@@ -128,9 +130,13 @@ class Batch:
         out = np.zeros(8)
         if self.lib.qpalm_b200_batch_stats(self.h, nb, fptr(out)):
             raise RuntimeError("batch_stats failed")
+        syrk = np.zeros(2)
+        if self.lib.qpalm_b200_batch_syrk_stats(self.h, nb, fptr(syrk)):
+            raise RuntimeError("batch_syrk_stats failed")
         return dict(inner=out[0], outer=out[1], refactorizations=out[2], refactor_J_sum=out[3],
                     engine={1: "lockstep", 2: "persistent"}.get(int(out[4]), "?"),
-                    updown_sweeps=out[5], updown_rank_sum=out[6], updown_failed=out[7])
+                    updown_sweeps=out[5], updown_rank_sum=out[6], updown_failed=out[7],
+                    syrk_entries=syrk[0], scratch_rebuilds=syrk[1])
 
     def last_launches(self):
         return int(self.lib.qpalm_b200_batch_last_launches(self.h))

@@ -1151,6 +1151,17 @@ extern "C" int qpalm_b200_batch_stats(QPALMB200Batch *B, c_int nb, double *out8)
   return 0;
 }
 
+// persistent engine, totals over the instances of the last solve: [0] rows of A streamed through the H SYRK (summed over the
+// refactorisations), [1] refactorisations that rebuilt H from c Q
+extern "C" int qpalm_b200_batch_syrk_stats(QPALMB200Batch *B, c_int nb, double *out2) {
+  if (!B || nb <= 0 || nb > B->nb_max) return 1;
+  QB_CUDA_TRY(cudaMemcpy(B->ctl_host.data(), B->ctl, sizeof(BCtl) * (size_t)nb, cudaMemcpyDeviceToHost));
+  double e = 0, r = 0;
+  for (c_int b = 0; b < nb; b++) { e += (double)B->ctl_host[b].syrk_entries; r += B->ctl_host[b].n_scratch; }
+  out2[0] = e; out2[1] = r;
+  return 0;
+}
+
 extern "C" int qpalm_b200_batch_phase_profile(QPALMB200Batch *B, c_int nb, long long *out /* nb x 16 */) {
   if (!B || !B->prof) return 1;
   QB_CUDA_TRY(cudaMemcpy(out, B->prof, sizeof(long long) * 32 * (size_t)nb, cudaMemcpyDeviceToHost));
@@ -1189,7 +1200,7 @@ static int probe_newton(c_int shape, c_int nb_, c_int n_, c_int m_, const c_floa
   for (size_t b = 0; b < NB; b++) {
     const c_int *c = cnt + 4 * b;
     if (c[0] < 0 || c[0] > m || c[1] < 0 || c[1] > m || c[2] < 0 || c[2] > m || c[3] < 0 || c[3] > c[2]) return 1;
-    if (from_q && (c[0] || c[1])) return 1;   // the f.fq path factors the shared matrix itself: no SYRK lists
+    if (c[0] + c[1] > m) return 1;   // one SYRK stream holds both lists: at most m rows, as in the solver
     for (int k = 0; k < 4; k++) cnt_i[4 * b + k] = (int)c[k];
     for (int seg = 0; seg < 3; seg++)
       for (c_int q = 0; q < c[seg]; q++) {

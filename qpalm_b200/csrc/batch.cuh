@@ -17,6 +17,8 @@ struct BCtl {   // per-instance control state (device resident)
   long long refac_J;             // sum of |J| over the refactorisations
   int n_updown, n_updown_fail;   // rank-k update / downdate sweeps taken instead of a refactorisation (and downdates that lost definiteness)
   long long updown_ranks;        // sum of ranks over the sweeps
+  long long syrk_entries;        // persistent engine: rows of A streamed through the H SYRK, summed over the refactorisations
+  int n_scratch;                 // persistent engine: refactorisations that rebuilt H from c Q
 };
 
 struct BSet {   // settings the device needs (copied by value into kernels)
@@ -79,9 +81,10 @@ bool batchp4_supported(int n, int m);
 int batchp4_solve(QPALMB200Batch *B, int nb, int nwarm, int wx, int wy);
 
 // test probes of the persistent engine's in-CTA building blocks (device pointers; qpalm_b200_batchp_probe_* in batch.cu).
-// Per instance b: H0 is n x n (lds = n) at H0 + b n n, or with from_q the one shared matrix H0 scaled by sscale; cnt[4 b ..] =
-// {npos, nneg, nup, kpos}; lists / wts hold 3 m entries per instance: SYRK + rows at [0, m), SYRK - rows at [m, 2 m), update rows
-// at [2 m, 3 m).  H, L: ld x ld per instance, rdiag: ld per instance.  rounds > 0: then 2 rounds more solves per instance into
+// Per instance b: H0 is n x n (lds = n) at H0 + b n n, copied into H before the SYRK updates it in place; or with from_q the one
+// shared matrix H0 scaled by sscale, the base of the SYRK (the solver's rebuild from c Q), and without SYRK lists the matrix the
+// Cholesky factors directly (the solver's f.fq path); cnt[4 b ..] = {npos, nneg, nup, kpos}, npos + nneg <= m; lists / wts hold
+// 3 m entries per instance: SYRK + rows at [0, m), SYRK - rows at [m, 2 m), update rows at [2 m, 3 m).  H, L: ld x ld per instance, rdiag: ld per instance.  rounds > 0: then 2 rounds more solves per instance into
 // d_rounds (nb x 2 rounds x n), see qpalm_b200_batchp_probe_solves.
 struct BpProbeArgs {
   int nb, n, m, ld, from_q, rounds;

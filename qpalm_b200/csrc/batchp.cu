@@ -11,13 +11,13 @@
 // per-instance H / L (n x n lower, column-major) and vectors are touched by one CTA only.  At 512 instances the factors
 // (2 x 230 KB each) do not fit the L2 and stream from HBM, which is why every pass over them is written as a batch of
 // requests (cp.async, eight loads in flight, rows requested one block ahead) rather than load -> use.  Shared memory per CTA
-// (72 KB at 3 CTAs / SM, 55 KB at 4) holds one panel of the factor (Cholesky, triangular solves, SYRK chunks) -- or, during an
+// (72 KB at 3 CTAs / SM, 55 KB at 4) holds one panel of the factor (Cholesky, triangular solves), the SYRK's double-buffered rows of A' -- or, during an
 // update sweep, the rows of W, the chain warp's ring of window blocks and the row owners' staging ring --, the radix-sort
 // buffers of the line search (2m <= 2048 keys) and the staged GEMV operand.
 //
 // The Newton system (Q + A_J' Sigma_J A_J + I/gamma) d = -dphi  (src/newton.c:96-118, solver_interface.c:319-519):
-//   H is kept per instance and updated incrementally (+ entering / - leaving / +- sigma changes) by an in-CTA SYRK in chunks of
-//   one panel width, L <- chol(H + beta I) by an in-CTA right-looking blocked Cholesky (diagonal sub-blocks in one warp's
+//   H is kept per instance and updated incrementally (+ entering / - leaving / +- sigma changes) or rebuilt from c Q by an in-CTA
+//   tile-stationary SYRK (cta_syrk), L <- chol(H + beta I) by an in-CTA right-looking blocked Cholesky (diagonal sub-blocks in one warp's
 //   registers, panel solve one row per thread); SYRK and trailing updates run on the FP64 tensor pipe (mma.sync m8n8k4, 16 x 16
 //   tiles per warp); then two blocked triangular solves.  When the active set changes by at most min(0.1 (n + m),
 //   max_rank_update) rows -- and at most 40, see p_control -- and the factor is current, the factor is UPDATED in place instead
@@ -610,8 +610,8 @@ __device__ __forceinline__ void bp_dmma884(double &d0, double &d1, double a, dou
   asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};" : "+d"(d0), "+d"(d1) : "d"(a), "d"(b));
 }
 
-// dst(i, j) = base(i, j) + sign * sum_{c < w} U[c][i] U[c][j]   for r0 <= j <= i < n   (the SYRK of the H record and the trailing
-// update of the in-CTA Cholesky), base = first ? sscale * src + diag_add I : dst.  U = shared panel, column c at U + c * LDP - u0.
+// dst(i, j) = base(i, j) + sign * sum_{c < w} U[c][i] U[c][j]   for r0 <= j <= i < n   (the trailing update of the in-CTA
+// Cholesky), base = first ? sscale * src + diag_add I : dst.  U = shared panel, column c at U + c * LDP - u0.
 // Round 2: the products run on the FP64 tensor pipe.  Each warp takes 16 x 16 tiles of the lower triangle (2 x 2 DMMA tiles,
 // round-robin over the warps); per 4 columns of U it loads two A and two B fragments from shared memory and issues four
 // mma.sync.m8n8k4 -- a quarter of the shared-memory wavefronts and a sixth of the instructions of the 4 x 4 scalar register
@@ -694,6 +694,8 @@ __device__ __forceinline__ void bp_cp_async8(double *smem_dst, const double *gsr
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(d), "l"(gsrc) : "memory");
 }
 __device__ __forceinline__ void bp_cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
+__device__ __forceinline__ void bp_cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N> __device__ __forceinline__ void bp_cp_async_wait_group() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 // Pn[t][r] <- L(k0 + r, k0 + t) for t <= r < rows, t < w; zeros above the diagonal of the w x w block.  Rows fastest (coalesced).
 // The caller's __syncthreads() publishes the panel.
 __device__ __forceinline__ void panel_load_async(double *Pn, const double *L, int ld, int k0, int w, int rows) {
@@ -854,31 +856,162 @@ __device__ __forceinline__ void cta_potrf(double *L, int ld, const double *src, 
 #undef PQ
 }
 
-// dst(lower) += sign * sum_{c < cnt} (wgt[c] A'[:, list[c]]) (...)'   in chunks of PW list entries staged in the panel
-__device__ __forceinline__ void cta_syrk_list(double *dst, int ld, int n, const double *__restrict__ At, const int *__restrict__ list,
-                              const double *__restrict__ wgt, int cnt, double sign, const Smem &S) {
+// Tile-stationary SYRK of the Newton matrix:
+//   dst(i, j) = base(i, j) + sum_{e < npos} wpos[e]^2 a_e(i) a_e(j) - sum_{e < nneg} wneg[e]^2 a'_e(i) a'_e(j)   for j <= i < n,
+// a_e = A'[:, lpos[e]], a'_e = A'[:, lneg[e]]; base = 0, dst itself, or sscale * src (lds): the zeroed Gershgorin matrix of
+// p_boost, the incremental H record, the rebuild from c Q.  Both lists form ONE stream of signed weights s w^2, applied to the
+// A fragment in registers.  The 16 x 16 tiles of the lower triangle are taken in passes over a group of 4 x 2 tiles (one per
+// warp, its DMMA accumulators in registers) while the whole list streams past in stages of SY_C entries: each tile of dst is
+// read once and written once, which matters because at 512 instances the per-instance H streams from HBM.  A stage
+// holds only the rows of A' its group needs -- 64 rows for a diagonal group, 96 for an off-diagonal one -- gathered with
+// 16-byte cp.async copies of whole 16-row segments (A' is L2-resident) into a double buffer: one barrier per stage.
+constexpr int SY_BI = 4, SY_BJ = 2;               // a tile group: 4 i blocks x 2 j blocks of 16 rows, one tile per warp
+constexpr int SY_LD = (SY_BI + SY_BJ) * 16 + 4;   // 100 rows per staged column: the fragment loads of a half warp hit 16 banks
+constexpr int SY_C = (QB_BP_PW == 32) ? 36 : 24;  // list entries per stage (two stages + the list indices fill the union region)
+static_assert(NW == SY_BI * SY_BJ, "one tile per warp");
+static_assert(2 * SY_C * SY_LD * sizeof(double) + VS_LEN * sizeof(int) <= kUnionBytes, "two stages + the list indices must fit the union region");
+enum { SY_ZERO = 0, SY_DST = 1, SY_SRC = 2 };
+
+__device__ __forceinline__ void bp_cp_async16(double *smem_dst, const double *gsrc) {
+  const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gsrc) : "memory");
+}
+__device__ __forceinline__ double sy_lds(unsigned a) {
+  double v;
+  asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a));
+  return v;
+}
+
+// The job of one cta_syrk call, in shared memory: the loops reload what they need after each barrier, so that little more
+// than the tile's accumulators stays in registers across a stage.  With the arguments in registers, or with one flat loop over
+// (group, stage), ptxas kept the accumulators in local memory around the product loop at 64 and at 80 registers alike.
+struct SyJob {
+  double *dst; const double *src, *At; long long *pf; double sscale;
+  int ld, lds, n, base, cnt, nst, vec16;
+};
+
+// stage `st` of group (gi, gj) into buf: columns c < SY_C = list entries st SY_C + c (entries past the list read column 0 of A'
+// and carry weight 0), rows = the group's j blocks at 16 sl (sl < SY_BJ), its i blocks at 16 (SY_BJ + sl).  Rows >= n are not
+// copied: they only reach tile entries that are never stored.
+__device__ __forceinline__ void sy_gather(double *buf, const SyJob &J, const int *lidx, int st, int gi, int gj) {
+  const bool diag = SY_BJ * gj >= SY_BI * gi;
+  const int per = diag ? SY_BI * 8 : (SY_BI + SY_BJ) * 8;   // 16-byte copies per staged column
+  const int n = J.n, cnt = J.cnt;
+  const double *At = J.At;
+  for (int q = threadIdx.x; q < SY_C * per; q += NT) {
+    const int c = diag ? q / (SY_BI * 8) : q / ((SY_BI + SY_BJ) * 8), r = q - c * per;
+    const int sl = (diag ? SY_BJ : 0) + (r >> 3), h = r & 7;
+    const int row = 16 * (sl < SY_BJ ? SY_BJ * gj + sl : SY_BI * gi + sl - SY_BJ) + 2 * h;
+    if (row < n) {
+      const int e = st * SY_C + c;
+      const double *g = At + (size_t)n * (size_t)(e < cnt ? lidx[e] : 0) + row;
+      double *d = buf + c * SY_LD + 16 * sl + 2 * h;
+      if (J.vec16) bp_cp_async16(d, g);
+      else { bp_cp_async8(d, g); if (row + 1 < n) bp_cp_async8(d + 1, g + 1); }
+    }
+  }
+  bp_cp_async_commit();
+}
+
+__device__ __forceinline__ void cta_syrk(double *dst, int ld, int n, int base, const double *src, int lds, double sscale,
+                                      const double *__restrict__ At, const int *lpos, const double *wpos, int npos, const int *lneg,
+                                      const double *wneg, int nneg, const Smem &S, long long *pf) {
+  __shared__ SyJob J;
   const int tid = threadIdx.x;
-  for (int off = 0; off < cnt; off += PW) {
-    const int w = (cnt - off < PW) ? cnt - off : PW;
-    const int wpad = (w + 3) & ~3;   // the DMMA product loop walks 4 columns at a time: zero the pad columns
-    // gather: thread = row, eight columns (list entries) requested before any is stored -- the one-element-at-a-time form chained
-    // list[c] -> A'[:, list[c]] loads behind an integer division per element
-    for (int i = tid; i < n; i += NT) {
-      for (int c0 = 0; c0 < wpad; c0 += 8) {
-        double v[8];
+  const int cnt = npos + nneg, nst = (cnt + SY_C - 1) / SY_C;
+  if (nst == 0) {   // empty list: dst = base
+    if (base != SY_DST)
+      for (int idx = tid; idx < n * n; idx += NT) {
+        const int j = idx / n, i = idx - j * n;
+        if (i >= j) dst[(size_t)i + (size_t)ld * j] = (base == SY_SRC) ? sscale * src[(size_t)i + (size_t)lds * j] : 0.0;
+      }
+    __syncthreads();
+    return;
+  }
+  double *buf0 = S.panel;
+  int *lidx = reinterpret_cast<int *>(S.panel + 2 * SY_C * SY_LD);
+  double *sw = S.vs;   // signed weights, padded with zeros to nst SY_C entries (runs on into S.v, free during the SYRK)
+  for (int e = tid; e < nst * SY_C; e += NT) {
+    double v = 0.0;
+    if (e < cnt) {
+      const bool p = e < npos;
+      const double w = p ? wpos[e] : wneg[e - npos];
+      lidx[e] = p ? lpos[e] : lneg[e - npos];
+      v = p ? w * w : -(w * w);
+    }
+    sw[e] = v;
+  }
+  if (tid == 0) {
+    J.dst = dst; J.src = src; J.At = At; J.pf = pf; J.sscale = sscale;
+    J.ld = ld; J.lds = lds; J.n = n; J.base = base; J.cnt = cnt; J.nst = nst;
+    J.vec16 = !(n & 1) && !(reinterpret_cast<size_t>(At) & 15);
+  }
+  __syncthreads();
+  const int NGI = (((n + 15) >> 4) + SY_BI - 1) / SY_BI, ngp = (SY_BI / SY_BJ) * NGI * (NGI + 1) / 2;
+  sy_gather(buf0, J, lidx, 0, 0, 0);
+  int gi = 0, gj = 0;
+  for (int gp = 0; gp < ngp; gp++) {
+    const int warp = threadIdx.x >> 5;
+    double acc[2][2][2];   // [a][e][h]: entry (16 ib + 8 a + fr, 16 jb + 8 e + 2 fk + h) of the warp's tile (ib, jb)
 #pragma unroll
-        for (int u = 0; u < 8; u++) {
-          const int c = c0 + u;
-          v[u] = (c < w) ? wgt[off + c] * At[(size_t)i + (size_t)n * list[off + c]] : 0.0;
-        }
+    for (int a = 0; a < 2; a++)
 #pragma unroll
-        for (int u = 0; u < 8; u++) if (c0 + u < wpad) S.panel[(c0 + u) * LDP + i] = v[u];
+      for (int e = 0; e < 2; e++) { acc[a][e][0] = 0.0; acc[a][e][1] = 0.0; }
+    const int nst_ = J.nst;
+    for (int st = 0; st < nst_; st++) {
+      const long long tw = clock64();
+      bp_cp_async_wait_group<0>();
+      __syncthreads();   // this stage is visible; every warp is done with the other buffer
+      if (J.pf) { const long long t_ = clock64(); if (threadIdx.x == NT - 1) atomicAdd(reinterpret_cast<unsigned long long *>(J.pf + 15), (unsigned long long)(t_ - tw)); }
+      const int g = gp * nst_ + st;
+      if (st + 1 < nst_) sy_gather(buf0 + ((g + 1) & 1) * SY_C * SY_LD, J, lidx, st + 1, gi, gj);
+      else if (gp + 1 < ngp) {
+        const bool wrap = SY_BJ * (gj + 1) >= SY_BI * (gi + 1);
+        sy_gather(buf0 + ((g + 1) & 1) * SY_C * SY_LD, J, lidx, 0, wrap ? gi + 1 : gi, wrap ? 0 : gj + 1);
+      }
+      const int lane = threadIdx.x & 31, fr = lane >> 2, fk = lane & 3;
+      if (st + 1 == nst_ && lane < 16 && J.base != SY_ZERO) {   // the tile's base column segments (128 bytes each) into the L2 under the last stage
+        const int i = 16 * (SY_BI * gi + (warp >> 1)), j = 16 * (SY_BJ * gj + (warp & 1)) + lane;
+        if (i < J.n && j < J.n)
+          asm volatile("prefetch.global.L2 [%0];" ::"l"(J.base == SY_DST ? J.dst + (size_t)i + (size_t)J.ld * j : J.src + (size_t)i + (size_t)J.lds * j));
+      }
+      const bool diag = SY_BJ * gj >= SY_BI * gi;
+      const unsigned ub = (unsigned)__cvta_generic_to_shared(buf0 + (g & 1) * SY_C * SY_LD + fk * SY_LD);
+      const unsigned aa = ub + 8u * (unsigned)(16 * (SY_BJ + (warp >> 1)) + fr);
+      const unsigned ab = ub + 8u * (unsigned)(16 * (diag ? SY_BJ + SY_BJ * gj - SY_BI * gi + (warp & 1) : (warp & 1)) + fr);
+      const unsigned wk = (unsigned)__cvta_generic_to_shared(S.vs + st * SY_C + fk);
+#pragma unroll 3
+      for (int kc = 0; kc < SY_C; kc += 4) {
+        const unsigned o = (unsigned)(kc * SY_LD * 8);
+        const double s_ = sy_lds(wk + 8u * kc);
+        const double fa0 = sy_lds(aa + o) * s_, fa1 = sy_lds(aa + o + 64) * s_;
+        const double fb0 = sy_lds(ab + o), fb1 = sy_lds(ab + o + 64);
+        bp_dmma884(acc[0][0][0], acc[0][0][1], fa0, fb0);
+        bp_dmma884(acc[0][1][0], acc[0][1][1], fa0, fb1);
+        bp_dmma884(acc[1][0][0], acc[1][0][1], fa1, fb0);
+        bp_dmma884(acc[1][1][0], acc[1][1][1], fa1, fb1);
       }
     }
-    __syncthreads();
-    cta_rank_update_lower(dst, ld, nullptr, 0, 0.0, 0.0, false, 0, n, S.panel, 0, w, sign);
-    __syncthreads();
+    {   // H(tile) <- base + the stream's sum: each tile of dst is read once and written once
+      const int lane = threadIdx.x & 31, fr = lane >> 2, fk = lane & 3, n_ = J.n, base_ = J.base;
+      const int ib = SY_BI * gi + (warp >> 1), jb = SY_BJ * gj + (warp & 1);
+#pragma unroll
+      for (int a = 0; a < 2; a++)
+#pragma unroll
+        for (int e = 0; e < 2; e++)
+#pragma unroll
+          for (int h = 0; h < 2; h++) {
+            const int i = 16 * ib + 8 * a + fr, j = 16 * jb + 8 * e + 2 * fk + h;
+            if (i < n_ && j <= i) {
+              double *d = J.dst + (size_t)i + (size_t)J.ld * j;
+              const double v = (base_ == SY_DST) ? *d : ((base_ == SY_SRC) ? J.sscale * J.src[(size_t)i + (size_t)J.lds * j] : 0.0);
+              *d = v + acc[a][e][h];
+            }
+          }
+    }
+    if (SY_BJ * (gj + 1) >= SY_BI * (gi + 1)) { gi++; gj = 0; } else gj++;
   }
+  __syncthreads();   // the stages and weights are free for the caller
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -925,8 +1058,6 @@ __device__ __forceinline__ void ud_mbar_wait(unsigned long long *bar, unsigned p
   asm volatile("{\n.reg .pred p;\nWAIT_%=:\nmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n@p bra DONE_%=;\nbra WAIT_%=;\nDONE_%=:\n}\n" ::"r"(a), "r"(parity) : "memory");
 #endif
 }
-__device__ __forceinline__ void bp_cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void bp_cp_async_wait_group() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 // chain warp: request the 32 x 16 window block at (k0, k0) -- lane = row k0 + lane, columns c <= lane -- into Pb[c * PBL + lane]
 __device__ __forceinline__ void ud_block_prefetch(double *Pb, const double *L, int ld, int k0, int n, int lane) {
@@ -1422,6 +1553,7 @@ __device__ __noinline__ void p_lists(const Args &P, int b, int refac) {
   if (tid == 0) {
     BCtl &c = P.ctl[b];
     c.npos = base0; c.nneg = base1; c.H_valid = 1; c.scratch = scratch_mode;
+    c.syrk_entries += base0 + base1; c.n_scratch += scratch_mode;
   }
 }
 
@@ -1481,10 +1613,7 @@ __device__ __noinline__ void p_boost(const Args &P, int b, double *scratch, cons
     __syncthreads();
     double *Lb = P.L + (size_t)b * P.sLL;
     const int ld = P.ld;
-    for (int idx = tid; idx < n * n; idx += NT) { const int j = idx / n, i = idx - j * n; if (i >= j) Lb[(size_t)i + (size_t)ld * j] = 0.0; }
-    __syncthreads();
-    cta_syrk_list(Lb, ld, n, P.At, P.list_pos + om, P.w_pos + om, P.ctl[b].npos, 1.0, S);
-    __syncthreads();
+    cta_syrk(Lb, ld, n, SY_ZERO, nullptr, 0, 0.0, P.At, P.list_pos + om, P.w_pos + om, P.ctl[b].npos, nullptr, nullptr, 0, S, nullptr);
     double ub = -1.0e300;
     for (int i = tid; i < n; i += NT) {   // Gershgorin: |row i| of the symmetric matrix
       double acc = 0.0;
@@ -1798,22 +1927,9 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_solve(const Args P) {
         __syncthreads();
         PH(5);
         if (refac) {
-          const BCtl c = P.ctl[b];
-          if (c.scratch) {
-            for (int i = tid; i < n; i += NT) {   // H <- c Q (lower): thread = row, eight columns in flight
-              for (int j0 = 0; j0 <= i; j0 += 8) {
-                double v[8];
-#pragma unroll
-                for (int u = 0; u < 8; u++) v[u] = (j0 + u <= i) ? P.Qs[(size_t)i + (size_t)n * (j0 + u)] : 0.0;
-#pragma unroll
-                for (int u = 0; u < 8; u++) if (j0 + u <= i) Hb[(size_t)i + (size_t)ld * (j0 + u)] = v[u] * c.c;
-              }
-            }
-            __syncthreads();
-          }
-          for (int pass = 0; pass < 2; pass++)   // + entering / grown sigma, then - leaving (one inlined copy of the SYRK)
-            cta_syrk_list(Hb, ld, n, P.At, (pass ? P.list_neg : P.list_pos) + om, (pass ? P.w_neg : P.w_pos) + om,
-                          pass ? c.nneg : c.npos, pass ? -1.0 : 1.0, S);
+          const BCtl c = P.ctl[b];   // scratch: H <- c Q + the lists, else H += / -= the lists
+          cta_syrk(Hb, ld, n, c.scratch ? SY_SRC : SY_DST, P.Qs, n, c.c, P.At, P.list_pos + om, P.w_pos + om, c.npos, P.list_neg + om,
+                   P.w_neg + om, c.nneg, S, P.prof ? P.prof + (size_t)b * 32 : nullptr);
         }
         PH(6);
         for (int i = tid; i < n; i += NT) S.v[i] = P.dphi[on + i] * -1;
@@ -1912,23 +2028,20 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_probe_newton(const BpProbe
     const double *wt = P.wts + (size_t)b * 3 * m;
     const double *src = P.from_q ? P.H0 : P.H0 + (size_t)b * n * n;
     const double sc = P.from_q ? P.sscale : 1.0;
-    for (int i = tid; i < n; i += NT) {   // H <- sc * src (lower), kbp_solve's scratch copy of c Q
-      for (int j0 = 0; j0 <= i; j0 += 8) {
-        double v[8];
-#pragma unroll
-        for (int u = 0; u < 8; u++) v[u] = (j0 + u <= i) ? src[(size_t)i + (size_t)n * (j0 + u)] : 0.0;
-#pragma unroll
-        for (int u = 0; u < 8; u++) if (j0 + u <= i) Hb[(size_t)i + (size_t)ld * (j0 + u)] = v[u] * sc;
-      }
+    if (P.from_q)   // kbp_solve's rebuild: H <- sscale Q + the lists
+      cta_syrk(Hb, ld, n, SY_SRC, P.H0, n, sc, P.At, lst, wt, npos, lst + m, wt + m, nneg, S, nullptr);
+    else {          // the incremental form: H <- H0, then H += / -= the lists in place
+      for (int i = tid; i < n; i += NT)
+        for (int j = 0; j <= i; j++) Hb[(size_t)i + (size_t)ld * j] = src[(size_t)i + (size_t)n * j];
+      __syncthreads();
+      cta_syrk(Hb, ld, n, SY_DST, nullptr, 0, 0.0, P.At, lst, wt, npos, lst + m, wt + m, nneg, S, nullptr);
     }
-    __syncthreads();
-    for (int pass = 0; pass < 2; pass++)
-      cta_syrk_list(Hb, ld, n, P.At, lst + pass * m, wt + pass * m, pass ? nneg : npos, pass ? -1.0 : 1.0, S);
     for (int i = tid; i < n; i += NT) S.v[i] = P.rhs[on + i];
     __syncthreads();
     if (tid == 0) s_info = 0;
-    // from_q: the f.fq path, the factor reads the shared source (lds = n) directly; else the refactorisation of H (lds = ld)
-    cta_potrf(Lb, ld, P.from_q ? P.H0 : Hb, P.from_q ? n : ld, sc, P.beta, n, rdg, S, &s_info, nullptr);
+    // from_q without lists: the f.fq path, the factor reads the shared source (lds = n) directly; else the refactorisation of H
+    const bool fq = P.from_q && npos + nneg == 0;
+    cta_potrf(Lb, ld, fq ? P.H0 : Hb, fq ? n : ld, fq ? sc : 1.0, P.beta, n, rdg, S, &s_info, nullptr);
     cta_chol_solve(Lb, ld, n, rdg, S, s_udbar, ud_phase, nullptr);
     for (int i = tid; i < n; i += NT) P.d_fused[on + i] = S.v[i];
     __syncthreads();

@@ -20,14 +20,17 @@ assert h.lib.qpalm_b200_batch_phase_profile(h.h, nb, out.ctypes.data) == 0
 x, y, infos = h.download(nb)
 iters = np.array([i["iter"] for i in infos])
 names = ["init", "res_m", "gemv_Atyh", "res_n+control", "outer/sigma/boost", "lists", "H syrk", "potrf", "solve", "gemv Qd+Ad",
-         "ls_build", "sort", "select+update", "gemv Qd", "rank-k update sweeps", "", "potrf: panel load", "potrf: diag16", "potrf: solve16", "potrf: update16",
+         "ls_build", "sort", "select+update", "gemv Qd", "rank-k update sweeps", "H syrk: A' gather + stage wait", "potrf: panel load", "potrf: diag16", "potrf: solve16", "potrf: update16",
          "potrf: store", "potrf: trailing", "sweep: gather W", "sweep chain warp: block prologue", "sweep: whole block loop (row owner's clock)", "sweep chain warp: column loop",
          "sweep chain warp: block epilogue", "sweep chain warp: wait for the row owners",
          "solve fwd chain warp: column loop", "solve fwd chain warp: block ends + window waits",
          "solve bwd chain warp: column loop", "solve bwd chain warp: block ends + window waits"]
-tot = out[:, :16].sum(axis=1)
+tot = out[:, :15].sum(axis=1)   # slots 15 .. 31 split phases 6 .. 8 and 14
 print(f"nb={nb} solve {ms:.2f} ms; mean iters {iters.mean():.1f} max {iters.max()}; mean clocks/instance {tot.mean():.3e} ({tot.mean()/1.965e3:.0f} us)")
 st = h.stats(nb)
 print(f"per instance: refactorizations {st['refactorizations']/nb:.1f}, update sweeps {st['updown_sweeps']/nb:.1f} (ranks {st['updown_rank_sum']/nb:.1f}, failed {st['updown_failed']/nb:.2f}), inner {st['inner']/nb:.1f}")
-for k in list(range(15)) + list(range(16, 32)):
+nr = max(st["refactorizations"], 1)
+print(f"H syrk: {st['syrk_entries']/nr:.1f} list entries per refactorization, scratch rebuilds {st['scratch_rebuilds']/nb:.1f} "
+      f"per instance ({100*st['scratch_rebuilds']/nr:.0f}% of the refactorizations)")
+for k in list(range(32)):
     print(f"{names[k]:22s} {out[:,k].mean()/1.965e3:10.1f} us/instance  {100*out[:,k].sum()/tot.sum():6.2f}%   per-iter {out[:,k].sum()/iters.sum()/1.965e3:7.2f} us")
