@@ -296,9 +296,9 @@ int qpalm_b200_lobpcg(const solver_sparse *Q, const c_float *x0, c_float *lambda
  * C(n x n lower) = W W' with W n x k; returns the average ms per call over `reps` calls. */
 int qpalm_b200_bench_dsyrk(c_int n, c_int k, c_int reps, double *ms_out);
 int qpalm_b200_bench_potrf(c_int n, c_int reps, double *ms_out);
-/* one rank-k dataflow sweep (updown_flow.cu) on an n x n factor, k <= 64: average ms per sweep */
+/* one rank-k update or downdate of an n x n factor as the solver runs it (updown_gen.cu: generator-form passes, <= 32
+ * columns each, each followed by the refresh of the inverted diagonal blocks), k >= 1: average ms per update or downdate */
 int qpalm_b200_bench_updown(c_int n, c_int k, c_int reps, double *ms_out);
-int qpalm_b200_bench_updown_clocks(c_int n, c_int k, long long *out32);
 /* FP64 tensor-pipe (DMMA) issue-rate peak in TFLOP/s: register-resident mma.sync chains, no memory traffic. */
 int qpalm_b200_bench_dmma_peak(double *tflops_out);
 /* scalar FP64 FMA (DFMA) issue-rate peak in TFLOP/s, same method: the bound of the kernels that use plain fma() */

@@ -400,15 +400,13 @@ static bool prefer_updown(const Engine *e, int k) {
   if (k <= 0) return false;
   if (e->kkt) return false;   // KKT path: a changed row is rewritten and the system refactorised (kkt.cu)
   if (e->updown_max_rank == 0) return false;   // QPALM_B200_UPDOWN_MAX_RANK=0: always refactorise, whatever the update path
-  const bool flow = !e->sp && e->updown_flow_ok && e->npad >= 256;   // one-launch dataflow sweep, <= 64 ranks each (updown_flow.cu)
-  const bool gen = use_updown_gen(e);                                // generator-form passes, <= 32 ranks each (updown_gen.cu)
-  if (gen) {
+  if (use_updown_gen(e)) {   // generator-form passes, <= 32 ranks each (updown_gen.cu)
     if (e->updown_force) return true;
     // STATIC model again: per pass a chain of npad/128 block steps of the k-column triangular solve (step time set by the
     // 128 x 128 x k products of one SM), the tile-parallel apply pass over the factor, the small generator kernels and the
     // refresh of the inverted diagonal blocks.  Measured on B200, see DESIGN.md section 4.
     // pass time (ms) = a * (npad / 128) + b * (npad / 8064)^2 + c, fitted to the measured passes at npad = 1024 and 8064:
-    //   <= 8 columns 0.11 / 0.48 ms, <= 16 columns 0.13 / 0.56 ms, <= 32 columns 0.17 / 0.95 ms  (the dataflow sweep: 0.43 / 3.2 ms)
+    //   <= 8 columns 0.11 / 0.48 ms, <= 16 columns 0.13 / 0.56 ms, <= 32 columns 0.17 / 0.95 ms
     const double nblk = e->npad / 128.0, sz = (e->npad / 8064.0) * (e->npad / 8064.0);
     const double pass8 = 0.0030 * nblk + 0.21 * sz + 0.085, pass16 = 0.0035 * nblk + 0.25 * sz + 0.09, pass32 = 0.0065 * nblk + 0.42 * sz + 0.12;
     const int full = k / 32, rem = k % 32;
@@ -416,8 +414,8 @@ static bool prefer_updown(const Engine *e, int k) {
     const double t_rf = (e->npad / 128.0) * 0.12 + ((double)e->n * e->n * e->n / 3.0) / 25e9;
     return t_ud < t_rf;
   }
-  if (e->sh_world > 1 && !flow) return false;   // row-sharded: only the dataflow path allreduces the gathered rows
-  if (!flow && k > (e->sp ? 8 * e->updown_max_rank : e->updown_max_rank)) return false;
+  if (e->sh_world > 1) return false;   // row-sharded factor without the generator form: refactorise
+  if (k > (e->sp ? 8 * e->updown_max_rank : e->updown_max_rank)) return false;
   if (e->updown_force) return true;
   if (e->sp) {
     // Sparse factor: a STATIC rule as well (round 1 compared measured times here, which made re-solves irreproducible).  A sweep
@@ -433,15 +431,6 @@ static bool prefer_updown(const Engine *e, int k) {
   // problems (tests/src/test_dua_inf_qp.c) round alike.
   if (e->npad <= 128) return true;
   const double t_rf = (e->npad / 128.0) * 0.12 + ((double)e->n * e->n * e->n / 3.0) / 25e9;      // ms: panel chain + DMMA flops
-  if (flow) {
-    // the sweep is a chain of npad/32 panel steps whose length does not depend on the rank (<= 64 columns per sweep),
-    // plus the refresh of the inverted diagonal blocks
-    // (measured on B200: 13.5 us per panel in the 32-column shape, 17.9 us in the 64-column shape)
-    const int full = k / 64, rem = k % 64;
-    const double per_panel = full * e->updown_panel_ms64 + (rem > 32 ? e->updown_panel_ms64 : (rem > 0 ? e->updown_panel_ms : 0.0));
-    const double t_ud = (e->npad / 32.0) * per_panel + 0.08;
-    return t_ud < t_rf;
-  }
   const double t_ud = (e->npad / 32.0) * (0.060 + 0.008 * k);                                   // ms, B200 (measured 83 us per 32-column panel step at n = 8000)
   return t_ud < t_rf;
 }

@@ -7,7 +7,7 @@ NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 FLAGS="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC -fmad=false $QB_EXTRA_FLAGS"
 mkdir -p build
 pids=()
-for f in dense updown_flow updown_gen kernels api ops compat kkt batch batchp prof shard sparse sparse_sym qps; do
+for f in dense updown_gen kernels api ops compat kkt batch batchp prof shard sparse sparse_sym qps; do
   if [ ! -f build/$f.o ] || [ $f.cu -nt build/$f.o ] || [ engine.cuh -nt build/$f.o ] || [ dense.cuh -nt build/$f.o ] || [ common.cuh -nt build/$f.o ] || [ batch.cuh -nt build/$f.o ] || [ sparse.cuh -nt build/$f.o ] || [ sparse_host.h -nt build/$f.o ] || [ chol32.cuh -nt build/$f.o ] || [ ../../include/qpalm_b200.h -nt build/$f.o ]; then
     $NVCC $FLAGS -c $f.cu -o build/$f.o &
     pids+=($!)
@@ -27,5 +27,5 @@ for v in batchp_probe batchp4_probe; do
   fi
 done
 for p in "${pids[@]}"; do wait $p; done
-$NVCC -shared -o ../libqpalm_b200.so build/dense.o build/updown_flow.o build/updown_gen.o build/kernels.o build/api.o build/ops.o build/compat.o build/kkt.o build/batch.o build/batchp.o build/batchp4.o build/batchp_probe.o build/batchp4_probe.o build/prof.o build/shard.o build/sparse.o build/sparse_sym.o build/qps.o -lcudart -ldl
+$NVCC -shared -o ../libqpalm_b200.so build/dense.o build/updown_gen.o build/kernels.o build/api.o build/ops.o build/compat.o build/kkt.o build/batch.o build/batchp.o build/batchp4.o build/batchp_probe.o build/batchp4_probe.o build/prof.o build/shard.o build/sparse.o build/sparse_sym.o build/qps.o -lcudart -ldl
 echo "built $(cd .. && pwd)/libqpalm_b200.so"

@@ -19,22 +19,20 @@ long long g_kernel_launches = 0;
 
 // ================================================================================================
 // DMMA NT GEMM:  C = beta*C + alpha * A * B'
-// CTA tile 128 x 128 x 16, 8 warps (2 x 4), warp tile 64 x 32 = 8 x 4 m8n8k4 fragments,
-// 3-stage cp.async pipeline, k-major shared tiles padded to 132 doubles (conflict-free 64-bit
-// fragment loads: lane -> (k = lane & 3, row = lane >> 2) hits 16 distinct 8-byte banks per half warp).
+// CTA tile BM_ x 128 x 16, 8 consumer warps + 1 producer warp, a 4-stage ring of k-major shared tiles padded to BM_ + 4 / 132
+// doubles (conflict-free 64-bit fragment loads: lane -> (k = lane & 3, row = lane >> 2) hits 16 distinct 8-byte banks per half warp).
+// The tile movement is on the TMA engine: bulk asynchronous copies (cp.async.bulk, SASS UBLKCP) issued by the PRODUCER warp
+// and completed on mbarriers (its predecessor issued 16 cp.async (LDGSTS) instructions per thread and stage; DESIGN.md
+// section 4 has both rates).
+//   * warps 0-7 only compute (no address arithmetic, no copy instructions, no __syncthreads in the main loop);
+//   * warp 8 owns the pipeline: per k-tile it waits for the stage's `empty` barrier (one arrival per consumer warp), posts
+//     the expected byte count on the `full` barrier and issues ONE bulk copy per lane: lanes 0-15 the 16 k-columns of the A
+//     tile, lanes 16-31 those of the B tile (each a contiguous run of BM_ / BN doubles of the column-major operand, landing
+//     in the padded k-major row the fragment loads expect).
+// Every operand column start is 16-byte aligned (leading dimensions are multiples of 128, tile origins multiples of 64).
 // ================================================================================================
 namespace gemm {
-constexpr int BM = 128, BN = 128, BK = 16, STAGES = 3;
-template <int BM_> constexpr size_t smem_bytes() { return sizeof(double) * STAGES * BK * ((BM_ + 4) + (BN + 4)); }
-constexpr size_t kSmemBytes = smem_bytes<BM>();
-
-__device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src) {
-  unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gmem_src));
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N)); }
+constexpr int BM = 128, BN = 128, BK = 16;
 
 __device__ __forceinline__ void dmma884(double &d0, double &d1, double a, double b) {
   asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
@@ -42,118 +40,6 @@ __device__ __forceinline__ void dmma884(double &d0, double &d1, double a, double
       : "d"(a), "d"(b));
 }
 
-// BM_ = 128: CTA tile 128 x 128, warps 2 x 4, warp tile 64 x 32.  BM_ = 64: CTA tile 64 x 128, warps 1 x 8, warp tile
-// 64 x 16 -- twice as many CTAs of half the work each, for the panel solves and in-block updates of the Cholesky chain
-// whose 128-row grids fill less than one wave of the 148 SMs.
-template <int BM_>
-__global__ void __launch_bounds__(256, 1)
-k_dgemm_nt(int K, const double *A, int lda, const double *B, int ldb,
-           double *C, int ldc, double alpha, double beta, int lower_only,
-           long long sA, long long sB, long long sC, const int *Kz, const int *maskz) {
-  constexpr int SROWA = BM_ + 4, SROWB = BN + 4;
-  constexpr int WM = BM_ / 64, WN = 8 / WM, NF = BN / (8 * WN);   // warps along M / N, n-fragments per warp
-  // blockIdx.z: batch instance (strides sA/sB/sC, optional per-instance K and activity mask)
-  const int bm = blockIdx.x, bn = blockIdx.y;
-  if (lower_only && bn * BN >= (bm + 1) * BM_) return;
-  if (maskz && !maskz[blockIdx.z]) return;
-  if (Kz) K = Kz[blockIdx.z];
-  if (K <= 0 && beta == 1.0) return;
-  A += (size_t)blockIdx.z * sA; B += (size_t)blockIdx.z * sB; C += (size_t)blockIdx.z * sC;
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  typedef double TileA[BK][SROWA];
-  typedef double TileB[BK][SROWB];
-  TileA *As = reinterpret_cast<TileA *>(smem_raw);
-  TileB *Bs = reinterpret_cast<TileB *>(smem_raw + sizeof(double) * STAGES * BK * SROWA);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, wm = warp % WM, wn = warp / WM;
-  const double *Ag = A + (size_t)bm * BM_;
-  const double *Bg = B + (size_t)bn * BN;
-  const int KT = K / BK;
-
-  auto load_stage = [&](int stage, int kt) {
-    const int k0 = kt * BK;
-#pragma unroll
-    for (int c = tid; c < BK * BM_ / 2; c += 256) {
-      const int kk = c / (BM_ / 2), mc = (c % (BM_ / 2)) * 2;
-      cp_async16(&As[stage][kk][mc], Ag + mc + (size_t)(k0 + kk) * lda);
-    }
-#pragma unroll
-    for (int c = tid; c < BK * BN / 2; c += 256) {
-      const int kk = c / (BN / 2), mc = (c % (BN / 2)) * 2;
-      cp_async16(&Bs[stage][kk][mc], Bg + mc + (size_t)(k0 + kk) * ldb);
-    }
-  };
-
-  double acc[8][NF][2];
-#pragma unroll
-  for (int i = 0; i < 8; i++)
-#pragma unroll
-    for (int j = 0; j < NF; j++) acc[i][j][0] = acc[i][j][1] = 0.0;
-
-#pragma unroll
-  for (int s = 0; s < STAGES - 1; s++) {
-    if (s < KT) load_stage(s, s);
-    cp_async_commit();
-  }
-  const int fr = lane >> 2, fk = lane & 3;
-  for (int kt = 0; kt < KT; kt++) {
-    cp_async_wait<STAGES - 2>();
-    __syncthreads();
-    {
-      const int nk = kt + STAGES - 1;
-      if (nk < KT) load_stage(nk % STAGES, nk);
-      cp_async_commit();
-    }
-    const int st = kt % STAGES;
-    double a[2][8], b[2][NF];
-#pragma unroll
-    for (int mb = 0; mb < 8; mb++) a[0][mb] = As[st][fk][wm * 64 + mb * 8 + fr];
-#pragma unroll
-    for (int nb = 0; nb < NF; nb++) b[0][nb] = Bs[st][fk][wn * (8 * NF) + nb * 8 + fr];
-#pragma unroll
-    for (int ks = 0; ks < 4; ks++) {
-      const int cur = ks & 1, nxt = cur ^ 1;
-      if (ks < 3) {
-#pragma unroll
-        for (int mb = 0; mb < 8; mb++) a[nxt][mb] = As[st][(ks + 1) * 4 + fk][wm * 64 + mb * 8 + fr];
-#pragma unroll
-        for (int nb = 0; nb < NF; nb++) b[nxt][nb] = Bs[st][(ks + 1) * 4 + fk][wn * (8 * NF) + nb * 8 + fr];
-      }
-#pragma unroll
-      for (int mb = 0; mb < 8; mb++)
-#pragma unroll
-        for (int nb = 0; nb < NF; nb++) dmma884(acc[mb][nb][0], acc[mb][nb][1], a[cur][mb], b[cur][nb]);
-    }
-  }
-  cp_async_wait<0>();
-  __syncthreads();  // all global reads of this CTA have landed: C may alias A from here on
-
-  const bool use_beta = (beta != 0.0);
-#pragma unroll
-  for (int mb = 0; mb < 8; mb++) {
-    const int row = bm * BM_ + wm * 64 + mb * 8 + fr;
-#pragma unroll
-    for (int nb = 0; nb < NF; nb++) {
-      const int col = bn * BN + wn * (8 * NF) + nb * 8 + 2 * fk;
-      double *c0 = C + row + (size_t)col * ldc;
-      double *c1 = c0 + ldc;
-      double v0 = alpha * acc[mb][nb][0], v1 = alpha * acc[mb][nb][1];
-      if (use_beta) { v0 += beta * (*c0); v1 += beta * (*c1); }
-      *c0 = v0; *c1 = v1;
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------------------------------
-// The same GEMM with the tile movement on the TMA engine: bulk asynchronous copies (cp.async.bulk, SASS UBLKCP) issued by a
-// PRODUCER warp and completed on mbarriers, instead of 16 cp.async (LDGSTS) instructions per thread and stage.
-//   * warps 0-7 only compute (no address arithmetic, no copy instructions, no __syncthreads in the main loop);
-//   * warp 8 owns the pipeline: per k-tile it waits for the stage's `empty` barrier (one arrival per consumer warp), posts
-//     the expected byte count on the `full` barrier and issues ONE bulk copy per lane: lanes 0-15 the 16 k-columns of the A
-//     tile, lanes 16-31 those of the B tile (each a contiguous run of BM_ / BN doubles of the column-major operand, landing
-//     in the padded k-major row the fragment loads expect);
-//   * 4 stages instead of 3 (the registers the consumers no longer spend on copies pay for nothing else, shared memory does).
-// Every operand column start is 16-byte aligned (leading dimensions are multiples of 128, tile origins multiples of 64).
-// ------------------------------------------------------------------------------------------------------------------
 constexpr int TSTAGES = 4;
 template <int BM_> constexpr size_t smem_bytes_tma() { return sizeof(double) * TSTAGES * BK * ((BM_ + 4) + (BN + 4)) + 2 * TSTAGES * sizeof(unsigned long long); }
 
@@ -183,6 +69,9 @@ __device__ __forceinline__ void bulk_g2s(void *smem_dst, const void *gmem_src, u
                "l"(gmem_src), "r"(bytes), "r"((unsigned)__cvta_generic_to_shared(bar)) : "memory");
 }
 
+// BM_ = 128: CTA tile 128 x 128, warps 2 x 4, warp tile 64 x 32.  BM_ = 64: CTA tile 64 x 128, warps 1 x 8, warp tile
+// 64 x 16 -- twice as many CTAs of half the work each, for the panel solves and in-block updates of the Cholesky chain
+// whose 128-row grids fill less than one wave of the 148 SMs.
 template <int BM_>
 __global__ void __launch_bounds__(288, 1)
 k_dgemm_nt_tma(int K, const double *A, int lda, const double *B, int ldb,
@@ -281,8 +170,6 @@ k_dgemm_nt_tma(int K, const double *A, int lda, const double *B, int ldb,
 static int gemm_attr() {
   static bool attr_set = false;
   if (!attr_set) {
-    QB_CUDA_TRY(cudaFuncSetAttribute(gemm::k_dgemm_nt<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm::smem_bytes<128>()));
-    QB_CUDA_TRY(cudaFuncSetAttribute(gemm::k_dgemm_nt<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm::smem_bytes<64>()));
     QB_CUDA_TRY(cudaFuncSetAttribute(gemm::k_dgemm_nt_tma<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm::smem_bytes_tma<128>()));
     QB_CUDA_TRY(cudaFuncSetAttribute(gemm::k_dgemm_nt_tma<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm::smem_bytes_tma<64>()));
     attr_set = true;
@@ -304,21 +191,14 @@ int dgemm_nt_batched(cudaStream_t s, int nb, int M, int N, int K, const int *Kz,
   const long long tiles = (lower_only ? (nt <= mt ? nt * mt - nt * (nt - 1) / 2 : mt * (mt + 1) / 2) : mt * nt) * nb;
   static int num_sms = 0;
   if (!num_sms) { int dev = 0; QB_CUDA_TRY(cudaGetDevice(&dev)); QB_CUDA_TRY(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev)); }
-  // tile movement on the TMA engine (bulk async copies + mbarriers, producer warp) unless QPALM_B200_GEMM_LDGSTS=1 (A/B runs);
-  // the in-place panel solve (C aliases A across CTAs of one tile column is CTA-local, see the kernel) takes either path
-  static const bool legacy = getenv("QPALM_B200_GEMM_LDGSTS") != nullptr;
   if (tiles < num_sms) {
     dim3 grid(M / 64, N / gemm::BN, nb);
-    if (legacy) QB_LAUNCH(gemm::k_dgemm_nt<64>, grid, 256, gemm::smem_bytes<64>(), s, K, A, lda, B, ldb, C, ldc, alpha, beta,
-                          lower_only ? 1 : 0, sA, sB, sC, Kz, maskz);
-    else QB_LAUNCH(gemm::k_dgemm_nt_tma<64>, grid, 288, gemm::smem_bytes_tma<64>(), s, K, A, lda, B, ldb, C, ldc, alpha, beta,
-                   lower_only ? 1 : 0, sA, sB, sC, Kz, maskz);
+    QB_LAUNCH(gemm::k_dgemm_nt_tma<64>, grid, 288, gemm::smem_bytes_tma<64>(), s, K, A, lda, B, ldb, C, ldc, alpha, beta,
+              lower_only ? 1 : 0, sA, sB, sC, Kz, maskz);
   } else {
     dim3 grid(M / gemm::BM, N / gemm::BN, nb);
-    if (legacy) QB_LAUNCH(gemm::k_dgemm_nt<128>, grid, 256, gemm::smem_bytes<128>(), s, K, A, lda, B, ldb, C, ldc, alpha, beta,
-                          lower_only ? 1 : 0, sA, sB, sC, Kz, maskz);
-    else QB_LAUNCH(gemm::k_dgemm_nt_tma<128>, grid, 288, gemm::smem_bytes_tma<128>(), s, K, A, lda, B, ldb, C, ldc, alpha, beta,
-                   lower_only ? 1 : 0, sA, sB, sC, Kz, maskz);
+    QB_LAUNCH(gemm::k_dgemm_nt_tma<128>, grid, 288, gemm::smem_bytes_tma<128>(), s, K, A, lda, B, ldb, C, ldc, alpha, beta,
+              lower_only ? 1 : 0, sA, sB, sC, Kz, maskz);
   }
   QB_CUDA_TRY(cudaGetLastError());
   return 0;

@@ -42,16 +42,10 @@ void chol_solve_release(cudaStream_t s);
 int chol_updown(cudaStream_t s, int npad, double *L, int ld, double *W, int ldw, int k, int sign,
                 double *coef, int *info_dev);
 
-// One-launch dataflow sweep (updown_flow.cu): L <- chol(L L' + W S W'), S = diag(+1 x kpos, -1 x (k - kpos)), k <= 64 per call;
-// W (npad x k, ldw) is only read.  Returns 0 when it ran, 1 when the cooperative kernel is not available (use chol_updown).
-int chol_updown_flow(cudaStream_t s, int npad, double *L, int ld, const double *W, int ldw, int k, int kpos, int *info_dev,
-                     long long *clk_dev = nullptr /* instrumented runs: 32 clock64 stamps of the chain CTA */);
-int chol_updown_flow_max_rank();
-void chol_updown_flow_release(cudaStream_t s);
-
-// Generator-form pass (updown_gen.cu): the same result as chol_updown_flow for k <= 32 columns, reached by ONE triangular solve with
-// k right-hand sides (the only serial chain, npad / 128 steps) + fully parallel passes.  invdiag = inverses of the diagonal blocks
-// of the current L (input; refresh it afterwards with trtri_diag_blocks).  Returns 0 when it ran, 1 when unavailable.
+// Generator-form pass (updown_gen.cu): L <- chol(L L' + W S W'), S = diag(+1 x kpos, -1 x (k - kpos)), k <= 32 per call, reached by
+// ONE triangular solve with k right-hand sides (the only serial chain, npad / 128 steps) + fully parallel passes; W (npad x k, ldw)
+// is only read.  invdiag = inverses of the diagonal blocks of the current L (input; refresh it afterwards with trtri_diag_blocks).
+// Returns 0 when it ran, 1 when unavailable (no cooperative launch, or no room for its work space: use chol_updown), < 0 on a CUDA error.
 int chol_updown_gen(cudaStream_t s, int npad, double *L, int ld, const double *invdiag, const double *W, int ldw, int k, int kpos,
                     int *info_dev);
 int chol_updown_gen_max_rank();

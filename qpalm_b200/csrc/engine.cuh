@@ -109,10 +109,8 @@ struct Engine {
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, evs0 = nullptr, evs1 = nullptr;
   // tunables
   int updown_max_rank = 8;           // one sweep of the rank-k kernel
-  bool updown_gen_ok = true;         // cleared when the generator-form update pass (updown_gen.cu) cannot launch on this device
-  bool updown_flow_ok = true;        // cleared when the cooperative dataflow sweep cannot launch on this device
+  bool updown_gen_ok = true;         // cleared when the generator-form update pass (updown_gen.cu) is unavailable on this device
   double updown_gen_scale = 1.0;     // static cost model of the generator-form passes (api.cu prefer_updown): scale factor, QPALM_B200_UPDOWN_GEN_SCALE
-  double updown_panel_ms = 0.0135, updown_panel_ms64 = 0.0179;   // static cost model: one panel step of the dataflow sweep, <= 32 / <= 64 ranks (B200)
   int updown_force = 0;              // QPALM_B200_UPDOWN_FORCE=1: bypass the cost model (tests)
   double last_updown_ms = -1.0;      // CUDA-event time of the most recent update/downdate call (sparse cost model)
   double last_refactor_ms = -1.0;    // CUDA-event time of the most recent refactorisation (cost model input)

@@ -594,19 +594,11 @@ int step_newton_refactor(Engine *e, bool with_constraints, bool from_scratch, do
   return 0;
 }
 
-// the one-launch dataflow sweep (updown_flow.cu) serves factors of at least two 128-column blocks; below that the
-// per-panel kernels of dense.cu cost a handful of launches
-static bool use_updown_flow(const Engine *e) {
-  static const int min_npad = [] { const char *s = getenv("QPALM_B200_UPDOWN_FLOW_MIN"); return s ? atoi(s) : 256; }();
-  return !e->sp && e->npad >= min_npad && e->updown_flow_ok;
-}
-
-// generator-form passes (updown_gen.cu): <= 32 columns each, entering and leaving rows share a pass; the inverted diagonal
+// generator-form passes (updown_gen.cu) serve factors of at least two 128-column blocks; below that the per-panel kernels of
+// dense.cu cost a handful of launches.  <= 32 columns per pass, entering and leaving rows share a pass; the inverted diagonal
 // blocks are refreshed after every pass (the next pass's triangular solve needs them, and so do the Newton solves)
 bool use_updown_gen(const Engine *e) {
-  const char *s = getenv("QPALM_B200_UPDOWN_GEN");      // read per call: the tests run both update paths in one process
-  const bool off = s && atoi(s) == 0;
-  return !off && !e->sp && e->npad >= 256 && e->updown_gen_ok;
+  return !e->sp && e->npad >= 256 && e->updown_gen_ok;
 }
 static int updown_gen_lists(Engine *e, const int *pos, const double *pos_scale, bool pos_by_row, int npos,
                             const int *neg, const double *neg_scale, bool neg_by_row, int nneg) {
@@ -617,39 +609,17 @@ static int updown_gen_lists(Engine *e, const int *pos, const double *pos_scale, 
     const int kn = (nneg - in < KMAX - kp) ? nneg - in : KMAX - kp;
     if (int r = gather_rows(e, pos + ip, pos_by_row ? pos_scale : pos_scale + ip, pos_by_row, kp, kp, 0)) return r;
     if (int r = gather_rows(e, neg + in, neg_by_row ? neg_scale : neg_scale + in, neg_by_row, kn, kn, kp)) return r;
+    // row-sharded problem: every rank gathered the rows it owns (zero columns for the others); the sum over ranks is the full
+    // n x k block, and every rank then runs the same pass on its replica of L
     if (e->sh_world > 1) { if (int r = shard_allreduce(e->W, e->W, (size_t)e->ld * (kp + kn), false, e->stream)) return r; }
     const int rc = chol_updown_gen(e->stream, e->npad, e->L, e->ld, e->invdiag, e->W, e->ld, kp + kn, kp, e->info_dev);
+    // 1: unavailable -- it fails on the first pass or never, so nothing has been applied and the caller can fall back to the
+    // per-panel kernels; < 0: CUDA error
     if (rc) return (rc == 1 && ip == 0 && in == 0) ? 1 : (rc < 0 ? rc : -999);
     if (int r = trtri_diag_blocks(e->stream, e->npad, e->L, e->ld, e->invdiag)) return r;
     e->n_updown++; e->updown_rank_sum += kp + kn;
     e->dense_flops += 2.0 * (kp + kn) * (double)e->n * e->n;
     e->alg_bytes += 3.0 * 8.0 * (double)e->n * (e->n + 1) / 2;
-    ip += kp; in += kn;
-  }
-  return 0;
-}
-
-// L <- chol(L L' + sum_enter w w' - sum_leave w w'): entering and leaving rows share sweeps of <= 64 columns
-// (weight pattern S = diag(+1.., -1..), see updown_flow.cu)
-static int updown_flow_lists(Engine *e, const int *pos, const double *pos_scale, bool pos_by_row, int npos,
-                             const int *neg, const double *neg_scale, bool neg_by_row, int nneg) {
-  const int KMAX = chol_updown_flow_max_rank();
-  int ip = 0, in = 0;
-  while (ip < npos || in < nneg) {
-    const int kp = (npos - ip < KMAX) ? npos - ip : KMAX;
-    const int kn = (nneg - in < KMAX - kp) ? nneg - in : KMAX - kp;
-    if (int r = gather_rows(e, pos + ip, pos_by_row ? pos_scale : pos_scale + ip, pos_by_row, kp, kp, 0)) return r;
-    if (int r = gather_rows(e, neg + in, neg_by_row ? neg_scale : neg_scale + in, neg_by_row, kn, kn, kp)) return r;
-    // row-sharded problem: every rank gathered the rows it owns (zero columns for the others); the sum over ranks is the full
-    // n x k block, and every rank then runs the same sweep on its replica of L
-    if (e->sh_world > 1) { if (int r = shard_allreduce(e->W, e->W, (size_t)e->ld * (kp + kn), false, e->stream)) return r; }
-    const int rc = chol_updown_flow(e->stream, e->npad, e->L, e->ld, e->W, e->ld, kp + kn, kp, e->info_dev);
-    // 1: cooperative launch unavailable -- it fails on the first chunk or never, so nothing has been applied and the caller
-    // can fall back to the per-panel kernels; < 0: CUDA error
-    if (rc) return (rc == 1 && ip == 0 && in == 0) ? 1 : (rc < 0 ? rc : -999);
-    e->n_updown++; e->updown_rank_sum += kp + kn;
-    e->dense_flops += 2.0 * (kp + kn) * (double)e->n * e->n;
-    e->alg_bytes += 2.0 * 8.0 * (double)e->n * (e->n + 1) / 2;
     ip += kp; in += kn;
   }
   return 0;
@@ -662,17 +632,7 @@ int step_newton_updown(Engine *e, int nb_enter, int nb_leave) {
     const int rc = updown_gen_lists(e, e->enter, e->sqrt_sigma, true, nb_enter, e->leave, e->sqrt_sigma, true, nb_leave);
     if (rc < 0) return rc;
     if (rc == 0) { QB_CUDA_TRY(cudaEventRecord(e->evs1, e->stream)); return 0; }
-    e->updown_gen_ok = false;
-  }
-  if (use_updown_flow(e)) {
-    const int rc = updown_flow_lists(e, e->enter, e->sqrt_sigma, true, nb_enter, e->leave, e->sqrt_sigma, true, nb_leave);
-    if (rc < 0) return rc;
-    if (rc == 0) {
-      if (int r = trtri_diag_blocks(e->stream, e->npad, e->L, e->ld, e->invdiag)) return r;
-      QB_CUDA_TRY(cudaEventRecord(e->evs1, e->stream));
-      return 0;
-    }
-    e->updown_flow_ok = false;   // no cooperative launch on this device / partition: per-panel kernels from now on
+    e->updown_gen_ok = false;   // unavailable on this device / partition: per-panel kernels from now on
   }
   for (int pass = 0; pass < 2; pass++) {
     const int *list = pass == 0 ? e->enter : e->leave;
@@ -687,6 +647,7 @@ int step_newton_updown(Engine *e, int nb_enter, int nb_leave) {
         continue;
       }
       if (int r = gather_rows(e, list + off, e->sqrt_sigma, true, k, 8)) return r;
+      if (e->sh_world > 1) { if (int r = shard_allreduce(e->W, e->W, (size_t)e->ld * 8, false, e->stream)) return r; }   // as in updown_gen_lists
       if (int r = chol_updown(e->stream, e->npad, e->L, e->ld, e->W, e->ld, k, pass == 0 ? +1 : -1, e->ud_coef, e->info_dev)) return r;
       e->n_updown++; e->updown_rank_sum += k;
       e->dense_flops += 2.0 * k * (double)e->n * e->n;
@@ -707,16 +668,6 @@ int sigma_changed_update(Engine *e, int nb_changed) {
     if (rc == 0) { QB_CUDA_TRY(cudaEventRecord(e->evs1, e->stream)); return 0; }
     e->updown_gen_ok = false;
   }
-  if (use_updown_flow(e)) {
-    const int rc = updown_flow_lists(e, e->changed, e->w_pos, false, nb_changed, nullptr, nullptr, false, 0);
-    if (rc < 0) return rc;
-    if (rc == 0) {
-      if (int r = trtri_diag_blocks(e->stream, e->npad, e->L, e->ld, e->invdiag)) return r;
-      QB_CUDA_TRY(cudaEventRecord(e->evs1, e->stream));
-      return 0;
-    }
-    e->updown_flow_ok = false;
-  }
   for (int off = 0; off < nb_changed; off += 8) {
     const int k = nb_changed - off < 8 ? nb_changed - off : 8;
     if (e->sp) {
@@ -726,6 +677,7 @@ int sigma_changed_update(Engine *e, int nb_changed) {
       continue;
     }
     if (int r = gather_rows(e, e->changed + off, e->w_pos + off, false, k, 8)) return r;
+    if (e->sh_world > 1) { if (int r = shard_allreduce(e->W, e->W, (size_t)e->ld * 8, false, e->stream)) return r; }
     if (int r = chol_updown(e->stream, e->npad, e->L, e->ld, e->W, e->ld, k, +1, e->ud_coef, e->info_dev)) return r;
     e->n_updown++; e->updown_rank_sum += k;
     e->dense_flops += 2.0 * k * (double)e->n * e->n;
@@ -2057,7 +2009,6 @@ static int engine_create_impl(Engine *e, Engine **out, int n, int m, const long 
   if (const char *s = getenv("QPALM_B200_UPDOWN_MAX_RANK")) e->updown_max_rank = atoi(s);
   if (const char *s = getenv("QPALM_B200_UPDOWN_FORCE")) e->updown_force = atoi(s);
   if (const char *s = getenv("QPALM_B200_UPDOWN_GEN_SCALE")) e->updown_gen_scale = atof(s);
-  if (const char *s = getenv("QPALM_B200_UPDOWN_PANEL_MS")) { e->updown_panel_ms = atof(s); e->updown_panel_ms64 = 1.33 * e->updown_panel_ms; }
   QB_CUDA_TRY(cudaDeviceSynchronize());
   lap("factor storage + scratch");
   *out = e;
@@ -2085,7 +2036,7 @@ void engine_destroy(Engine *e) {
   if (e->ev1) cudaEventDestroy(e->ev1);
   if (e->evs0) cudaEventDestroy(e->evs0);
   if (e->evs1) cudaEventDestroy(e->evs1);
-  if (e->stream) { chol_solve_release(e->stream); chol_updown_flow_release(e->stream); chol_updown_gen_release(e->stream); cudaStreamDestroy(e->stream); }
+  if (e->stream) { chol_solve_release(e->stream); chol_updown_gen_release(e->stream); cudaStreamDestroy(e->stream); }
   delete e;
 }
 

@@ -220,10 +220,7 @@ extern "C" int qpalm_b200_updown(c_int n_, c_int k_, c_float *L, const c_float *
   QB_CUDA_TRY(cudaMemcpy(e->L, Lp.data(), sizeof(double) * Lp.size(), cudaMemcpyHostToDevice));
   QB_CUDA_TRY(cudaMemset(e->info_dev, 0, sizeof(int)));
   rc = 0;
-  static const int flow_min = [] { const char *s = getenv("QPALM_B200_UPDOWN_FLOW_MIN"); return s ? atoi(s) : 256; }();
-  bool flow = npad >= flow_min;   // same dispatch as step_newton_updown: one dataflow launch per <= 64 columns
-  const int chunk = flow ? chol_updown_flow_max_rank() : 8;
-  bool gen = use_updown_gen(e);   // ... preceded by the generator-form passes of <= 32 columns (updown_gen.cu)
+  bool gen = use_updown_gen(e);   // same dispatch as step_newton_updown: generator-form passes of <= 32 columns (updown_gen.cu)
   for (int off = 0; off < k && !rc && gen; off += chol_updown_gen_max_rank()) {
     const int kk = k - off < chol_updown_gen_max_rank() ? k - off : chol_updown_gen_max_rank();
     std::vector<double> Wp((size_t)ld * kk, 0.0);
@@ -232,19 +229,9 @@ extern "C" int qpalm_b200_updown(c_int n_, c_int k_, c_float *L, const c_float *
     QB_CUDA_TRY(cudaMemcpy(e->W, Wp.data(), sizeof(double) * Wp.size(), cudaMemcpyHostToDevice));
     rc = trtri_diag_blocks(e->stream, npad, e->L, ld, e->invdiag);
     if (!rc) rc = chol_updown_gen(e->stream, npad, e->L, ld, e->invdiag, e->W, ld, kk, update ? kk : 0, e->info_dev);
-    if (rc == 1 && off == 0) { gen = false; rc = 0; }
+    if (rc == 1 && off == 0) { gen = false; rc = 0; }   // unavailable here: per-panel kernels below
   }
-  if (gen) flow = false;
-  for (int off = 0; off < k && !rc && flow; off += chunk) {
-    const int kk = k - off < chunk ? k - off : chunk;
-    std::vector<double> Wp((size_t)ld * kk, 0.0);
-    for (int c = 0; c < kk; c++) for (int i = 0; i < n; i++) Wp[(size_t)i + (size_t)ld * c] = W[(size_t)i + (size_t)n * (off + c)];
-    QB_CUDA_TRY(cudaStreamSynchronize(e->stream));
-    QB_CUDA_TRY(cudaMemcpy(e->W, Wp.data(), sizeof(double) * Wp.size(), cudaMemcpyHostToDevice));
-    rc = chol_updown_flow(e->stream, npad, e->L, ld, e->W, ld, kk, update ? kk : 0, e->info_dev);
-    if (rc == 1 && off == 0) { flow = false; rc = 0; }   // no cooperative launch here: per-panel kernels below
-  }
-  for (int off = 0; off < k && !rc && !flow && !gen; off += 8) {
+  for (int off = 0; off < k && !rc && !gen; off += 8) {
     const int kk = k - off < 8 ? k - off : 8;
     std::vector<double> Wp((size_t)ld * 8, 0.0);
     for (int c = 0; c < kk; c++) for (int i = 0; i < n; i++) Wp[(size_t)i + (size_t)ld * c] = W[(size_t)i + (size_t)n * (off + c)];
@@ -426,11 +413,12 @@ extern "C" int qpalm_b200_bench_potrf(c_int n_, c_int reps, double *ms_out) {
   return rc ? rc : hinfo;
 }
 
-// one rank-k sweep (update, then the matching downdate so the factor stays bounded) on a factored random SPD matrix:
-// ms per sweep, averaged over 2 * reps sweeps
+// one rank-k update (then the matching downdate so the factor stays bounded) on a factored random SPD matrix, as the solver
+// runs it: generator-form passes of <= 32 columns, each with the refresh of the inverted diagonal blocks the next pass needs.
+// ms per rank-k update or downdate, averaged over 2 * reps of them
 extern "C" int qpalm_b200_bench_updown(c_int n_, c_int k_, c_int reps, double *ms_out) {
   const int n = round_up((int)n_, 128), k = (int)k_;
-  if (k < 1 || k > chol_updown_flow_max_rank()) return 1;
+  if (k < 1) return 1;
   double *L = nullptr, *X = nullptr, *W = nullptr; int *info = nullptr;
   QB_CUDA_TRY(cudaMalloc(&L, sizeof(double) * (size_t)n * n));
   QB_CUDA_TRY(cudaMalloc(&X, sizeof(double) * (size_t)n * 128));
@@ -445,19 +433,15 @@ extern "C" int qpalm_b200_bench_updown(c_int n_, c_int k_, c_int reps, double *m
   int rc = potrf_lower(s, n, L, n, X, info);
   cudaEvent_t a, b; cudaEventCreate(&a); cudaEventCreate(&b);
   float total = 0;
-  const char *genv = getenv("QPALM_B200_UPDOWN_GEN");
-  const bool gen = !(genv && atoi(genv) == 0);
+  const int KMAX = chol_updown_gen_max_rank();
   for (int r = 0; r < reps + 1 && !rc; r++) {
     cudaEventRecord(a, s);
-    if (gen && k <= chol_updown_gen_max_rank()) {     // each pass with the refresh of the inverted diagonal blocks it needs
-      rc = chol_updown_gen(s, n, L, n, X, W, n, k, k, info);
-      if (!rc) rc = trtri_diag_blocks(s, n, L, n, X);
-      if (!rc) rc = chol_updown_gen(s, n, L, n, X, W, n, k, 0, info);
-      if (!rc) rc = trtri_diag_blocks(s, n, L, n, X);
-    } else {
-      rc = chol_updown_flow(s, n, L, n, W, n, k, k, info);
-      if (!rc) rc = chol_updown_flow(s, n, L, n, W, n, k, 0, info);
-    }
+    for (int update = 1; update >= 0 && !rc; update--)
+      for (int off = 0; off < k && !rc; off += KMAX) {
+        const int kk = k - off < KMAX ? k - off : KMAX;
+        rc = chol_updown_gen(s, n, L, n, X, W + (size_t)n * off, n, kk, update ? kk : 0, info);
+        if (!rc) rc = trtri_diag_blocks(s, n, L, n, X);
+      }
     cudaEventRecord(b, s);
     QB_CUDA_TRY(cudaEventSynchronize(b));
     float ms = 0; cudaEventElapsedTime(&ms, a, b);
@@ -465,7 +449,7 @@ extern "C" int qpalm_b200_bench_updown(c_int n_, c_int k_, c_int reps, double *m
   }
   *ms_out = total / (2.0 * (reps > 0 ? reps : 1));
   int hinfo = 0; cudaMemcpy(&hinfo, info, sizeof(int), cudaMemcpyDeviceToHost);
-  chol_updown_flow_release(s); chol_updown_gen_release(s);
+  chol_updown_gen_release(s);
   cudaEventDestroy(a); cudaEventDestroy(b); cudaStreamDestroy(s); cudaFree(L); cudaFree(X); cudaFree(W); cudaFree(info);
   return rc ? rc : hinfo;
 }
@@ -493,32 +477,6 @@ extern "C" int qpalm_b200_bench_spmv(const solver_sparse *A, const solver_sparse
   cudaEventDestroy(a); cudaEventDestroy(b);
   engine_destroy(e);
   return 0;
-}
-
-// stage clocks of the chain CTA of one sweep (panels 100 and 101): out32 receives up to 32 clock64 stamps
-extern "C" int qpalm_b200_bench_updown_clocks(c_int n_, c_int k_, long long *out32) {
-  const int n = round_up((int)n_, 128), k = (int)k_;
-  double *L = nullptr, *X = nullptr, *W = nullptr; int *info = nullptr; long long *clk = nullptr;
-  QB_CUDA_TRY(cudaMalloc(&L, sizeof(double) * (size_t)n * n));
-  QB_CUDA_TRY(cudaMalloc(&X, sizeof(double) * (size_t)n * 128));
-  QB_CUDA_TRY(cudaMalloc(&W, sizeof(double) * (size_t)n * k));
-  QB_CUDA_TRY(cudaMalloc(&info, sizeof(int)));
-  QB_CUDA_TRY(cudaMalloc(&clk, sizeof(long long) * 32));
-  QB_CUDA_TRY(cudaMemset(info, 0, sizeof(int)));
-  QB_CUDA_TRY(cudaMemset(clk, 0, sizeof(long long) * 32));
-  cudaStream_t s; QB_CUDA_TRY(cudaStreamCreate(&s));
-  QB_LAUNCH(k_fill_rand, 1024, 256, 0, s, L, (size_t)n * n, 99ull);
-  QB_LAUNCH(k_fill_rand, 256, 256, 0, s, W, (size_t)n * k, 7ull);
-  dim3 g(cdiv(n, 256), n);
-  QB_LAUNCH(k_make_spd, g, 256, 0, s, n, L);
-  int rc = potrf_lower(s, n, L, n, X, info);
-  if (!rc) rc = chol_updown_flow(s, n, L, n, W, n, k, k, info);          // warm
-  if (!rc) rc = chol_updown_flow(s, n, L, n, W, n, k, 0, info, clk);
-  QB_CUDA_TRY(cudaStreamSynchronize(s));
-  QB_CUDA_TRY(cudaMemcpy(out32, clk, sizeof(long long) * 32, cudaMemcpyDeviceToHost));
-  chol_updown_flow_release(s);
-  cudaStreamDestroy(s); cudaFree(L); cudaFree(X); cudaFree(W); cudaFree(info); cudaFree(clk);
-  return rc;
 }
 
 // ---- batch API: implemented in batch.cu ---------------------------------------------------------------

@@ -17,14 +17,14 @@
 // What is serial, and what is not:
 //   1. k_fwd_multi  -- What = inv(L) W: ONE cooperative dataflow launch, CTA c owns the 128-row blocks c, c + G, ...;
 //      solution blocks travel as epoch-tagged 16-byte packets (as flow::k_solve_flow).  This is the only chain: npad / 128
-//      steps (the dataflow sweep of updown_flow.cu: npad / 32 steps of a much longer step).  On its way the owner of block
+//      steps.  On its way the owner of block
 //      row I stores its running sums  sum_{J' < J} L(I, J') What(J')  for every tile (I, J): the start value of t in step 3.
 //   2. k_gen_gram / k_gen_scan / k_gen_rows -- Gram matrices of 32-row blocks of What, their exclusive prefix (+ S) = M at
 //      the start of each block, then per block (one warp each, all blocks in parallel) inv(M) by Gauss-Jordan in
 //      registers and 32 Sherman-Morrison steps giving d_j and z_j.
 //   3. k_gen_apply  -- every 128 x 128 tile of L independently: one thread per row walks the tile's columns.
 // Every sum has a fixed order (no atomics): re-solves are bit-reproducible (tests/src/test_basic_qp.c:298-305).
-// The caller refreshes the inverses of the diagonal blocks afterwards (trtri_diag_blocks), as after the dataflow sweep.
+// The caller refreshes the inverses of the diagonal blocks afterwards (trtri_diag_blocks).
 #include "dense.cuh"
 #include "chol32.cuh"
 #include <map>
@@ -418,8 +418,8 @@ static int run(cudaStream_t s, State &st, int slot, int npad, double *L, int ld,
 
 int chol_updown_gen_max_rank() { return 32; }
 
-// returns 0 when the pass ran, 1 when the cooperative kernel is not available on this device / partition (the caller
-// uses the dataflow sweep or the per-panel launches), < 0 on a CUDA error.  invdiag must hold the inverses of the
+// returns 0 when the pass ran, 1 when the cooperative kernel is not available on this device / partition or the pass's work
+// space cannot be allocated (the caller uses the per-panel launches), < 0 on a CUDA error.  invdiag must hold the inverses of the
 // diagonal blocks of the CURRENT L; the caller refreshes it afterwards (trtri_diag_blocks).
 int chol_updown_gen(cudaStream_t s, int npad, double *L, int ld, const double *invdiag, const double *W, int ldw, int k, int kpos,
                     int *info_dev) {
@@ -435,7 +435,7 @@ int chol_updown_gen(cudaStream_t s, int npad, double *L, int ld, const double *i
     st.packets = nullptr; st.buf = nullptr; st.tdump = nullptr; st.cap_npad = 0;
     const size_t nblk = (size_t)npad / NB, nblocks = (size_t)npad / GB;
     // work space of a pass: 16 B x 32 per row of packets, 65 doubles per row of What | Z | D, the Gram prefixes and the running sums of
-    // every tile (n = 8000: 66 MB; n = 30 000: 0.9 GB).  If HBM cannot hold it the caller takes the dataflow sweep, which needs none.
+    // every tile (n = 8000: 66 MB; n = 30 000: 0.9 GB).  If HBM cannot hold it the caller takes the per-panel kernels, which need none.
     const cudaError_t e1 = cudaMalloc(&st.packets, sizeof(uint4) * (size_t)npad * 32);
     const cudaError_t e2 = e1 == cudaSuccess ? cudaMalloc(&st.buf, sizeof(double) * ((size_t)npad * 65 + nblocks * 32 * 32)) : e1;
     const cudaError_t e3 = e2 == cudaSuccess ? cudaMalloc(&st.tdump, sizeof(double) * (nblk * (nblk + 1) / 2) * NB * 32) : e2;

@@ -1,5 +1,5 @@
-"""The cholmod_updown replacement on the dense Newton system (updown_gen.cu: generator-form passes of <= 32 columns, the
-default; updown_flow.cu: one cooperative dataflow launch per <= 64 ranks) -- operator level against the oracle's restatement of CHOLMOD's recurrence (Modify/t_cholmod_updown_numkr.c:289-376)
+"""The cholmod_updown replacement on the dense Newton system (updown_gen.cu: generator-form passes of <= 32 columns) --
+operator level against the oracle's restatement of CHOLMOD's recurrence (Modify/t_cholmod_updown_numkr.c:289-376)
 and solver level: the rank-update branch of newton_set_direction (src/newton.c:96-108) and ldlupdate_sigma_changed
 (src/solver_interface.c:443-503, caller src/iteration.c:135-144) must actually be TAKEN on the GPU, with the same
 solutions and iteration counts as the reference."""
@@ -20,24 +20,9 @@ def _rel(a, b):
     return np.max(np.abs(a - b)) / max(1.0, np.max(np.abs(b))) if a.size else 0.0
 
 
-@pytest.fixture(params=["gen", "flow"])
-def update_path(request):
-    """The dense factor has two one-launch update paths: generator-form passes of <= 32 columns (updown_gen.cu, the default)
-    and the dataflow sweep of <= 64 columns (updown_flow.cu, QPALM_B200_UPDOWN_GEN=0).  Both stay under test."""
-    import os
-    old = os.environ.get("QPALM_B200_UPDOWN_GEN")
-    os.environ["QPALM_B200_UPDOWN_GEN"] = "1" if request.param == "gen" else "0"
-    yield request.param
-    if old is None:
-        os.environ.pop("QPALM_B200_UPDOWN_GEN", None)
-    else:
-        os.environ["QPALM_B200_UPDOWN_GEN"] = old
-
-
 @pytest.mark.parametrize("n,k", [(256, 1), (300, 33), (500, 9), (777, 64), (1000, 70), (1400, 40), (2304, 64), (3000, 150)])
-def test_dataflow_rank_k_update_and_downdate(gpu_ops, oracle_ops, update_path, n, k):
-    """L L' +- W W' for factors of >= 2 blocks (generator form: passes of <= 8 / 16 / 32 columns; dataflow sweep: k > 64 takes
-    several sweeps, k > 32 the 64-column shape)."""
+def test_dataflow_rank_k_update_and_downdate(gpu_ops, oracle_ops, n, k):
+    """L L' +- W W' for factors of >= 2 blocks (generator form: passes of <= 8 / 16 / 32 columns, k > 32 takes several)."""
     rng = np.random.default_rng(n + k)
     M = rng.standard_normal((n, n))
     H = M @ M.T + n * np.eye(n)
@@ -54,8 +39,8 @@ def test_dataflow_rank_k_update_and_downdate(gpu_ops, oracle_ops, update_path, n
     assert _rel(Ld_g, L) < 1e-9           # update then downdate is the identity
 
 
-def test_mixed_update_downdate_pass_matches_cholesky(update_path):
-    """Entering and leaving rows share a pass / sweep (S = diag(+1.., -1..)): solver-level check that a step with both kinds of
+def test_mixed_update_downdate_pass_matches_cholesky():
+    """Entering and leaving rows share a pass (S = diag(+1.., -1..)): solver-level check that a step with both kinds of
     change lands on the factor of the new matrix -- forced updates against forced refactorisations on a problem whose active
     set churns (the operator entry point only takes one sign per call)."""
     p = problems.random_qp(520, 1100, 1.0, 1.0, seed=21)
@@ -66,27 +51,18 @@ def test_mixed_update_downdate_pass_matches_cholesky(update_path):
     assert _rel(g1.x, g0.x) < 1e-8 and _rel(g1.y, g0.y) < 1e-8
 
 
-def test_generator_and_dataflow_paths_agree(gpu_ops):
-    """Same update through both paths: factors agree to rounding."""
-    import os
+def test_update_then_partial_downdate_matches_cholesky(gpu_ops):
+    """A 24-column update followed by a downdate of 7 of those columns lands on the factor of H + W W' - W_7 W_7'."""
     n, k = 1152, 24
     rng = np.random.default_rng(5)
     M = rng.standard_normal((n, n)); H = M @ M.T + n * np.eye(n)
     L = np.linalg.cholesky(H); W = rng.standard_normal((n, k))
-    out = {}
-    old = os.environ.get("QPALM_B200_UPDOWN_GEN")
-    try:
-        for name, flag in (("gen", "1"), ("flow", "0")):
-            os.environ["QPALM_B200_UPDOWN_GEN"] = flag
-            out[name] = gpu_ops.updown(gpu_ops.updown(L, W, 1), W[:, :7], 0)
-    finally:
-        os.environ.pop("QPALM_B200_UPDOWN_GEN", None) if old is None else os.environ.__setitem__("QPALM_B200_UPDOWN_GEN", old)
-    assert _rel(out["gen"], out["flow"]) < 1e-11
+    Lg = gpu_ops.updown(gpu_ops.updown(L, W, 1), W[:, :7], 0)
     Href = H + W @ W.T - W[:, :7] @ W[:, :7].T
-    assert _rel(out["gen"] @ out["gen"].T, Href) < 1e-12
+    assert _rel(Lg @ Lg.T, Href) < 1e-12
 
 
-def test_downdate_that_loses_definiteness_is_reported(gpu_ops, update_path):
+def test_downdate_that_loses_definiteness_is_reported(gpu_ops):
     """A downdate past positive definiteness must come back as an error code (the solver then refactorises), not hang."""
     n = 512
     L = np.linalg.cholesky(np.eye(n) * 4.0)
@@ -122,7 +98,7 @@ def _parity(g, r, tol=1e-8, iter_tol=0.05):
 
 
 @pytest.mark.parametrize("n,m,dA,dM,seed", [(600, 1200, 1.0, 1.0, 3), (1000, 2000, 0.3, 1.0, 4), (400, 900, 1.0, 1.0, 6)])
-def test_rank_update_branch_is_taken_with_default_settings(update_path, n, m, dA, dM, seed):
+def test_rank_update_branch_is_taken_with_default_settings(n, m, dA, dM, seed):
     """newton.c:98-108 with the DEFAULT settings (max_rank_update 160, fraction 0.1): the GPU must take rank updates where the
     reference does (updown_calls > 0) and land on the same solution / iteration counts."""
     p = problems.random_qp(n, m, dA, dM, seed=seed)
@@ -133,7 +109,7 @@ def test_rank_update_branch_is_taken_with_default_settings(update_path, n, m, dA
     assert st.refactorizations < g.iter        # not one refactorisation per iteration any more
 
 
-def test_sigma_changed_update_is_taken(update_path):
+def test_sigma_changed_update_is_taken():
     """a10 ldlupdate_sigma_changed: with gamma at gamma_max from the start (default settings) a small number of sigma changes at
     an outer iteration is absorbed by a rank update; assert the branch ran and parity holds."""
     hit = 0
@@ -148,7 +124,7 @@ def test_sigma_changed_update_is_taken(update_path):
     assert hit > 0, "no instance took the sigma-changed rank update"
 
 
-def test_forced_updates_match_forced_refactorisations(update_path):
+def test_forced_updates_match_forced_refactorisations():
     """Same matrix either way: with every eligible step forced through the update sweep (max_rank_update_fraction = 1, rank limit
     raised) the solution equals the refactorise-always run."""
     p = problems.random_qp(700, 1400, 1.0, 1.0, seed=9)

@@ -18,7 +18,5 @@ timeout 900 ncu --metrics gpu__time_duration.sum --clock-control none -c 20000 -
    python bench.py --workload dense --steps 1 --warmup 1 --no-cpu > gpurun_out/ncu_dense.log 2>&1
 timeout 900 ncu --set full --clock-control none --import-source on -k regex:kbp_solve -s 1 -c 1 -f -o gpurun_out/full_kbp_solve \
    python bench.py --steps 1 --warmup 1 --no-dense --no-cpu > gpurun_out/ncu_full_batch.log 2>&1
-timeout 900 ncu --set full --clock-control none --import-source on -k regex:k_updown_flow -s 10 -c 1 -f -o gpurun_out/full_k_updown_flow \
-   python bench.py --workload dense --steps 1 --warmup 1 --no-cpu > gpurun_out/ncu_full_updown.log 2>&1
 tail -5 gpurun_out/pytest_gpu.log; tail -2 gpurun_out/smoke.log; tail -c 1500 gpurun_out/bench.log; tail -c 800 gpurun_out/bench_ref.log; tail -c 800 gpurun_out/bench_dense.log
 ls -la gpurun_out

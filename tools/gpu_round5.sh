@@ -11,7 +11,6 @@ echo "pytest exit $?" >> gpurun_out/pytest_gpu.log
 ( time timeout 600 python bench.py --impl reference --steps 2 --warmup 1 ) > gpurun_out/bench_ref.log 2>&1
 ( time timeout 900 python bench.py --workload dense --steps 3 --warmup 3 ) > gpurun_out/bench_dense.log 2>&1
 python tools/batch_phases.py 512 > gpurun_out/batch_phases.txt 2>&1
-( for n in 8000 1024; do echo "== generator form n=$n"; python tools/prof_dense.py $n updown; python tools/prof_dense.py $n updown 16; echo "== dataflow sweep n=$n"; QPALM_B200_UPDOWN_GEN=0 python tools/prof_dense.py $n updown; done ) > gpurun_out/updown_gen_bench.txt 2>&1
 ( timeout 600 python tools/c3_trace.py ) > gpurun_out/c3_trace_gen.txt 2>&1
 ( timeout 300 python tools/prof_config.py c3; timeout 300 python tools/prof_config.py c1; timeout 300 python tools/prof_config.py c5 ) > gpurun_out/prof_c3_c1_c5.txt 2>&1
 ( QPALM_B200_MF_CLOCKS=1 timeout 600 python tools/prof_config.py grid300; QPALM_B200_MF_PER_BLOCK=1 timeout 600 python tools/prof_config.py grid300 | head -3 ) > gpurun_out/prof_grid300_cluster.txt 2>&1

@@ -1,5 +1,5 @@
 #!/bin/bash
-# compute-sanitizer memcheck + racecheck on the flag / queue based kernels (kbp_solve, flow::k_solve_flow, udflow::k_updown_flow)
+# compute-sanitizer memcheck + racecheck on the flag / queue based kernels (kbp_solve, flow::k_solve_flow)
 mkdir -p gpurun_out
 CS=/usr/local/cuda/bin/compute-sanitizer
 for which in batch dense sparse; do

@@ -25,18 +25,6 @@ elif what == "updown":
         npad = (n + 127) // 128 * 128
         print("updown sweep n", n, "k", k, "rc", rc, "ms", round(ms.value, 4), "us per 32-column panel", round(1e3 * ms.value / (npad / 32), 3),
               "GB/s (2 B_L)", round(2 * 8 * npad * (npad + 1) / 2 / ms.value / 1e6, 1))
-elif what == "updown_clocks":
-    lib.qpalm_b200_bench_updown_clocks.argtypes = [abi.c_int, abi.c_int, C.POINTER(C.c_longlong)]
-    names = ["strip combine", "B = W1 G", "H11", "chol | V solve (+ wait for the I/O warp)", "Ca | Y solves", "G update", "prefetch commit + barrier"]
-    for k in (8, 64):
-        out = (C.c_longlong * 32)()
-        rc = lib.qpalm_b200_bench_updown_clocks(n, k, out)
-        v = [x for x in out if x]
-        print(f"chain CTA stage clocks, k = {k} (rc {rc}), panels 100 and 101:")
-        for half in range(2):
-            seg = v[8 * half: 8 * half + 8]
-            d = np.diff(seg)
-            print("  panel", 100 + half, "total", int(seg[-1] - seg[0]), "clocks:", ", ".join(f"{nm} {int(x)}" for nm, x in zip(names, d)))
 elif what == "potrf_prof":
     # per-kernel CUDA-event breakdown of one blocked Cholesky
     lib.qpalm_b200_bench_potrf.argtypes = [abi.c_int, abi.c_int, C.POINTER(C.c_double)]
