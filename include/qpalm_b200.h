@@ -364,6 +364,10 @@ int  qpalm_b200_batch_stats(QPALMB200Batch *batch, c_int nb, double *out8);
 /* persistent engine, totals of the last solve over instances 0..nb-1: out2 = {rows of A streamed through the H SYRK, summed
  * over the refactorisations; refactorisations that rebuilt H from c Q} (zeros after a lock-step solve) */
 int  qpalm_b200_batch_syrk_stats(QPALMB200Batch *batch, c_int nb, double *out2);
+/* persistent engine, totals of the last solve over instances 0..nb-1, summed over the line searches: out2 = {breakpoints
+ * with s > 0 (the ones the line search sorts); sorted breakpoints its walk read, up to and including the one that fixed
+ * tau} (zeros after a lock-step solve) */
+int  qpalm_b200_batch_linesearch_stats(QPALMB200Batch *batch, c_int nb, double *out2);
 /* persistent engine, QPALM_B200_BATCH_PROF=1 at setup: per-instance SM-clock totals of 16 phases of the last solve */
 int  qpalm_b200_batch_phase_profile(QPALMB200Batch *batch, c_int nb, long long *out);
 long long qpalm_b200_batch_last_launches(const QPALMB200Batch *batch);   /* kernels launched by the last solve */
@@ -392,7 +396,8 @@ int qpalm_b200_batchp_probe_newton(c_int shape, c_int nb, c_int n, c_int m, cons
 int qpalm_b200_batchp_probe_solves(c_int shape, c_int nb, c_int n, c_int m, const c_float *At, const c_float *H0, c_int from_q,
         c_float sscale, const c_int *cnt, const c_int *lists, const c_float *wts, c_float beta, const c_float *rhs,
         c_float *H_out, c_float *L_out, c_float *d_fused, c_float *d_after, c_int *info, c_int rounds, c_float *d_rounds);
-/* the line search's stable radix sort on nb independent arrays of N <= 2048 (key, val) pairs (nb x N each), in place */
+/* the line search's in-CTA sort on nb independent arrays of N <= 2048 (key, val) pairs (nb x N each), in place: keys ascending
+ * as unsigned integers, equal keys in their input order (the solver sorts (key, position) pairs) */
 int qpalm_b200_batchp_probe_sort(c_int shape, c_int nb, c_int N, unsigned long long *keys, unsigned int *vals);
 
 #ifdef __cplusplus

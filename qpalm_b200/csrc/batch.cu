@@ -1162,6 +1162,17 @@ extern "C" int qpalm_b200_batch_syrk_stats(QPALMB200Batch *B, c_int nb, double *
   return 0;
 }
 
+// persistent engine, totals over the instances of the last solve: [0] line-search breakpoints with s > 0 (the ones sorted),
+// [1] sorted breakpoints the walk read (up to and including the one that fixed tau), both summed over the line searches
+extern "C" int qpalm_b200_batch_linesearch_stats(QPALMB200Batch *B, c_int nb, double *out2) {
+  if (!B || nb <= 0 || nb > B->nb_max) return 1;
+  QB_CUDA_TRY(cudaMemcpy(B->ctl_host.data(), B->ctl, sizeof(BCtl) * (size_t)nb, cudaMemcpyDeviceToHost));
+  double k = 0, w = 0;
+  for (c_int b = 0; b < nb; b++) { k += (double)B->ctl_host[b].ls_breakpoints; w += (double)B->ctl_host[b].ls_walked; }
+  out2[0] = k; out2[1] = w;
+  return 0;
+}
+
 extern "C" int qpalm_b200_batch_phase_profile(QPALMB200Batch *B, c_int nb, long long *out /* nb x 16 */) {
   if (!B || !B->prof) return 1;
   QB_CUDA_TRY(cudaMemcpy(out, B->prof, sizeof(long long) * 32 * (size_t)nb, cudaMemcpyDeviceToHost));
@@ -1271,15 +1282,15 @@ extern "C" int qpalm_b200_batchp_probe_sort(c_int shape, c_int nb_, c_int N_, un
   const size_t T = (size_t)nb * N;
   ProbeBufs d;
   unsigned long long *dk = d.get<unsigned long long>(T);
-  unsigned int *dv = d.get<unsigned int>(T);
+  unsigned int *dv = d.get<unsigned int>(T), *dv_out = d.get<unsigned int>(T);   // the sort permutes positions: vals are gathered
   int *dq = d.get<int>(1);
   if (d.failed) return 2;
   const cudaStream_t s = 0;
   QB_CUDA_TRY(cudaMemcpyAsync(dk, keys, sizeof(unsigned long long) * T, cudaMemcpyHostToDevice, s));
   QB_CUDA_TRY(cudaMemcpyAsync(dv, vals, sizeof(unsigned int) * T, cudaMemcpyHostToDevice, s));
-  if (int r = shape == 4 ? batchp4_probe_sort(nb, N, dk, dv, dq, s) : batchp_probe_sort(nb, N, dk, dv, dq, s)) return r;
+  if (int r = shape == 4 ? batchp4_probe_sort(nb, N, dk, dv, dv_out, dq, s) : batchp_probe_sort(nb, N, dk, dv, dv_out, dq, s)) return r;
   QB_CUDA_TRY(cudaMemcpyAsync(keys, dk, sizeof(unsigned long long) * T, cudaMemcpyDeviceToHost, s));
-  QB_CUDA_TRY(cudaMemcpyAsync(vals, dv, sizeof(unsigned int) * T, cudaMemcpyDeviceToHost, s));
+  QB_CUDA_TRY(cudaMemcpyAsync(vals, dv_out, sizeof(unsigned int) * T, cudaMemcpyDeviceToHost, s));
   QB_CUDA_TRY(cudaStreamSynchronize(s));
   return 0;
 }

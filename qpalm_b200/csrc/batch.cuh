@@ -19,6 +19,8 @@ struct BCtl {   // per-instance control state (device resident)
   long long updown_ranks;        // sum of ranks over the sweeps
   long long syrk_entries;        // persistent engine: rows of A streamed through the H SYRK, summed over the refactorisations
   int n_scratch;                 // persistent engine: refactorisations that rebuilt H from c Q
+  long long ls_breakpoints;      // persistent engine: line-search breakpoints with s > 0 (nL), summed over the line searches
+  long long ls_walked;           // persistent engine: sorted breakpoints the walk read before it stopped, summed likewise
 };
 
 struct BSet {   // settings the device needs (copied by value into kernels)
@@ -96,6 +98,7 @@ struct BpProbeArgs {
 };
 int batchp_probe_newton(const BpProbeArgs &P, cudaStream_t s);
 int batchp4_probe_newton(const BpProbeArgs &P, cudaStream_t s);
-int batchp_probe_sort(int nb, int N, unsigned long long *keys, unsigned int *vals, int *queue, cudaStream_t s);
-int batchp4_probe_sort(int nb, int N, unsigned long long *keys, unsigned int *vals, int *queue, cudaStream_t s);
+// the line-search sort: keys (nb x N) sorted in place, vals_out (nb x N) <- vals permuted alike
+int batchp_probe_sort(int nb, int N, unsigned long long *keys, const unsigned int *vals, unsigned int *vals_out, int *queue, cudaStream_t s);
+int batchp4_probe_sort(int nb, int N, unsigned long long *keys, const unsigned int *vals, unsigned int *vals_out, int *queue, cudaStream_t s);
 }  // namespace qb

@@ -12,8 +12,8 @@
 // (2 x 230 KB each) do not fit the L2 and stream from HBM, which is why every pass over them is written as a batch of
 // requests (cp.async, eight loads in flight, rows requested one block ahead) rather than load -> use.  Shared memory per CTA
 // (72 KB at 3 CTAs / SM, 55 KB at 4) holds one panel of the factor (Cholesky, triangular solves), the SYRK's double-buffered rows of A' -- or, during an
-// update sweep, the rows of W, the chain warp's ring of window blocks and the row owners' staging ring --, the radix-sort
-// buffers of the line search (2m <= 2048 keys) and the staged GEMV operand.
+// update sweep, the rows of W, the chain warp's ring of window blocks and the row owners' staging ring --, the line search's
+// two merge-sort buffers of (key, position) pairs (its nL <= 2m <= 2048 breakpoints s > 0) and the staged GEMV operand.
 //
 // The Newton system (Q + A_J' Sigma_J A_J + I/gamma) d = -dphi  (src/newton.c:96-118, solver_interface.c:319-519):
 //   H is kept per instance and updated incrementally (+ entering / - leaving / +- sigma changes) or rebuilt from c Q by an in-CTA
@@ -28,16 +28,19 @@
 #include "chol32.cuh"
 #include <math.h>
 #include <string.h>
+#ifdef QB_BP_DEBUG   // device-side checks of the engine's invariants (-DQB_BP_DEBUG through QB_EXTRA_FLAGS)
+#include <assert.h>
+#endif
 
 using namespace qb;
 
 // Build-time shape of a CTA; this file is compiled twice (build.sh), and each shape once more with -DQB_BP_PROBE, which
 // replaces the solver kernel by the test probes of its building blocks (see kbp_probe_newton):
-//   default            8 warps, 32-column panel (16-wide sub-panels), both sort buffers in shared memory: 80 registers x 256
-//                      threads, 72 KB -> 3 CTAs / SM (444 slots on a B200).  Best per-wave throughput: 444 instances in
-//                      57.9 ms (7675 solves/s), 4096 instances in 488 ms (8396 solves/s) at the end of round 2.
-//   -DQB_BP_VARIANT4   8 warps, 24-column panel (-DQB_BP_SW=8: 8-wide sub-panels), one sort buffer in shared memory and the other
-//                      in the instance's global arrays, registers capped at 64: 55 KB -> 4 CTAs / SM (592 slots).  Slower per
+//   default            8 warps, 32-column panel (16-wide sub-panels): 80 registers x 256 threads, 72 KB -> 3 CTAs / SM (444
+//                      slots on a B200).  Best per-wave throughput: 444 instances in 57.9 ms (7675 solves/s), 4096 instances
+//                      in 488 ms (8396 solves/s) at the end of round 2.
+//   -DQB_BP_VARIANT4   8 warps, 24-column panel (-DQB_BP_SW=8: 8-wide sub-panels), registers capped at 64: 55 KB -> 4 CTAs / SM
+//                      (592 slots).  Both sort buffers (40 KB) fit the union region of either shape.  Slower per
 //                      instance (64 registers: several loops are shaped around that, see QB_BP_SW and p_gemv_rows) but the
 //                      BASELINE sweep of 512 instances per GPU fits in ONE wave: 78.8 ms against 90.3 ms with the 68-instance
 //                      tail of the default shape.  batch.cu picks it when 3 * SMs < nb <= 4 * SMs.
@@ -57,7 +60,6 @@ using namespace qb;
 #ifndef QB_BP_PW
 #define QB_BP_PW 24
 #endif
-#define QB_BP_SORT_GLOBAL 1
 #define QB_BP_MINB 4
 #else
 #define QB_BP_NAMESPACE bp
@@ -80,9 +82,6 @@ using namespace qb;
 #ifndef QB_BP_PW
 #define QB_BP_PW 32
 #endif
-#ifndef QB_BP_SORT_GLOBAL
-#define QB_BP_SORT_GLOBAL 0
-#endif
 namespace qb {
 namespace QB_BP_NAMESPACE {
 
@@ -92,8 +91,10 @@ constexpr int NMAX = 240;         // largest n of this engine (panel = PW x LDP 
 constexpr int LDP = NMAX + 1;     // odd leading dimension: conflict-free row and column access
 static_assert(NMAX <= NT, "the update sweep maps thread t to row t of the factor");
 constexpr int SORT_MAX = 2048;    // largest 2m
+static_assert(SORT_MAX <= 8 * NT && SORT_MAX <= 65536, "the sort's register runs (8 per thread) cover SORT_MAX; positions fit 16 bits");
 constexpr int VS_LEN = (QB_BP_PW == 32) ? 1024 : 960;   // staged GEMV operand (max(n, m) doubles)
-constexpr size_t kSortBytes = (size_t)SORT_MAX * (QB_BP_SORT_GLOBAL ? 1 : 2) * (8 + 4) + sizeof(unsigned) * (NW * 256 + 256 + 256);
+// the line search's two ping-pong buffers of SORT_MAX (u64 key, u16 position) pairs (ls_keys / ls_pos)
+constexpr size_t kSortBytes = (size_t)SORT_MAX * 2 * (sizeof(unsigned long long) + sizeof(unsigned short));
 constexpr size_t kPanelBytes = sizeof(double) * PW * LDP;
 constexpr size_t kUnionBytes = kSortBytes > kPanelBytes ? kSortBytes : kPanelBytes;
 constexpr size_t kSmemBytes = kUnionBytes + sizeof(double) * (VS_LEN + NMAX + 16 + 2 * PW);
@@ -112,7 +113,7 @@ struct Args {
   double *sigmaH, *w_pos, *w_neg;
   double *H, *L, *rdiag;
   long long sLL, sR;
-  unsigned long long *keys; unsigned int *vals; double *ls_da, *ls_db;
+  double *ls_da, *ls_db;
   double *scal;
   BCtl *ctl;
   int *queue;
@@ -130,6 +131,13 @@ struct Smem {
   double *v;             // Newton rhs / solution (NMAX + 16)
   double *rd;            // 1 / l_jj of the current panel (PW), spare (PW)
 };
+// the line search's (key, position) buffers 0 and 1 in the union region (kSortBytes)
+__device__ __forceinline__ unsigned long long *ls_keys(const Smem &S, int buf) {
+  return reinterpret_cast<unsigned long long *>(S.u) + (size_t)buf * SORT_MAX;
+}
+__device__ __forceinline__ unsigned short *ls_pos(const Smem &S, int buf) {
+  return reinterpret_cast<unsigned short *>(S.u + 2 * SORT_MAX * sizeof(unsigned long long)) + (size_t)buf * SORT_MAX;
+}
 
 // ------------------------------------------------------------------------------------------------
 // small helpers
@@ -1647,9 +1655,16 @@ __device__ __noinline__ void p_boost(const Args &P, int b, double *scratch, cons
 // ------------------------------------------------------------------------------------------------
 // line search (linesearch.c:14-120)
 // ------------------------------------------------------------------------------------------------
-__device__ __noinline__ void p_ls_build(const Args &P, int b, double *part) {
-  const int n = P.n, m = P.m;
+// The breakpoints s > 0 (+inf included) go to buffer 0 of the sort as (bit pattern of s, index) pairs, compacted: a warp
+// takes its slots with one shared atomic, so their order varies from run to run, which the sort's total order makes
+// irrelevant.  The others (s <= 0 or NaN) are never walked by p_ls_select and are not stored.  Their count is S_NL.
+__device__ __noinline__ void p_ls_build(const Args &P, int b, double *part, const Smem &S) {
+  __shared__ unsigned n_brk;
+  const int n = P.n, m = P.m, lane = threadIdx.x & 31;
   const size_t on = (size_t)b * n, om = (size_t)b * m, o2 = (size_t)b * 2 * m;
+  unsigned long long *bk = ls_keys(S, 0);
+  unsigned short *bp = ls_pos(S, 0);
+  if (threadIdx.x == 0) n_brk = 0;
   const double inv_gamma = 1 / P.ctl[b].gamma;
   double eta = 0, beta = 0;
   for (int j = threadIdx.x; j < n; j += NT) {
@@ -1658,120 +1673,147 @@ __device__ __noinline__ void p_ls_build(const Args &P, int b, double *part) {
     if (P.st.proximal) { qd = qd + inv_gamma * dj; P.Qd[on + j] = qd; }
     eta += dj * qd; beta += dj * P.df[on + j];
   }
+  __syncthreads();   // n_brk = 0 before the first slot is taken
   double a_part = 0, b_part = 0, n_l = 0;
-  for (int i = threadIdx.x; i < m; i += NT) {
-    const double ss = P.sqrt_sigma[om + i], sg = P.sigma[om + i], ax = P.Ax[om + i], yi = P.y[om + i];
-    const double t = ss * P.Ad[om + i];
-    double dl[2], al[2];
-    dl[1] = t; dl[0] = t * -1;
-    double u = ax - P.bmin[om + i]; u = sg * u; u = yi + u; al[0] = u / ss;
-    u = P.bmax[om + i] - ax; u = sg * u; u = u - yi; al[1] = u / ss;
+  for (int i0 = 0; i0 < m; i0 += NT) {   // whole warps per step: the ballots below
+    const int i = i0 + threadIdx.x;
+    bool inL[2] = {false, false};
+    double sv[2] = {0.0, 0.0};
+    if (i < m) {
+      const double ss = P.sqrt_sigma[om + i], sg = P.sigma[om + i], ax = P.Ax[om + i], yi = P.y[om + i];
+      const double t = ss * P.Ad[om + i];
+      double dl[2], al[2];
+      dl[1] = t; dl[0] = t * -1;
+      double u = ax - P.bmin[om + i]; u = sg * u; u = yi + u; al[0] = u / ss;
+      u = P.bmax[om + i] - ax; u = sg * u; u = u - yi; al[1] = u / ss;
 #pragma unroll
-    for (int hh = 0; hh < 2; hh++) {
-      const int idx = i + hh * m;
-      const double s = al[hh] / dl[hh];
-      const bool inL = s > 0, inP = dl[hh] > 0;
-      P.keys[o2 + idx] = inL ? (unsigned long long)__double_as_longlong(s) : ~0ull;
-      P.vals[o2 + idx] = (unsigned int)idx;
-      const double d2 = dl[hh] * dl[hh], dalp = dl[hh] * al[hh];
-      P.ls_da[o2 + idx] = inP ? d2 : -d2;
-      P.ls_db[o2 + idx] = inP ? -dalp : dalp;
-      if ((int)inL + (int)inP == 1) { a_part += d2; b_part += dalp; }
-      n_l += inL;
+      for (int hh = 0; hh < 2; hh++) {
+        const int idx = i + hh * m;
+        const double s = al[hh] / dl[hh];
+        const bool inP = dl[hh] > 0;
+        inL[hh] = s > 0; sv[hh] = s;
+        const double d2 = dl[hh] * dl[hh], dalp = dl[hh] * al[hh];
+        P.ls_da[o2 + idx] = inP ? d2 : -d2;
+        P.ls_db[o2 + idx] = inP ? -dalp : dalp;
+        if ((int)inL[hh] + (int)inP == 1) { a_part += d2; b_part += dalp; }
+        n_l += inL[hh];
+      }
     }
+    const unsigned b0 = __ballot_sync(0xffffffffu, inL[0]), b1 = __ballot_sync(0xffffffffu, inL[1]);
+    unsigned at = 0;
+    if (lane == 0 && (b0 | b1)) at = atomicAdd(&n_brk, (unsigned)(__popc(b0) + __popc(b1)));
+    at = __shfl_sync(0xffffffffu, at, 0);
+    const unsigned lt = (1u << lane) - 1u;
+    if (inL[0]) { const unsigned k = at + __popc(b0 & lt); bk[k] = (unsigned long long)__double_as_longlong(sv[0]); bp[k] = (unsigned short)i; }
+    if (inL[1]) { const unsigned k = at + __popc(b0) + __popc(b1 & lt); bk[k] = (unsigned long long)__double_as_longlong(sv[1]); bp[k] = (unsigned short)(i + m); }
   }
   const double vals[5] = {eta, beta, a_part, b_part, n_l};
   const int ops[5] = {RED_SUM, RED_SUM, RED_SUM, RED_SUM, RED_SUM};
   const int slots[5] = {S_ETA, S_BETA, S_LS_A, S_LS_B, S_NL};
   block_red_multi<5>(P, b, vals, ops, slots, part);
-}
-
-// stable LSD radix sort of N <= SORT_MAX (key, val) pairs in shared memory; sorted pairs are written back to global
-__device__ __forceinline__ void p_sort(int N, unsigned long long *kg, unsigned int *vg, const Smem &S) {
-  // ping-pong between ONE shared-memory buffer and the instance's global (kg, vg) arrays (L2-resident, 23 KB): a second
-  // shared buffer would cost the fourth CTA per SM
-#if QB_BP_SORT_GLOBAL
-  unsigned long long *k0 = reinterpret_cast<unsigned long long *>(S.u);
-  unsigned int *v0 = reinterpret_cast<unsigned int *>(k0 + SORT_MAX);
-  unsigned int *warp_cnt = v0 + SORT_MAX;            // [NW][256]
-  unsigned long long *kalt = kg;
-  unsigned int *valt = vg;
-#else
-  unsigned long long *k0 = reinterpret_cast<unsigned long long *>(S.u), *kalt = k0 + SORT_MAX;
-  unsigned int *v0 = reinterpret_cast<unsigned int *>(kalt + SORT_MAX), *valt = v0 + SORT_MAX;
-  unsigned int *warp_cnt = valt + SORT_MAX;          // [NW][256]
+#ifdef QB_BP_DEBUG
+  __syncthreads();
+  if (threadIdx.x == 0) assert(n_brk == (unsigned)BSC(b, S_NL));
 #endif
-  unsigned int *running = warp_cnt + NW * 256;       // [256]
-  unsigned int *hist = running + 256;                // [256]
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  for (int i = tid; i < N; i += NT) { k0[i] = kg[i]; v0[i] = vg[i]; }
-  __syncthreads();
-  unsigned long long *kin = k0, *kout = kalt;
-  unsigned int *vin = v0, *vout = valt;
-  for (int pass = 0; pass < 8; pass++) {
-    const int shift = pass * 8;
-    for (int d = tid; d < 256; d += NT) hist[d] = 0;
-    __syncthreads();
-    for (int i = tid; i < N; i += NT) atomicAdd(&hist[(unsigned)(kin[i] >> shift) & 255u], 1u);
-    __syncthreads();
-    if (hist[(unsigned)(kin[0] >> shift) & 255u] == (unsigned)N) { __syncthreads(); continue; }   // all keys share this digit
-    if (warp == 0) {
-      unsigned int loc[8], sum = 0;
-#pragma unroll
-      for (int t = 0; t < 8; t++) { loc[t] = hist[lane * 8 + t]; sum += loc[t]; }
-      unsigned int inc = sum;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) { const unsigned int u = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += u; }
-      unsigned int run = inc - sum;
-#pragma unroll
-      for (int t = 0; t < 8; t++) { running[lane * 8 + t] = run; run += loc[t]; }
-    }
-    __syncthreads();
-    for (int start = 0; start < N; start += NT) {
-      for (int i = tid; i < NW * 256; i += NT) warp_cnt[i] = 0;
-      __syncthreads();
-      const int e = start + tid;
-      const bool valid = e < N;
-      unsigned long long k = 0; unsigned int v = 0; unsigned int dg = 0x10000u + lane;
-      if (valid) { k = kin[e]; v = vin[e]; dg = (unsigned)(k >> shift) & 255u; }
-      const unsigned peers = __match_any_sync(0xffffffffu, dg);
-      const int rank = __popc(peers & ((1u << lane) - 1u));
-      if (valid && rank == 0) warp_cnt[warp * 256 + dg] = __popc(peers);
-      __syncthreads();
-      if (valid) {
-        unsigned int off = running[dg];
-        for (int w = 0; w < warp; w++) off += warp_cnt[w * 256 + dg];
-        kout[off + rank] = k; vout[off + rank] = v;
-      }
-      __syncthreads();
-      for (int d = tid; d < 256; d += NT) {
-        unsigned int t = 0;
-#pragma unroll
-        for (int w = 0; w < NW; w++) t += warp_cnt[w * 256 + d];
-        running[d] += t;
-      }
-      __syncthreads();
-    }
-    unsigned long long *tk = kin; kin = kout; kout = tk;
-    unsigned int *tv = vin; vin = vout; vout = tv;
-  }
-  __syncthreads();
-  if (kin != kg) for (int i = tid; i < N; i += NT) { kg[i] = kin[i]; vg[i] = vin[i]; }
 }
 
-__device__ __noinline__ void p_ls_select(const Args &P, int b) {
+// (ka, pa) < (kb, pb) lexicographically.  The positions of one sort are distinct, so this is a total order and every sort by
+// it returns the permutation of a stable sort by key.  Keys compare as unsigned integers: for positive doubles and +inf that
+// is the order of the values.
+__device__ __forceinline__ bool kp_less(unsigned long long ka, unsigned pa, unsigned long long kb, unsigned pb) {
+  return (ka < kb) | ((ka == kb) & (pa < pb));   // no short circuit: predicates, not branches, in the network and the merges
+}
+
+// Sorts the N <= SORT_MAX (key, position) pairs of buffer 0 by kp_less; the result is in buffer 0.  Thread t sorts pairs
+// [8 t, 8 t + 8) in registers (a 19-comparator network), then each merge level doubles the run length: thread t writes
+// outputs [8 t, 8 t + 8) of its pair of runs, starting where a binary search of the merge path puts it.  One barrier per level
+// (8 at N = 2048).  The register stage writes to buffer (number of levels & 1), so the last level lands in buffer 0.
+__device__ __noinline__ void p_ls_sort(int N, const Smem &S) {
+  const int tid = threadIdx.x, o0 = 8 * tid;
+  int levels = 0;
+  for (int w = 8; w < N; w <<= 1) levels++;
+  int buf = levels & 1;
+  if (o0 < N) {
+    const unsigned long long *ki = ls_keys(S, 0);
+    const unsigned short *pi = ls_pos(S, 0);
+    unsigned long long k[8];
+    unsigned p[8];
+#pragma unroll
+    for (int u = 0; u < 8; u++) {   // past N: (~0, 0xFFFF) sorts after every pair of the input (positions < SORT_MAX)
+      k[u] = o0 + u < N ? ki[o0 + u] : ~0ull;
+      p[u] = o0 + u < N ? pi[o0 + u] : 0xFFFFu;
+    }
+    constexpr int NET[19][2] = {{0, 2}, {1, 3}, {4, 6}, {5, 7}, {0, 4}, {1, 5}, {2, 6}, {3, 7}, {0, 1}, {2, 3},
+                                {4, 5}, {6, 7}, {2, 4}, {3, 5}, {1, 4}, {3, 6}, {1, 2}, {3, 4}, {5, 6}};
+#pragma unroll
+    for (int c = 0; c < 19; c++) {
+      const int x = NET[c][0], y = NET[c][1];
+      const bool sw = kp_less(k[y], p[y], k[x], p[x]);
+      const unsigned long long kx = k[x];
+      const unsigned px = p[x];
+      k[x] = sw ? k[y] : k[x]; p[x] = sw ? p[y] : p[x];
+      k[y] = sw ? kx : k[y]; p[y] = sw ? px : p[y];
+    }
+    unsigned long long *ko = ls_keys(S, buf);
+    unsigned short *po = ls_pos(S, buf);
+#pragma unroll
+    for (int u = 0; u < 8; u++)
+      if (o0 + u < N) { ko[o0 + u] = k[u]; po[o0 + u] = (unsigned short)p[u]; }
+  }
+  for (int w = 8; w < N; w <<= 1) {
+    __syncthreads();
+    const unsigned long long *ki = ls_keys(S, buf);
+    const unsigned short *pi = ls_pos(S, buf);
+    unsigned long long *ko = ls_keys(S, buf ^ 1);
+    unsigned short *po = ls_pos(S, buf ^ 1);
+    if (o0 < N) {   // runs A = [a0, a0 + na), B = [a0 + w, a0 + w + nb); this thread's outputs start at d in their merge
+      const int a0 = o0 & ~(2 * w - 1), b0 = a0 + w, d = o0 - a0;
+      const int na = min(w, N - a0), nb = max(0, min(w, N - b0));
+      int lo = max(0, d - nb), hi = min(d, na);
+      while (lo < hi) {   // the number of A pairs among the first d outputs
+        const int mid = (lo + hi) >> 1;
+        if (kp_less(ki[a0 + mid], pi[a0 + mid], ki[b0 + d - mid - 1], pi[b0 + d - mid - 1])) lo = mid + 1;
+        else hi = mid;
+      }
+      int ia = lo, ib = d - lo;
+      // heads of the two runs; an exhausted run's head (~0, 0x10000) is greater than every pair
+      unsigned long long ka = ia < na ? ki[a0 + ia] : ~0ull, kb = ib < nb ? ki[b0 + ib] : ~0ull;
+      unsigned pa = ia < na ? pi[a0 + ia] : 0x10000u, pb = ib < nb ? pi[b0 + ib] : 0x10000u;
+      const int cnt = min(8, N - o0);
+#pragma unroll
+      for (int u = 0; u < 8; u++) {
+        if (u < cnt) {
+          const bool ta = kp_less(ka, pa, kb, pb);
+          ko[o0 + u] = ta ? ka : kb; po[o0 + u] = (unsigned short)(ta ? pa : pb);
+          if (ta) { ia++; ka = ia < na ? ki[a0 + ia] : ~0ull; pa = ia < na ? pi[a0 + ia] : 0x10000u; }
+          else { ib++; kb = ib < nb ? ki[b0 + ib] : ~0ull; pb = ib < nb ? pi[b0 + ib] : 0x10000u; }
+        }
+      }
+    }
+    buf ^= 1;
+  }
+}
+
+// Walks the sorted breakpoints (p_ls_sort's buffer 0; nothing may write the union region in between) in chunks of NT,
+// carrying the running (a, b) sums; tau = -b / a at the first breakpoint where a s + b > 0.
+__device__ __noinline__ void p_ls_select(const Args &P, int b, const Smem &S) {
   __shared__ double wa[NW], wb[NW];
   __shared__ double carry_a, carry_b;
   __shared__ int found;
   const size_t o2 = (size_t)b * 2 * P.m;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int nL = (int)BSC(b, S_NL);
-  if (tid == 0) { carry_a = BSC(b, S_ETA) + BSC(b, S_LS_A); carry_b = BSC(b, S_BETA) - BSC(b, S_LS_B); found = 0x7fffffff; }
+  const unsigned long long *sk = ls_keys(S, 0);
+  const unsigned short *sp = ls_pos(S, 0);
+  if (tid == 0) {
+    carry_a = BSC(b, S_ETA) + BSC(b, S_LS_A); carry_b = BSC(b, S_BETA) - BSC(b, S_LS_B); found = 0x7fffffff;
+    P.ctl[b].ls_breakpoints += nL;
+  }
   __syncthreads();
   for (int start = 0; start < nL; start += NT) {
     const int i = start + tid;
     double ta = 0.0, tb = 0.0, s = 0.0;
-    if (i < nL) { const unsigned int idx = P.vals[o2 + i]; ta = P.ls_da[o2 + idx]; tb = P.ls_db[o2 + idx]; s = __longlong_as_double((long long)P.keys[o2 + i]); }
+    if (i < nL) { const unsigned int idx = sp[i]; ta = P.ls_da[o2 + idx]; tb = P.ls_db[o2 + idx]; s = __longlong_as_double((long long)sk[i]); }
     double ia = ta, ib = tb;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
@@ -1788,13 +1830,13 @@ __device__ __noinline__ void p_ls_select(const Args &P, int b) {
     if (i < nL && (a_i * s + b_i > 0)) atomicMin(&found, i);
     __syncthreads();
     if (found != 0x7fffffff) {
-      if (i == found) BSC(b, S_TAU) = -b_i / a_i;
+      if (i == found) { BSC(b, S_TAU) = -b_i / a_i; P.ctl[b].ls_walked += i + 1; }
       return;
     }
     if (tid == NT - 1) { carry_a += oa + ia; carry_b += ob + ib; }
     __syncthreads();
   }
-  if (tid == 0) BSC(b, S_TAU) = -carry_b / carry_a;
+  if (tid == 0) { BSC(b, S_TAU) = -carry_b / carry_a; P.ctl[b].ls_walked += nL; }
 }
 
 __device__ void p_update_iterate(const Args &P, int b) {
@@ -1953,13 +1995,13 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_solve(const Args P) {
         p_gemv_rows(m, n, m, P.Am, P.d + on, P.Ad + om, 1.0, S);
         __syncthreads();
         PH(9);
-        p_ls_build(P, b, S.vs);
+        p_ls_build(P, b, S.vs, S);
         __syncthreads();
         PH(10);
-        p_sort(2 * m, P.keys + (size_t)b * 2 * m, P.vals + (size_t)b * 2 * m, S);
+        p_ls_sort((int)BSC(b, S_NL), S);
         __syncthreads();
         PH(11);
-        p_ls_select(P, b);
+        p_ls_select(P, b, S);
         __syncthreads();
         p_update_iterate(P, b);
         __syncthreads();
@@ -2076,8 +2118,10 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_probe_newton(const BpProbe
   }
 }
 
-// p_sort on instance b's N (key, val) pairs at keys + b N, vals + b N, in place
-__global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_probe_sort(int nb, int N, unsigned long long *keys, unsigned int *vals, int *queue) {
+// p_ls_sort on instance b's N (key, val) pairs at keys + b N, vals + b N, loaded the way p_ls_build leaves them (position =
+// index in the array): the keys are sorted in place, vals_out + b N receives the vals in the sorted order
+__global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_probe_sort(int nb, int N, unsigned long long *keys, const unsigned int *vals,
+                                                                 unsigned int *vals_out, int *queue) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ int s_b;
   const Smem S = probe_smem(smem_raw);
@@ -2087,7 +2131,12 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_probe_sort(int nb, int N, 
     __syncthreads();
     const int b = s_b;
     if (b >= nb) return;
-    p_sort(N, keys + (size_t)b * N, vals + (size_t)b * N, S);
+    unsigned long long *kb = keys + (size_t)b * N;
+    for (int i = threadIdx.x; i < N; i += NT) { ls_keys(S, 0)[i] = kb[i]; ls_pos(S, 0)[i] = (unsigned short)i; }
+    __syncthreads();
+    p_ls_sort(N, S);
+    __syncthreads();
+    for (int i = threadIdx.x; i < N; i += NT) { kb[i] = ls_keys(S, 0)[i]; vals_out[(size_t)b * N + i] = vals[(size_t)b * N + ls_pos(S, 0)[i]]; }
   }
 }
 
@@ -2130,7 +2179,7 @@ int QB_BP_SOLVE(QPALMB200Batch *B, int nb, int nwarm, int wx, int wy) {
   P.sLL = (long long)B->ld * B->npad; P.sR = (long long)B->npad * kPanel;
   P.prof = B->prof;
   P.nwarm = nwarm; P.x_ws = wx ? B->x_ws : nullptr; P.y_ws = wy ? B->y_ws : nullptr;
-  P.keys = B->keys; P.vals = B->vals; P.ls_da = B->ls_da; P.ls_db = B->ls_db; P.scal = B->scal; P.ctl = B->ctl; P.queue = B->queue;
+  P.ls_da = B->ls_da; P.ls_db = B->ls_db; P.scal = B->scal; P.ctl = B->ctl; P.queue = B->queue;
   static int ctas_per_sm = 0, num_sms = 0;
   if (!ctas_per_sm) {
     QB_CUDA_TRY(cudaFuncSetAttribute(kbp_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
@@ -2160,13 +2209,13 @@ int QB_BP_PROBE_NEWTON(const BpProbeArgs &P, cudaStream_t s) {
   return 0;
 }
 
-int QB_BP_PROBE_SORT(int nb, int N, unsigned long long *keys, unsigned int *vals, int *queue, cudaStream_t s) {
+int QB_BP_PROBE_SORT(int nb, int N, unsigned long long *keys, const unsigned int *vals, unsigned int *vals_out, int *queue, cudaStream_t s) {
   using namespace QB_BP_NAMESPACE;
   if (nb < 1 || N < 1 || N > SORT_MAX) return 1;
   int grid = 0;
   if (int r = probe_grid((const void *)kbp_probe_sort, nb, &grid)) return r;
   QB_CUDA_TRY(cudaMemsetAsync(queue, 0, sizeof(int), s));
-  QB_LAUNCH(kbp_probe_sort, grid, NT, kSmemBytes, s, nb, N, keys, vals, queue);
+  QB_LAUNCH(kbp_probe_sort, grid, NT, kSmemBytes, s, nb, N, keys, vals, vals_out, queue);
   QB_CUDA_TRY(cudaGetLastError());
   return 0;
 }

@@ -32,5 +32,8 @@ print(f"per instance: refactorizations {st['refactorizations']/nb:.1f}, update s
 nr = max(st["refactorizations"], 1)
 print(f"H syrk: {st['syrk_entries']/nr:.1f} list entries per refactorization, scratch rebuilds {st['scratch_rebuilds']/nb:.1f} "
       f"per instance ({100*st['scratch_rebuilds']/nr:.0f}% of the refactorizations)")
+nls = max(st["inner"], 1)
+print(f"line search: {st['ls_breakpoints']/nls:.1f} breakpoints sorted (s > 0 of 2m = {2*b.A.nrow}), {st['ls_walked']/nls:.1f} walked, "
+      f"per line search ({100*st['ls_walked']/max(st['ls_breakpoints'], 1):.1f}% of the sorted ones)")
 for k in list(range(32)):
     print(f"{names[k]:22s} {out[:,k].mean()/1.965e3:10.1f} us/instance  {100*out[:,k].sum()/tot.sum():6.2f}%   per-iter {out[:,k].sum()/iters.sum()/1.965e3:7.2f} us")
