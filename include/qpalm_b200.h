@@ -287,6 +287,25 @@ void  qpalm_b200_symbolic_free(QPALMB200Symbolic *S);
 int qpalm_b200_sparse_newton(const solver_sparse *Q, const solver_sparse *A, const c_float *sigma, const c_int *active,
         c_float beta, const c_float *rhs, c_float *d, c_float *L_out, c_int *perm_out, const c_int *enter, c_int nb_enter,
         const c_int *leave, c_int nb_leave, c_float *rowsums_out);
+/* Signed (L S L') supernodal factorization of a symmetric QUASI-DEFINITE matrix -- the factorization the KKT Newton path runs
+ * (csrc/kkt.cu), on a caller's matrix.  K: N x N, lower triangle in CSC (stype -1; rows strictly ascending per column, stored
+ * zeros stay in the pattern); original columns >= n_pos carry negative pivots (S = diag(+-1) in the permuted order).  One
+ * symbolic analysis, assembly, factorization and ONE solve  x = K^{-1} rhs  without iterative refinement.  Optional outputs:
+ * L_out (N x N column-major, PERMUTED order, lower factor with positive diagonal, K(perm, perm) = L S L') together with perm_out
+ * (perm[new] = old); panels_out receives the raw factor panels when panels_cap >= their length, which is written to
+ * *panels_len.  Returns 0, 1000 + info when a pivot did not have its a-priori sign (info - 1: a permuted column in the
+ * front of such a pivot or in a front above it), 1 / 2 for invalid arguments, or -(cudaError_t). */
+int qpalm_b200_sparse_ldl(const solver_sparse *K, c_int n_pos, const c_float *rhs, c_float *x, c_float *L_out,
+        c_int *perm_out, c_float *panels_out, c_int panels_cap, c_int *panels_len);
+/* The solver's KKT Newton step at given inputs (FACTORIZE_KKT, csrc/kkt.cu): the values of
+ * [Q + beta I, A_J'; A_J, -inv(Sigma_J)] (inactive rows: a decoupled -1), L S L', one solve and up to three iterative-
+ * refinement corrections, i.e. d = (Q + A_J' Sigma_J A_J + beta I)^{-1} rhs.  A must have at least one row and both matrices
+ * sparse storage.  refine_out (optional): corrections this solve applied; norms_out (optional, 2): {|res|inf, ref} of the
+ * last residual, refinement stops once |res|inf <= max(1e-10 ref, 1e-12).  Returns 0, 7 when the data do not take the KKT
+ * path (dense-classified A or Q), 1000 + info on a pivot without its a-priori sign, 1 for invalid arguments, or
+ * -(cudaError_t). */
+int qpalm_b200_kkt_newton(const solver_sparse *Q, const solver_sparse *A, const c_float *sigma, const c_int *active,
+        c_float beta, const c_float *rhs, c_float *d, c_int *refine_out, c_float *norms_out);
 
 /* lambda_min estimate -- replaces lobpcg (nonconvex.c:29-168).  x0 is the (un-normalised) start
  * vector the reference draws with rand(); returns the under-estimate the reference returns. */

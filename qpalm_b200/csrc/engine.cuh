@@ -187,6 +187,7 @@ int kkt_solve(KktEngine *K, Engine *e);                   // e->d from K z = [-d
 long long kkt_factor_nnz(const KktEngine *K);
 long long kkt_factor_count(const KktEngine *K);
 long long kkt_refine_count(const KktEngine *K);
+void kkt_last_norms(const KktEngine *K, double out2[2]);   // {|res|inf, ref} of the last residual kkt_solve formed
 
 // ---- LOBPCG (nonconvex.c:29-168) ---------------------------------------------------------------------
 int lobpcg_device(Engine *e, const double *x0_host, double *lambda_out, long long *iters_out);

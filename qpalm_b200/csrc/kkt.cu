@@ -195,6 +195,7 @@ void kkt_destroy(KktEngine *K) {
 long long kkt_factor_nnz(const KktEngine *K) { return K ? sparse_chol_info(K->sp)->nnzL : 0; }
 long long kkt_factor_count(const KktEngine *K) { return K ? K->n_factor : 0; }
 long long kkt_refine_count(const KktEngine *K) { return K ? K->n_refine : 0; }
+void kkt_last_norms(const KktEngine *K, double out2[2]) { out2[0] = K->norms_host[0]; out2[1] = K->norms_host[1]; }
 
 // values of K for the committed active set, then L S L'  (qpalm_form_kkt / qpalm_reform_kkt + ladel_factorize*)
 int kkt_refactor(KktEngine *K, Engine *e, double beta) {

@@ -343,6 +343,111 @@ extern "C" int qpalm_b200_sparse_newton(const solver_sparse *Q, const solver_spa
   return rc ? rc : (info ? 1000 + info : 0);
 }
 
+namespace {
+struct LdlBuffers {   // device buffers of one sparse_ldl call, released on every return path
+  SparseChol *sp = nullptr;
+  cudaStream_t st = nullptr;
+  int *Kp = nullptr, *Ki = nullptr, *info = nullptr;
+  double *Kx = nullptr, *panels = nullptr, *rhs = nullptr, *x = nullptr;
+  ~LdlBuffers() {
+    if (st) cudaStreamSynchronize(st);
+    sparse_chol_destroy(sp);
+    void *ptrs[] = {Kp, Ki, info, Kx, panels, rhs, x};
+    for (void *p : ptrs) if (p) cudaFree(p);
+    if (st) cudaStreamDestroy(st);
+  }
+};
+}  // namespace
+
+extern "C" int qpalm_b200_sparse_ldl(const solver_sparse *K, c_int n_pos, const c_float *rhs, c_float *x, c_float *L_out,
+        c_int *perm_out, c_float *panels_out, c_int panels_cap, c_int *panels_len) {
+  if (!K || !rhs || !x || K->nrow != K->ncol || K->ncol < 1 || K->ncol > (1 << 30) || n_pos < 0 || n_pos > K->ncol) return 1;
+  const int N = (int)K->ncol;
+  const long long *Kp = (const long long *)K->p, *Ki = (const long long *)K->i;
+  const double *Kv = (const double *)K->x;
+  // lower triangle, strictly ascending rows per column: the assembly stores (does not add) each entry, so a duplicate would be lost
+  std::vector<int> cnt((size_t)N + 1, 0);
+  for (int j = 0; j < N; j++) {
+    if (Kp[j + 1] < Kp[j]) return 2;
+    long long last = -1;
+    for (long long k = Kp[j]; k < Kp[j + 1]; k++) {
+      const long long i = Ki[k];
+      if (i < 0 || i >= N || i <= last) return 2;
+      last = i;
+      if (i < j) continue;
+      cnt[i]++;
+      if (i != j) cnt[j]++;
+    }
+  }
+  // full symmetric CSR (row i: entries (i, j <= i) in ascending j, then (i, k > i) in ascending k), as the engine keeps Q
+  std::vector<int> rp((size_t)N + 1, 0);
+  for (int i = 0; i < N; i++) rp[i + 1] = rp[i] + cnt[i];
+  const size_t nnzF = (size_t)rp[N];
+  std::vector<int> rj(nnzF + 1), fill(rp.begin(), rp.end());
+  std::vector<double> rx(nnzF + 1);
+  for (int j = 0; j < N; j++) for (long long k = Kp[j]; k < Kp[j + 1]; k++) if (Ki[k] >= j) { const int p = fill[Ki[k]]++; rj[p] = j; rx[p] = Kv[k]; }
+  for (int j = 0; j < N; j++) for (long long k = Kp[j]; k < Kp[j + 1]; k++) if (Ki[k] > j) { const int p = fill[j]++; rj[p] = (int)Ki[k]; rx[p] = Kv[k]; }
+
+  LdlBuffers b;
+  QB_CUDA_TRY(cudaStreamCreate(&b.st));
+  if (int r = sparse_ldl_analyze(&b.sp, N, (int)n_pos, Kp, Ki, b.st)) return r;
+  const SparseCholInfo *I = sparse_chol_info(b.sp);
+  if (panels_len) *panels_len = (c_int)I->nnzL;
+  QB_CUDA_TRY(cudaMalloc((void **)&b.Kp, sizeof(int) * ((size_t)N + 1)));
+  QB_CUDA_TRY(cudaMalloc((void **)&b.Ki, sizeof(int) * (nnzF + 1)));
+  QB_CUDA_TRY(cudaMalloc((void **)&b.Kx, sizeof(double) * (nnzF + 1)));
+  QB_CUDA_TRY(cudaMalloc((void **)&b.info, sizeof(int)));
+  QB_CUDA_TRY(cudaMalloc((void **)&b.panels, sizeof(double) * sparse_chol_factor_doubles(b.sp)));
+  QB_CUDA_TRY(cudaMalloc((void **)&b.rhs, sizeof(double) * (size_t)N));
+  QB_CUDA_TRY(cudaMalloc((void **)&b.x, sizeof(double) * (size_t)N));
+  QB_CUDA_TRY(cudaMemcpyAsync(b.Kp, rp.data(), sizeof(int) * ((size_t)N + 1), cudaMemcpyHostToDevice, b.st));
+  QB_CUDA_TRY(cudaMemcpyAsync(b.Ki, rj.data(), sizeof(int) * (nnzF + 1), cudaMemcpyHostToDevice, b.st));
+  QB_CUDA_TRY(cudaMemcpyAsync(b.Kx, rx.data(), sizeof(double) * (nnzF + 1), cudaMemcpyHostToDevice, b.st));
+  QB_CUDA_TRY(cudaMemcpyAsync(b.rhs, rhs, sizeof(double) * (size_t)N, cudaMemcpyHostToDevice, b.st));
+  QB_CUDA_TRY(cudaMemsetAsync(b.info, 0, sizeof(int), b.st));
+  if (int r = sparse_chol_assemble(b.sp, b.st, b.panels, true, b.Kp, b.Ki, b.Kx, nullptr, nullptr, nullptr, nullptr, nullptr,
+                                   nullptr, nullptr, nullptr, 0.0)) return r;
+  if (int r = sparse_chol_factor(b.sp, b.st, b.panels, b.info)) return r;
+  if (int r = sparse_chol_solve(b.sp, b.st, b.panels, b.rhs, b.x, false)) return r;
+  int info = 0;
+  QB_CUDA_TRY(cudaMemcpyAsync(x, b.x, sizeof(double) * (size_t)N, cudaMemcpyDeviceToHost, b.st));
+  QB_CUDA_TRY(cudaMemcpyAsync(&info, b.info, sizeof(int), cudaMemcpyDeviceToHost, b.st));
+  QB_CUDA_TRY(cudaStreamSynchronize(b.st));
+  if (panels_out && panels_cap >= I->nnzL)
+    QB_CUDA_TRY(cudaMemcpy(panels_out, b.panels, sizeof(double) * (size_t)I->nnzL, cudaMemcpyDeviceToHost));
+  if (L_out && perm_out)
+    if (int r = sparse_chol_download(b.sp, b.st, b.panels, L_out, (long long *)perm_out)) return r;
+  return info ? 1000 + info : 0;
+}
+
+extern "C" int qpalm_b200_kkt_newton(const solver_sparse *Q, const solver_sparse *A, const c_float *sigma, const c_int *active,
+        c_float beta, const c_float *rhs, c_float *d, c_int *refine_out, c_float *norms_out) {
+  if (!Q || !A || !sigma || !active || !rhs || !d || A->nrow < 1 || A->ncol != Q->ncol) return 1;
+  const int n = (int)Q->ncol, m = (int)A->nrow;
+  Engine *e = nullptr;
+  if (int rc = make_engine(&e, n, m, A, Q, false, 3)) return rc;   // 3: the KKT path asked for (FACTORIZE_KKT)
+  if (!e->kkt) { engine_destroy(e); return 7; }                   // dense-classified data never gets the KKT engine
+  std::vector<double> sinv((size_t)m);
+  for (int i = 0; i < m; i++) sinv[i] = 1.0 / sigma[i];
+  upload(e, e->sigma, sigma, m); upload(e, e->sigma_inv, sinv.data(), m);
+  std::vector<double> neg((size_t)n);
+  for (int i = 0; i < n; i++) neg[i] = -rhs[i];
+  upload(e, e->dphi, neg.data(), n);
+  cudaStreamSynchronize(e->stream);
+  up_int(e, e->active, active, m);
+  QB_CUDA_TRY(cudaMemset(e->info_dev, 0, sizeof(int)));
+  const long long r0 = kkt_refine_count(e->kkt);
+  int rc = kkt_refactor(e->kkt, e, beta);
+  if (!rc) rc = kkt_solve(e->kkt, e);
+  if (!rc) rc = download(e, d, e->d, n);
+  if (refine_out) *refine_out = (c_int)(kkt_refine_count(e->kkt) - r0);
+  if (norms_out) kkt_last_norms(e->kkt, norms_out);
+  int info = 0;
+  if (!rc) rc = -(int)cudaMemcpy(&info, e->info_dev, sizeof(int), cudaMemcpyDeviceToHost);
+  engine_destroy(e);
+  return rc ? rc : (info ? 1000 + info : 0);
+}
+
 extern "C" int qpalm_b200_lobpcg(const solver_sparse *Q, const c_float *x0, c_float *lambda_out, c_int *iters_out) {
   Engine *e = nullptr; int rc;
   if ((rc = make_engine(&e, (int)Q->ncol, 0, nullptr, Q))) return rc;

@@ -28,6 +28,10 @@ def _lib():
     lib.qpalm_b200_sparse_newton.argtypes = [C.POINTER(abi.SolverSparse), C.POINTER(abi.SolverSparse), abi.c_float_p, abi.c_int_p,
                                              C.c_double, abi.c_float_p, abi.c_float_p, abi.c_float_p, abi.c_int_p, abi.c_int_p,
                                              abi.c_int, abi.c_int_p, abi.c_int, abi.c_float_p]
+    lib.qpalm_b200_sparse_ldl.argtypes = [C.POINTER(abi.SolverSparse), abi.c_int, abi.c_float_p, abi.c_float_p, abi.c_float_p,
+                                          abi.c_int_p, abi.c_float_p, abi.c_int, abi.c_int_p]
+    lib.qpalm_b200_kkt_newton.argtypes = [C.POINTER(abi.SolverSparse), C.POINTER(abi.SolverSparse), abi.c_float_p, abi.c_int_p,
+                                          C.c_double, abi.c_float_p, abi.c_float_p, abi.c_int_p, abi.c_float_p]
     return lib
 
 
@@ -75,3 +79,46 @@ def sparse_newton(Q: abi.CSC, A: abi.CSC | None, sigma, active, beta, rhs, enter
     if rc:
         raise RuntimeError(f"qpalm_b200_sparse_newton failed with code {rc}")
     return d, L, perm, (float(bound[0]) if want_bound else None)
+
+
+def sparse_ldl(K: abi.CSC, n_pos: int, rhs, want_factor=False, panels_len=0):
+    """x = K^{-1} rhs through the signed supernodal factorization K(perm, perm) = L S L' of a quasi-definite K (lower
+    triangle CSC; original columns >= n_pos carry negative pivots), one solve without refinement.
+    Returns (rc, x, L_permuted or None, perm or None, panels or None): rc is 0, or 1000 + info when a pivot did not
+    have its a-priori sign (info - 1: a permuted column in the front of such a pivot or
+    in a front above it).  panels_len > 0 (symbolic(K, None)["nnzL"]) also returns the raw factor panels."""
+    lib = _lib()
+    N = K.ncol
+    rhs = np.ascontiguousarray(rhs, dtype=np.float64)
+    x = np.zeros(N)
+    L = np.zeros((N, N), order="F") if want_factor else None
+    perm = np.zeros(N, dtype=np.int64) if want_factor else None
+    panels = np.zeros(max(panels_len, 1)) if panels_len else None
+    plen = np.zeros(1, dtype=np.int64)
+    rc = lib.qpalm_b200_sparse_ldl(K.ptr(), int(n_pos), abi.fptr(rhs), abi.fptr(x),
+                                   L.ctypes.data_as(abi.c_float_p) if want_factor else None,
+                                   abi.iptr(perm) if want_factor else None,
+                                   abi.fptr(panels) if panels_len else None, int(panels_len), abi.iptr(plen))
+    if rc and rc < 1000:
+        raise RuntimeError(f"qpalm_b200_sparse_ldl failed with code {rc}")
+    if panels_len:
+        assert int(plen[0]) == panels_len, (int(plen[0]), panels_len)
+    return rc, x, L, perm, panels
+
+
+def kkt_newton(Q: abi.CSC, A: abi.CSC, sigma, active, beta, rhs):
+    """The KKT Newton step: d = (Q + A_J' Sigma_J A_J + beta I)^{-1} rhs through the L S L' factorization of
+    [Q + beta I, A_J'; A_J, -inv(Sigma_J)] and the solver's iterative refinement.
+    Returns (rc, d, refinement corrections applied, (|res|inf, ref) of the last residual)."""
+    lib = _lib()
+    sigma = np.ascontiguousarray(sigma, dtype=np.float64)
+    act = np.ascontiguousarray(active, dtype=np.int64)
+    rhs = np.ascontiguousarray(rhs, dtype=np.float64)
+    d = np.zeros(Q.ncol)
+    refine = np.zeros(1, dtype=np.int64)
+    norms = np.zeros(2)
+    rc = lib.qpalm_b200_kkt_newton(Q.ptr(), A.ptr(), abi.fptr(sigma), abi.iptr(act), float(beta), abi.fptr(rhs), abi.fptr(d),
+                                   abi.iptr(refine), abi.fptr(norms))
+    if rc and rc < 1000:
+        raise RuntimeError(f"qpalm_b200_kkt_newton failed with code {rc}")
+    return rc, d, int(refine[0]), (float(norms[0]), float(norms[1]))

@@ -93,3 +93,26 @@ def test_schur_fill_in_problem_selects_kkt_automatically():
     _parity(g, g1)
     print(f"kkt_standin n=2500: KKT {t_kkt:.3f} s (nnz(L) {st.sparse_factor_nnz}, {st.kkt_factorizations} factorizations, "
           f"{st.kkt_refinement_steps} refinement steps) vs Schur (dense) {t_schur:.3f} s")
+
+
+def test_forced_kkt_per_block_launches_equal_cluster_launches():
+    """random_qp(300, 600) has fronts above the shared-memory size (263 rows at most): the per-block launches and the cluster
+    launches of the signed factorization are bit-identical, so the whole trajectory must be too -- x, y, iteration counts
+    and the number of iterative-refinement corrections."""
+    import os
+    p = problems.random_qp(300, 600, 0.02, 0.01, seed=3)
+    out = {}
+    for mode, flag in (("per_block", "1"), ("cluster", "0")):
+        old = os.environ.get("QPALM_B200_MF_PER_BLOCK")
+        os.environ["QPALM_B200_MF_PER_BLOCK"] = flag
+        try:
+            out[mode] = _solve("b200", p, factorization_method=0)
+        finally:
+            os.environ.pop("QPALM_B200_MF_PER_BLOCK", None) if old is None else os.environ.__setitem__("QPALM_B200_MF_PER_BLOCK", old)
+    (a, sa, ma), (b, sb, mb) = out["per_block"], out["cluster"]
+    assert ma == mb == 0 and sa.kkt_factorizations > 0
+    assert np.array_equal(a.x, b.x) and np.array_equal(a.y, b.y)
+    assert (a.iter, a.iter_out) == (b.iter, b.iter_out)
+    assert (sa.kkt_factorizations, sa.kkt_refinement_steps) == (sb.kkt_factorizations, sb.kkt_refinement_steps)
+    print(f"random_qp(300, 600) forced KKT: {a.iter} iterations, {sa.kkt_factorizations} factorizations, "
+          f"{sa.kkt_refinement_steps} refinement corrections")
