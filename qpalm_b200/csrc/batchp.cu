@@ -17,8 +17,8 @@
 //
 // The Newton system (Q + A_J' Sigma_J A_J + I/gamma) d = -dphi  (src/newton.c:96-118, solver_interface.c:319-519):
 //   H is kept per instance and updated incrementally (+ entering / - leaving / +- sigma changes) or rebuilt from c Q by an in-CTA
-//   tile-stationary SYRK (cta_syrk), L <- chol(H + beta I) by an in-CTA right-looking blocked Cholesky (diagonal sub-blocks in one warp's
-//   registers, panel solve one row per thread); SYRK and trailing updates run on the FP64 tensor pipe (mma.sync m8n8k4, 16 x 16
+//   tile-stationary SYRK (cta_syrk), L <- chol(H + beta I) by an in-CTA right-looking blocked Cholesky (each panel as a dataflow: a chain warp
+//   on the diagonal, every other thread the owner of one panel row, per-column mbarriers); SYRK and trailing updates run on the FP64 tensor pipe (mma.sync m8n8k4, 16 x 16
 //   tiles per warp); then two blocked triangular solves.  When the active set changes by at most min(0.1 (n + m),
 //   max_rank_update) rows -- and at most 40, see p_control -- and the factor is current, the factor is UPDATED in place instead
 //   (cta_updown_sweep: <= 8 ranks per sweep, entering rows before leaving rows; a chain warp on the diagonal, every other thread
@@ -36,12 +36,12 @@ using namespace qb;
 
 // Build-time shape of a CTA; this file is compiled twice (build.sh), and each shape once more with -DQB_BP_PROBE, which
 // replaces the solver kernel by the test probes of its building blocks (see kbp_probe_newton):
-//   default            8 warps, 32-column panel (16-wide sub-panels): 80 registers x 256 threads, 72 KB -> 3 CTAs / SM (444
+//   default            8 warps, 32-column panel: 80 registers x 256 threads, 72 KB -> 3 CTAs / SM (444
 //                      slots on a B200).  Best per-wave throughput: 444 instances in 57.9 ms (7675 solves/s), 4096 instances
 //                      in 488 ms (8396 solves/s) at the end of round 2.
-//   -DQB_BP_VARIANT4   8 warps, 24-column panel (-DQB_BP_SW=8: 8-wide sub-panels), registers capped at 64: 55 KB -> 4 CTAs / SM
+//   -DQB_BP_VARIANT4   8 warps, 24-column panel, registers capped at 64: 55 KB -> 4 CTAs / SM
 //                      (592 slots).  Both sort buffers (40 KB) fit the union region of either shape.  Slower per
-//                      instance (64 registers: several loops are shaped around that, see QB_BP_SW and p_gemv_rows) but the
+//                      instance (64 registers: several loops are shaped around that, see p_gemv_rows) but the
 //                      BASELINE sweep of 512 instances per GPU fits in ONE wave: 78.8 ms against 90.3 ms with the 68-instance
 //                      tail of the default shape.  batch.cu picks it when 3 * SMs < nb <= 4 * SMs.
 // Other shapes measured in round 1 (512 instances): 192 threads / PW 24 / 4 per SM 138.6 ms; 192 / PW 16 / 4 per SM
@@ -86,8 +86,9 @@ namespace qb {
 namespace QB_BP_NAMESPACE {
 
 constexpr int NT = QB_BP_NT, NW = NT / 32;
-constexpr int PW = QB_BP_PW;      // panel width (sub-panels of 16 + 8 columns)
+constexpr int PW = QB_BP_PW;      // panel width (at most 32: the chain warp of the Cholesky holds a panel's diagonal rows)
 constexpr int NMAX = 240;         // largest n of this engine (panel = PW x LDP doubles of shared memory)
+static_assert(PW <= 32 && PW % 4 == 0, "one chain warp per panel; whole DMMA k-steps");
 constexpr int LDP = NMAX + 1;     // odd leading dimension: conflict-free row and column access
 static_assert(NMAX <= NT, "the update sweep maps thread t to row t of the factor");
 constexpr int SORT_MAX = 2048;    // largest 2m
@@ -717,153 +718,6 @@ __device__ __forceinline__ void panel_load_async(double *Pn, const double *L, in
   bp_cp_async_wait_all();
 }
 
-// The PW = 32 column panel is factorised as two 16-column sub-panels so that every per-thread register array is 16
-// doubles (a 32-wide version needs 64 registers per array and spills at 3 CTAs / SM).
-#ifndef QB_BP_SW
-#define QB_BP_SW 16
-#endif
-constexpr int SW = QB_BP_SW;          // sub-panel width of the in-CTA Cholesky (the diagonal block one warp factors in registers)
-static_assert(PW % SW == 0 || PW == 24, "panel = whole sub-panels (24 = 16 + 8 in the 16-wide build)");
-constexpr int UPW = PW - SW;          // columns of the panel to the right of a sub-panel (at most)
-
-// Cholesky of the 16 x 16 block at (c0, c0) of the panel (P[t][r], t = column, r = row), warp 0; lane = row, the row
-// lives in registers.  The column loop is ROLLED around a rotating register file: a[0] is always the current column and
-// every step shifts the row one register to the left while it applies the rank-1 update, so all register indices are
-// static although the loop is not unrolled.  The body is ~100 instructions and stays in the instruction cache.  (A fully
-// unrolled version is ~1k straight-line instructions executed once per call; with three CTAs per SM in different phases
-// of this large kernel it ran at instruction-fetch-miss speed: 27 us per block in situ, phase profile of round 1.)  The
-// arithmetic and its order are those of the unrolled form, so results are bit-identical to it.
-// Columns/rows >= w (ragged last panel) are skipped.  rd[c0 + j] = 1 / l_jj.
-__device__ __noinline__ void warp_factor_diag16(double *Pn, double *rd, double *colbuf, int c0, int w, int *info) {
-  const int lane = threadIdx.x & 31;
-  const int row = c0 + lane;
-  const int wend = (w - c0 < SW) ? w - c0 : SW;
-  const bool live = lane < wend;
-  double a[SW];
-#pragma unroll
-  for (int c = 0; c < SW; c++) a[c] = (live && c < wend) ? ((c <= lane) ? Pn[(c0 + c) * LDP + row] : 0.0) : ((c == lane) ? 1.0 : 0.0);
-  bool bad = false;
-  __syncwarp();
-#pragma unroll 1
-  for (int j = 0; j < SW; j++) {
-    const double pjj = __shfl_sync(0xffffffffu, a[0], j);
-    if (!(pjj > 0.0)) bad = true;
-    // branch-free sqrt / reciprocal (chol32.cuh): rsqrt() carries a slow-path CALL, and the values live across that call site were
-    // spilled and reloaded from local memory in every column (five dependent LDL per column under a thrashed 30 KB L1)
-    double ljj, inv;
-    chol32::sqrt_and_rcp(pjj, ljj, inv);
-    const double a0 = (lane == j) ? ljj : a[0] * inv;     // lanes < j: upper triangle, never used
-    if (lane == j) rd[c0 + j] = inv;
-    if (live && lane >= j && j < wend) Pn[(c0 + j) * LDP + row] = a0;
-    // column j is broadcast through shared memory (two alternating 32-entry buffers, one __syncwarp per column): the 15 loads are
-    // independent and issue back to back, where 15 64-bit shuffles each exposed their latency before the FMA that consumes them
-    // (the loop ran at ~1270 clocks per column on an otherwise idle SM)
-    double *cb = colbuf + ((j & 1) << 5);
-    cb[lane] = a0;
-    __syncwarp();
-#pragma unroll
-    for (int c = 1; c < SW; c++) {
-      const double lcj = cb[(j + c) & 31];
-      a[c - 1] = (lane >= j + c) ? fma(-a0, lcj, a[c]) : a[c];   // column j + c moves to register c - 1
-    }
-    a[SW - 1] = 0.0;
-  }
-  if (bad && lane == 0 && info) *info = 1;
-}
-
-// rows below the sub-panel's diagonal block: P[c0 + c][r] <- forward substitution against the factor at (c0, c0)
-__device__ __forceinline__ void panel_solve16(double *Pn, const double *rd, int c0, int w, int rows) {
-  const int wsub = (w - c0 < SW) ? w - c0 : SW;       // the second sub-panel of a 24-column panel has 8 columns
-  for (int r = c0 + wsub + threadIdx.x; r < rows; r += NT) {
-    double v[SW];
-#pragma unroll
-    for (int c = 0; c < SW; c++) v[c] = (c0 + c < w) ? Pn[(c0 + c) * LDP + r] : 0.0;
-#pragma unroll
-    for (int c = 0; c < SW; c++) {
-      if (c0 + c < w) {
-        double s = v[c];
-#pragma unroll
-        for (int t = 0; t < SW; t++) if (t < c) s = fma(-v[t], Pn[(c0 + t) * LDP + c0 + c], s);
-        v[c] = s * rd[c0 + c];
-      }
-    }
-#pragma unroll
-    for (int c = 0; c < SW; c++) if (c0 + c < w) Pn[(c0 + c) * LDP + r] = v[c];
-  }
-}
-
-// after sub-panel [c0, c0 + SW): the panel's columns to its right, rows r >= c0 + SW:
-//   P[c0 + SW + c][r] -= sum_{t < SW} P[c0 + t][r] P[c0 + t][c0 + SW + c]   for c0 + SW + c <= min(r, w - 1)
-__device__ __forceinline__ void panel_update16(double *Pn, int c0, int w, int rows) {
-  for (int r = c0 + SW + threadIdx.x; r < rows; r += NT) {
-    double acc[UPW];
-#pragma unroll
-    for (int c = 0; c < UPW; c++) acc[c] = 0.0;
-#pragma unroll 4
-    for (int t = 0; t < SW; t++) {
-      const double lr = Pn[(c0 + t) * LDP + r];
-#pragma unroll
-      for (int c = 0; c < UPW; c++) if (c0 + SW + c < PW) acc[c] = fma(lr, Pn[(c0 + t) * LDP + c0 + SW + c], acc[c]);
-    }
-#pragma unroll
-    for (int c = 0; c < UPW; c++) if (c0 + SW + c < w && c0 + SW + c <= r) Pn[(c0 + SW + c) * LDP + r] -= acc[c];
-  }
-}
-
-// L <- chol(sscale * src + beta I) (lower, n x n), right-looking with PW-column panels.  rdiag_g[j] = 1 / l_jj.
-__device__ __forceinline__ void cta_potrf(double *L, int ld, const double *src, int lds, double sscale, double beta, int n, double *rdiag_g,
-                          const Smem &S, int *info, long long *pf) {
-  const int tid = threadIdx.x;
-  double *Pn = S.panel;
-  long long tq = clock64();
-// Phase clocks: one predicated atomic, NO divergent region.  (An `if (tid == 0) { load; add; store }` body leaves lane 0 split
-// from the rest of warp 0 under independent thread scheduling; every __shfl_sync of the following single-warp phases then
-// takes the WARPSYNC.COLLECTIVE slow path -- measured 131k instead of 13.6k clocks per 16 x 16 diagonal block, which made
-// the profile of round 1 blame the wrong phase.)
-#define PQ(k) do { if (pf) { const long long t_ = clock64(); if (tid == NT - 1) atomicAdd(reinterpret_cast<unsigned long long *>(pf + (k)), (unsigned long long)(t_ - tq)); tq = t_; } } while (0)
-  for (int k0 = 0; k0 < n; k0 += PW) {
-    const int w = (n - k0 < PW) ? n - k0 : PW, rows = n - k0;
-    const bool first = (k0 == 0);
-    if (first) {
-      for (int idx = tid; idx < w * rows; idx += NT) {   // panel load, rows fastest (coalesced)
-        const int t = idx / rows, r = idx - t * rows;
-        double v = 0.0;
-        if (r >= t) { v = sscale * src[(size_t)r + (size_t)lds * t]; if (r == t) v += beta; }
-        Pn[t * LDP + r] = v;
-      }
-    } else panel_load_async(Pn, L, ld, k0, w, rows);
-    __syncthreads();
-    PQ(16);
-    for (int c0 = 0; c0 < w; c0 += SW) {   // sub-panels: diagonal block (one warp) -> rows below -> the panel's columns to the right
-      if (tid < 32) warp_factor_diag16(Pn, S.rd, S.vs, c0, w, info);
-      __syncthreads();
-      PQ(17);
-      panel_solve16(Pn, S.rd, c0, w, rows);
-      __syncthreads();
-      PQ(18);
-      if (c0 + SW < w) {
-        panel_update16(Pn, c0, w, rows);
-        __syncthreads();
-        PQ(19);
-      }
-    }
-    for (int idx = tid; idx < w * rows; idx += NT) {   // final columns of L
-      const int t = idx / rows, r = idx - t * rows;
-      if (r >= t) L[(size_t)(k0 + r) + (size_t)ld * (k0 + t)] = Pn[t * LDP + r];
-    }
-    if (tid < w) rdiag_g[k0 + tid] = S.rd[tid];
-    PQ(20);
-    if (w & 3) {   // ragged last panel: zero the pad columns the DMMA product loop reads (no trailing matrix then, but keep it defined)
-      for (int idx = tid; idx < (((w + 3) & ~3) - w) * rows; idx += NT) { const int t = w + idx / rows, r = idx - (t - w) * rows; Pn[t * LDP + r] = 0.0; }
-      __syncthreads();
-    }
-    cta_rank_update_lower(L, ld, src, lds, sscale, beta, first, k0 + w, n, Pn, k0, w, -1.0);
-    __syncthreads();
-    PQ(21);
-  }
-#undef PQ
-}
-
 // Tile-stationary SYRK of the Newton matrix:
 //   dst(i, j) = base(i, j) + sum_{e < npos} wpos[e]^2 a_e(i) a_e(j) - sum_{e < nneg} wneg[e]^2 a'_e(i) a'_e(j)   for j <= i < n,
 // a_e = A'[:, lpos[e]], a'_e = A'[:, lneg[e]]; base = 0, dst itself, or sscale * src (lds): the zeroed Gershgorin matrix of
@@ -1039,6 +893,7 @@ __device__ __forceinline__ void cta_syrk(double *dst, int ld, int n, int base, c
 constexpr int KU = 8, UW = 16, WIN = 32, PBL = 33;   // ranks per sweep, columns per block, rows of the chain warp's window, block row pitch
 constexpr int NRING = 3;                              // window-block buffers: in use by the chain / being requested / being written back
 constexpr int LVW = 8;                                // row owners: columns of their row's entries in flight (shared-memory staging ring)
+constexpr int NBAR = PW > UW ? PW : UW;               // per-column mbarriers: one per column of a Cholesky panel (the sweep and the solves use UW)
 static_assert((KU * LDP + NRING * UW * PBL + LVW * LDP) * sizeof(double) <= kUnionBytes,
               "W block + the ring of window-block buffers + the row owners' staging ring must fit the union region");
 
@@ -1476,6 +1331,135 @@ __device__ __noinline__ void cta_chol_solve(const double *L, int ld, int n, cons
   phase = ph + 2 * nblk;
 }
 
+// ------------------------------------------------------------------------------------------------
+// L <- chol(sscale * src + beta I) (lower, n x n), right-looking with PW-column panels.  rdiag_g[j] = 1 / l_jj.
+// A panel (its rows k0 .. n - 1 in S.panel, P[t][r], t = column, r = row - k0) is factorised as the dataflow of the update
+// sweep and the triangular solves:
+//   * the CHAIN WARP (warp 0) holds rows k0 .. k0 + 31 (lane = row): the w <= 32 diagonal rows and, in the 24-column shape,
+//     the first 8 rows below them.  Per column j: the pivot from lane j (one shuffle), l_jj and 1 / l_jj, the column scaled,
+//     published in the panel with rd[j], an arrive on column j's mbarrier, then column j applied to the window;
+//   * every other thread owns one panel row (thread t <-> row k0 + t; n <= NMAX <= NT): it waits on column j's mbarrier, scales
+//     its entry by rd[j] and applies column j to the rest of its row.
+// The rows stay in the panel (the odd LDP keeps a warp's accesses to one column conflict-free; 24 or 32 doubles per thread
+// in registers spill at 64 / 80 registers).  Each thread then stores its own row of L, so one barrier per panel remains
+// before the trailing DMMA update.  The form it replaces factored 16- or 8-column diagonal blocks in warp 0 with the seven
+// other warps parked at a barrier, then the rows below, then the columns to the right: about ten barriers per panel.
+// Rounding: every entry takes one fma per column in ascending column order, l_ij = a_ij * (1 / l_jj), whoever holds it.
+// bars: NBAR mbarriers (count 1); every panel completes one phase of each.  Barriers 0 .. UW - 1 are those of the sweep and
+// the solves (phase count `phase`), barriers UW .. NBAR - 1 serve only the factorisation (`phase_hi`).
+// ------------------------------------------------------------------------------------------------
+// apply column j (its entries l_cj in P[j][c], this row's l_rj = l) to columns j0 <= c < w of row r, r >= c only (rlim = r,
+// or -1 for a row outside the panel).  Four columns' loads are issued before their fmas and stores.
+__device__ __forceinline__ void potrf_row_apply(double *Pn, int r, int rlim, int j, int j0, int w, double l) {
+  int c = j0;
+#pragma unroll 1
+  for (; c + 4 <= w; c += 4) {
+    double lc[4], a[4];
+#pragma unroll
+    for (int u = 0; u < 4; u++) { lc[u] = Pn[j * LDP + c + u]; a[u] = Pn[(c + u) * LDP + r]; }
+#pragma unroll
+    for (int u = 0; u < 4; u++) if (rlim >= c + u) Pn[(c + u) * LDP + r] = fma(-l, lc[u], a[u]);
+  }
+#pragma unroll 1
+  for (; c < w; c++) if (rlim >= c) Pn[c * LDP + r] = fma(-l, Pn[j * LDP + c], Pn[c * LDP + r]);
+}
+
+// One panel after its load: factor, store its rows of L and 1 / l_jj, zero the pad columns [w, w + 3 & ~3) of every row for the
+// DMMA product loop.  par_lo / par_hi: the parity of this panel's phase of barriers < UW / >= UW.  The caller's
+// __syncthreads() ends the panel.  Phase clocks: 17 chain column loop, 18 chain store + wait (lane 31); 19 owners' column loop,
+// 20 owners' store + wait (thread 32, the first owner).
+__device__ __noinline__ void potrf_panel(double *Pn, double *rd, double *L, int ld, double *rdiag_g, int k0, int w, int rows,
+                                         unsigned long long *bars, unsigned par_lo, unsigned par_hi, int *info, long long *pf) {
+  const int tid = threadIdx.x;
+  long long tq = clock64();
+#define PQ(k, rec) do { if (pf) { const long long t_ = clock64(); if (rec) atomicAdd(reinterpret_cast<unsigned long long *>(pf + (k)), (unsigned long long)(t_ - tq)); tq = t_; } } while (0)
+  if (tid < WIN) {   // chain warp: no lane-dependent branch around the shuffles, __syncwarp and arrives (predicated stores only)
+    const int lane = tid;
+    const bool live = lane < rows;
+    const int rlim = live ? lane : -1;
+    double cur = live ? Pn[lane] : 0.0;   // this row's entry of the current column, final
+    double pv = __shfl_sync(0xffffffffu, cur, 0);
+    bool bad = false;
+#pragma unroll 1
+    for (int j = 0; j < w; j++) {
+      double ljj, inv;
+      chol32::sqrt_and_rcp(pv, ljj, inv);
+      if (!(pv > 0.0)) bad = true;   // pv is the same in every lane
+      const double l = (lane == j) ? ljj : cur * inv;
+      // the next pivot first: lane j + 1 needs only its own l_{j+1,j}, so the chain per column is one shuffle, sqrt / rcp, one
+      // multiply and one fma (the published column and the rest of the window follow)
+      const int j1 = (j + 1 < w) ? j + 1 : j;
+      const double a1 = Pn[j1 * LDP + lane];
+      pv = __shfl_sync(0xffffffffu, fma(-l, l, a1), (j + 1) & 31);
+      if (rlim >= j) Pn[j * LDP + lane] = l;
+      if (lane == j) rd[j] = inv;
+      __syncwarp();
+      ud_mbar_arrive_lane0(bars + j, lane);   // column j is published: the row owners may apply it
+      cur = fma(-l, Pn[j * LDP + j1], a1);    // column j + 1 of this row (lane j + 1: the pivot just shuffled)
+      potrf_row_apply(Pn, lane, rlim, j, j + 2, w, l);
+    }
+    for (int j = w; j < NBAR; j++) ud_mbar_arrive_lane0(bars + j, lane);   // ragged last panel: every barrier completes one phase
+    if (bad && lane == 0) *info = 1;
+    PQ(17, lane == 31);
+    if (live) {
+      for (int c = 0; c < w; c++) if (c <= lane) L[(size_t)(k0 + lane) + (size_t)ld * (k0 + c)] = Pn[c * LDP + lane];
+      for (int c = w; c < ((w + 3) & ~3); c++) Pn[c * LDP + lane] = 0.0;
+    }
+    if (lane < w) rdiag_g[k0 + lane] = rd[lane];   // rd[lane] was written by this lane
+  } else if (tid < rows) {   // row owner (row tid >= 32 > w: every column of the panel applies)
+    const int r = tid;
+#pragma unroll 1
+    for (int j = 0; j < w; j++) {
+      ud_mbar_wait(bars + j, j < UW ? par_lo : par_hi);
+      const double l = Pn[j * LDP + r] * rd[j];
+      Pn[j * LDP + r] = l;
+      potrf_row_apply(Pn, r, r, j, j + 1, w, l);
+    }
+    PQ(19, tid == WIN);
+    for (int c = 0; c < w; c++) L[(size_t)(k0 + r) + (size_t)ld * (k0 + c)] = Pn[c * LDP + r];
+    for (int c = w; c < ((w + 3) & ~3); c++) Pn[c * LDP + r] = 0.0;
+  }
+  __syncthreads();
+  PQ(tid == 31 ? 18 : 20, tid == 31 || tid == WIN);
+#undef PQ
+}
+
+__device__ __forceinline__ void cta_potrf(double *L, int ld, const double *src, int lds, double sscale, double beta, int n, double *rdiag_g,
+                          const Smem &S, int *info, unsigned long long *bars, unsigned &phase, unsigned &phase_hi, long long *pf) {
+  const int tid = threadIdx.x;
+  double *Pn = S.panel;
+  const unsigned ph = phase, phh = phase_hi;   // read and written once (they live in the caller's frame)
+  long long tq = clock64();
+// Phase clocks: one predicated atomic, NO divergent region.  (An `if (tid == 0) { load; add; store }` body leaves lane 0 split
+// from the rest of warp 0 under independent thread scheduling; every __shfl_sync of the following single-warp phases then
+// takes the WARPSYNC.COLLECTIVE slow path -- measured 131k instead of 13.6k clocks per 16 x 16 diagonal block, which made
+// the profile of round 1 blame the wrong phase.)
+#define PQ(k) do { if (pf) { const long long t_ = clock64(); if (tid == NT - 1) atomicAdd(reinterpret_cast<unsigned long long *>(pf + (k)), (unsigned long long)(t_ - tq)); tq = t_; } } while (0)
+  unsigned p = 0;
+  for (int k0 = 0; k0 < n; k0 += PW, p++) {
+    const int w = (n - k0 < PW) ? n - k0 : PW, rows = n - k0;
+    const bool first = (k0 == 0);
+    if (first) {
+      for (int idx = tid; idx < w * rows; idx += NT) {   // panel load, rows fastest (coalesced)
+        const int t = idx / rows, r = idx - t * rows;
+        double v = 0.0;
+        if (r >= t) { v = sscale * src[(size_t)r + (size_t)lds * t]; if (r == t) v += beta; }
+        Pn[t * LDP + r] = v;
+      }
+    } else panel_load_async(Pn, L, ld, k0, w, rows);
+    __syncthreads();
+    PQ(16);
+    potrf_panel(Pn, S.rd, L, ld, rdiag_g, k0, w, rows, bars, (ph + p) & 1u, (phh + p) & 1u, info, pf);
+    if (pf) tq = clock64();
+    cta_rank_update_lower(L, ld, src, lds, sscale, beta, first, k0 + w, n, Pn, k0, w, -1.0);
+    __syncthreads();
+    PQ(21);
+  }
+  phase = ph + p;
+  phase_hi = phh + p;
+#undef PQ
+}
+
 // ordered lists of the entering (candidate active, not in the factor) and leaving rows, entering first, weights sqrt(sigma):
 // list_pos[0 .. ne + nl), w_pos likewise (set_entering_leaving_constraints, newton.c:134-149).  Returns counts through ctl.npos / nneg.
 __device__ __noinline__ void p_updown_lists(const Args &P, int b) {
@@ -1891,10 +1875,10 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_solve(const Args P) {
   __shared__ int s_b;
   __shared__ Flags s_f;
   __shared__ int s_info;
-  __shared__ __align__(8) unsigned long long s_udbar[UW];   // per-column mbarriers of the update sweep (chain warp -> row owners)
-  unsigned ud_phase = 0;
+  __shared__ __align__(8) unsigned long long s_udbar[NBAR];   // per-column mbarriers of the dataflows (chain warp -> row owners)
+  unsigned ud_phase = 0, ud_phase_hi = 0;                      // phases so far of barriers < UW / >= UW (see cta_potrf)
   if (threadIdx.x == 0) {
-    for (int j = 0; j < UW; j++) ud_mbar_init(s_udbar + j, 1);
+    for (int j = 0; j < NBAR; j++) ud_mbar_init(s_udbar + j, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncthreads();
@@ -1980,7 +1964,7 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_solve(const Args P) {
           const double beta = P.ctl[b].beta;
           if (tid == 0) s_info = 0;
           cta_potrf(Lb, ld, f.fq ? P.Qs : Hb, f.fq ? n : ld, f.fq ? P.ctl[b].c : 1.0, beta, n, rdg, S, &s_info,
-                    P.prof ? P.prof + (size_t)b * 32 : nullptr);
+                    s_udbar, ud_phase, ud_phase_hi, P.prof ? P.prof + (size_t)b * 32 : nullptr);
         }
         PH(7);
         cta_chol_solve(Lb, ld, n, rdg, S, s_udbar, ud_phase, P.prof ? P.prof + (size_t)b * 32 : nullptr);
@@ -2027,7 +2011,7 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_solve(const Args P) {
 // (same CTA shape, launch bounds, shared-memory carving, per-column mbarriers whose phase carries across the sweeps and the
 // instances of a CTA, persistent CTAs on an atomic queue), so that a test checks the code the solver executes.
 // They are built from this file in objects of their own (build.sh, -DQB_BP_PROBE): with a second caller in the same
-// translation unit, the __noinline__ building blocks (cta_updown_sweep, warp_factor_diag16) would no longer see kbp_solve's
+// translation unit, the __noinline__ building blocks (cta_updown_sweep, potrf_panel) would no longer see kbp_solve's
 // __shared__ mbarrier and info addresses as constants, and kbp_solve would be compiled differently (more spills).
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ Smem probe_smem(unsigned char *smem_raw) {
@@ -2048,10 +2032,10 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_probe_newton(const BpProbe
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ int s_b;
   __shared__ int s_info;
-  __shared__ __align__(8) unsigned long long s_udbar[UW];
-  unsigned ud_phase = 0;
+  __shared__ __align__(8) unsigned long long s_udbar[NBAR];
+  unsigned ud_phase = 0, ud_phase_hi = 0;
   if (threadIdx.x == 0) {
-    for (int j = 0; j < UW; j++) ud_mbar_init(s_udbar + j, 1);
+    for (int j = 0; j < NBAR; j++) ud_mbar_init(s_udbar + j, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncthreads();
@@ -2083,7 +2067,7 @@ __global__ void __launch_bounds__(NT, QB_BP_MINB) kbp_probe_newton(const BpProbe
     if (tid == 0) s_info = 0;
     // from_q without lists: the f.fq path, the factor reads the shared source (lds = n) directly; else the refactorisation of H
     const bool fq = P.from_q && npos + nneg == 0;
-    cta_potrf(Lb, ld, fq ? P.H0 : Hb, fq ? n : ld, fq ? sc : 1.0, P.beta, n, rdg, S, &s_info, nullptr);
+    cta_potrf(Lb, ld, fq ? P.H0 : Hb, fq ? n : ld, fq ? sc : 1.0, P.beta, n, rdg, S, &s_info, s_udbar, ud_phase, ud_phase_hi, nullptr);
     cta_chol_solve(Lb, ld, n, rdg, S, s_udbar, ud_phase, nullptr);
     for (int i = tid; i < n; i += NT) P.d_fused[on + i] = S.v[i];
     __syncthreads();

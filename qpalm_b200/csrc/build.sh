@@ -15,13 +15,13 @@ for f in dense updown_gen kernels api ops compat kkt batch batchp prof shard spa
 done
 # the persistent batch engine a second time in its 4-CTAs-per-SM shape (see the header of batchp.cu)
 if [ ! -f build/batchp4.o ] || [ batchp.cu -nt build/batchp4.o ] || [ batch.cuh -nt build/batchp4.o ] || [ common.cuh -nt build/batchp4.o ] || [ engine.cuh -nt build/batchp4.o ]; then
-  $NVCC $FLAGS -DQB_BP_VARIANT4 ${QB_BP4_FLAGS:--DQB_BP_SW=8} -c batchp.cu -o build/batchp4.o &
+  $NVCC $FLAGS -DQB_BP_VARIANT4 $QB_BP4_FLAGS -c batchp.cu -o build/batchp4.o &
   pids+=($!)
 fi
 # and both shapes once more with the test probes of its building blocks instead of the solver kernel (-DQB_BP_PROBE)
 for v in batchp_probe batchp4_probe; do
   if [ ! -f build/$v.o ] || [ batchp.cu -nt build/$v.o ] || [ batch.cuh -nt build/$v.o ] || [ common.cuh -nt build/$v.o ] || [ engine.cuh -nt build/$v.o ] || [ chol32.cuh -nt build/$v.o ] || [ ../../include/qpalm_b200.h -nt build/$v.o ]; then
-    if [ $v = batchp4_probe ]; then VF="-DQB_BP_VARIANT4 ${QB_BP4_FLAGS:--DQB_BP_SW=8}"; else VF=""; fi
+    if [ $v = batchp4_probe ]; then VF="-DQB_BP_VARIANT4 $QB_BP4_FLAGS"; else VF=""; fi
     $NVCC $FLAGS $VF -DQB_BP_PROBE -c batchp.cu -o build/$v.o &
     pids+=($!)
   fi

@@ -20,8 +20,8 @@ assert h.lib.qpalm_b200_batch_phase_profile(h.h, nb, out.ctypes.data) == 0
 x, y, infos = h.download(nb)
 iters = np.array([i["iter"] for i in infos])
 names = ["init", "res_m", "gemv_Atyh", "res_n+control", "outer/sigma/boost", "lists", "H syrk", "potrf", "solve", "gemv Qd+Ad",
-         "ls_build", "sort", "select+update", "gemv Qd", "rank-k update sweeps", "H syrk: A' gather + stage wait", "potrf: panel load", "potrf: diag16", "potrf: solve16", "potrf: update16",
-         "potrf: store", "potrf: trailing", "sweep: gather W", "sweep chain warp: block prologue", "sweep: whole block loop (row owner's clock)", "sweep chain warp: column loop",
+         "ls_build", "sort", "select+update", "gemv Qd", "rank-k update sweeps", "H syrk: A' gather + stage wait", "potrf: panel load", "potrf: chain column loop", "potrf: chain waiting",
+         "potrf: owners' column loop", "potrf: store", "potrf: trailing", "sweep: gather W", "sweep chain warp: block prologue", "sweep: whole block loop (row owner's clock)", "sweep chain warp: column loop",
          "sweep chain warp: block epilogue", "sweep chain warp: wait for the row owners",
          "solve fwd chain warp: column loop", "solve fwd chain warp: block ends + window waits",
          "solve bwd chain warp: column loop", "solve bwd chain warp: block ends + window waits"]
@@ -35,5 +35,8 @@ print(f"H syrk: {st['syrk_entries']/nr:.1f} list entries per refactorization, sc
 nls = max(st["inner"], 1)
 print(f"line search: {st['ls_breakpoints']/nls:.1f} breakpoints sorted (s > 0 of 2m = {2*b.A.nrow}), {st['ls_walked']/nls:.1f} walked, "
       f"per line search ({100*st['ls_walked']/max(st['ls_breakpoints'], 1):.1f}% of the sorted ones)")
+ncol = max(st["refactorizations"], 1) * b.q.shape[1]   # panel columns factored in all
+print(f"potrf per column: chain loop {out[:, 17].sum() / ncol:.0f} clocks, owners' loop {out[:, 19].sum() / ncol:.0f} clocks "
+      f"(chain lane 31 / first owner)")
 for k in list(range(32)):
     print(f"{names[k]:22s} {out[:,k].mean()/1.965e3:10.1f} us/instance  {100*out[:,k].sum()/tot.sum():6.2f}%   per-iter {out[:,k].sum()/iters.sum()/1.965e3:7.2f} us")
