@@ -419,6 +419,30 @@ int qpalm_b200_batchp_probe_solves(c_int shape, c_int nb, c_int n, c_int m, cons
  * as unsigned integers, equal keys in their input order (the solver sorts (key, position) pairs) */
 int qpalm_b200_batchp_probe_sort(c_int shape, c_int nb, c_int N, unsigned long long *keys, unsigned int *vals);
 
+/* Test probes of the dense Newton-system kernels (dense.cu), called unchanged on host data through a fresh non-blocking
+ * stream.  Matrices are column-major; instance b of a batched buffer starts b strides in.  Each returns 0, 1 for invalid
+ * arguments, 2 when device memory is short, < 0 for a CUDA error.
+ * gemm:  C[b] = beta C[b] + alpha A[b][:, :k] B[b][:, :k]' (M x N, M and N multiples of 128, K of 16; leading dimensions and
+ *        strides even), k = Kz[b] (a multiple of 16, at most K) or K; instances with mask[b] == 0 untouched; lower_only: only
+ *        128 x 128 tiles on or below the diagonal written.  in_place: A is C itself (N = 128, K <= 128; A, lda, sA ignored),
+ *        the form of the Cholesky's panel solve.  tile_rows (may be NULL) receives the tile rows of the kernel that ran (64, 128).
+ * potrf: L (nb x npad x npad, lower triangle) <- its Cholesky factor, invdiag (nb x npad x 128) <- the inverses of its 128 x 128
+ *        diagonal blocks, info[b] set to 1 + the first column with a non-positive pivot (it must come in as 0; with mask[b] == 0
+ *        L, invdiag and info stay as they came).  mode 0: the single-matrix entry (nb = 1, no mask; look-ahead for
+ *        npad > 1024); mode 1: the batched schedule (mask NULL: every instance).
+ * trtri: invdiag (npad x 128) <- the inverses of the diagonal blocks of the factor L (npad x npad).
+ * solve: V[b][r] <- (L L')^{-1} V[b][r] for rounds r = 0 .. rounds - 1 in turn on one stream (V: nb x rounds x npad), with the
+ *        leading sizes[r] x sizes[r] block of L (sizes NULL: npad; multiples of 128); entries beyond it untouched.  mode 0: the
+ *        single-matrix solve (nb = 1, no mask), grid[r] = its cooperative grid, 0 for the per-block launches; mode 1: the batched
+ *        per-block launches with the mask, grid[r] = 0.  grid may be NULL. */
+int qpalm_b200_dense_probe_gemm(c_int nb, c_int M, c_int N, c_int K, const c_int *Kz, const c_int *mask, const c_float *A, c_int lda,
+        c_int sA, const c_float *B, c_int ldb, c_int sB, c_float *C, c_int ldc, c_int sC, c_float alpha, c_float beta,
+        c_int lower_only, c_int in_place, c_int *tile_rows);
+int qpalm_b200_dense_probe_potrf(c_int nb, c_int npad, c_float *L, c_float *invdiag, const c_int *mask, c_int *info, c_int mode);
+int qpalm_b200_dense_probe_trtri(c_int npad, const c_float *L, c_float *invdiag);
+int qpalm_b200_dense_probe_solve(c_int nb, c_int npad, const c_float *L, const c_float *invdiag, c_float *V, c_int rounds,
+        const c_int *sizes, const c_int *mask, c_int mode, c_int *grid);
+
 #ifdef __cplusplus
 }
 #endif

@@ -177,9 +177,13 @@ static int gemm_attr() {
   return 0;
 }
 
+static thread_local int g_gemm_last_rows = 0;   // tile rows (64 or 128) of this thread's last dgemm_nt_batched launch
+int dgemm_last_tile_rows() { return g_gemm_last_rows; }
+
 int dgemm_nt_batched(cudaStream_t s, int nb, int M, int N, int K, const int *Kz, const double *A, int lda, long long sA,
                      const double *B, int ldb, long long sB, double *C, int ldc, long long sC, double alpha, double beta,
                      bool lower_only, const int *maskz) {
+  g_gemm_last_rows = 0;
   if (M <= 0 || N <= 0 || nb <= 0) return 0;
   if ((M % gemm::BM) || (N % gemm::BN) || (K % gemm::BK)) {
     fprintf(stderr, "[qpalm_b200] dgemm_nt: bad shape M=%d N=%d K=%d\n", M, N, K);
@@ -191,6 +195,7 @@ int dgemm_nt_batched(cudaStream_t s, int nb, int M, int N, int K, const int *Kz,
   const long long tiles = (lower_only ? (nt <= mt ? nt * mt - nt * (nt - 1) / 2 : mt * (mt + 1) / 2) : mt * nt) * nb;
   static int num_sms = 0;
   if (!num_sms) { int dev = 0; QB_CUDA_TRY(cudaGetDevice(&dev)); QB_CUDA_TRY(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev)); }
+  g_gemm_last_rows = tiles < num_sms ? 64 : gemm::BM;
   if (tiles < num_sms) {
     dim3 grid(M / 64, N / gemm::BN, nb);
     QB_LAUNCH(gemm::k_dgemm_nt_tma<64>, grid, 288, gemm::smem_bytes_tma<64>(), s, K, A, lda, B, ldb, C, ldc, alpha, beta,
@@ -934,6 +939,9 @@ static std::mutex g_flow_mu;
 static std::map<cudaStream_t, FlowState> g_flow;
 }  // namespace flow
 
+static thread_local int g_solve_last_grid = 0;   // cooperative grid of this thread's last chol_solve, 0: per-block launches
+int chol_solve_last_grid() { return g_solve_last_grid; }
+
 // returns 0 when the dataflow solve ran, 1 when it is not available (caller falls back to the per-block launches), < 0 on error
 static int chol_solve_flow(cudaStream_t s, int npad, const double *L, int ld, const double *invdiag, double *v) {
   static const bool off = getenv("QPALM_B200_NO_FLOW_SOLVE") != nullptr;
@@ -978,6 +986,7 @@ static int chol_solve_flow(cudaStream_t s, int npad, const double *L, int ld, co
     return 1;
   }
   ++g_kernel_launches;
+  g_solve_last_grid = grid;
   return 0;
 }
 
@@ -1004,6 +1013,7 @@ int chol_solve_batched(cudaStream_t s, int nb, int npad, const double *L, int ld
   return 0;
 }
 int chol_solve(cudaStream_t s, int npad, const double *L, int ld, const double *invdiag, double *v) {
+  g_solve_last_grid = 0;
   if (npad > 2 * kPanel) {
     const int rc = chol_solve_flow(s, npad, L, ld, invdiag, v);
     if (rc <= 0) return -rc;

@@ -14,10 +14,14 @@ int dgemm_nt(cudaStream_t s, int M, int N, int K, const double *A, int lda, cons
              double *C, int ldc, double alpha, double beta, bool lower_only);
 
 // Batched variants (grid.z / grid.y = instance; element strides sA.. between instances; Kz: optional per-instance K,
-// maskz: optional per-instance activity flags).
+// maskz: optional per-instance activity flags).  Kz entries must be multiples of 16 and at most K: the kernel runs Kz / 16
+// k-tiles, dropping a remainder silently (the lock-step engine pads its row lists to a multiple of 16 with zero rows).
 int dgemm_nt_batched(cudaStream_t s, int nb, int M, int N, int K, const int *Kz, const double *A, int lda, long long sA,
                      const double *B, int ldb, long long sB, double *C, int ldc, long long sC, double alpha, double beta,
                      bool lower_only, const int *maskz);
+// tile rows (64 or 128) of the kernel this thread's last dgemm_nt_batched call launched, 0 if it launched none.  The 64-row
+// kernel runs when the tiles with work number fewer than the SMs.
+int dgemm_last_tile_rows();
 int potrf_lower_batched(cudaStream_t s, int nb, int npad, double *L, int ld, long long sL, double *invdiag, long long sX,
                         int *info_dev, const int *mask);
 int chol_solve_batched(cudaStream_t s, int nb, int npad, const double *L, int ld, long long sL, const double *invdiag,
@@ -33,6 +37,8 @@ int trtri_diag_blocks(cudaStream_t s, int npad, const double *L, int ld, double 
 
 // v <- (L L')^{-1} v, v of length npad (pad entries must be 0).
 int chol_solve(cudaStream_t s, int npad, const double *L, int ld, const double *invdiag, double *v);
+// cooperative grid of the one-launch dataflow solve of this thread's last chol_solve, 0 when it ran the per-block launches
+int chol_solve_last_grid();
 // releases the per-stream scratch chol_solve keeps (flag buffer of the one-launch dataflow solve); call before destroying s
 void chol_solve_release(cudaStream_t s);
 

@@ -698,3 +698,130 @@ extern "C" int qpalm_b200_bench_gemv(c_int n_, c_int m_, c_int reps, double *ms_
   cudaStreamDestroy(e.stream);
   return 0;
 }
+
+// ---- test probes of the dense Newton-system kernels (dense.cu), run unchanged on caller data ---------------------------
+// Host buffers in and out; the work runs on a fresh non-blocking stream, as in the engines.
+namespace {
+struct DenseProbe {   // stream and device buffers of one probe call, released on every return path
+  cudaStream_t s = nullptr;
+  std::vector<void *> p;
+  bool failed = false;
+  template <typename T> T *get(size_t count) {
+    void *q = nullptr;
+    if (dev_alloc(&q, sizeof(T) * (count ? count : 1))) { failed = true; return nullptr; }
+    p.push_back(q);
+    return static_cast<T *>(q);
+  }
+  template <typename T> T *up(const T *src, size_t count) {   // nullptr for a null source
+    if (!src) return nullptr;
+    T *d = get<T>(count);
+    if (d && cudaMemcpyAsync(d, src, sizeof(T) * count, cudaMemcpyHostToDevice, s) != cudaSuccess) { failed = true; return nullptr; }
+    return d;
+  }
+  std::vector<int> flags(const c_int *src, size_t count) {   // c_int (64-bit) array -> int array
+    std::vector<int> t(count + 1, 0);
+    for (size_t i = 0; i < count; i++) t[i] = (int)src[i];
+    return t;
+  }
+  ~DenseProbe() {
+    if (s) { cudaStreamSynchronize(s); chol_solve_release(s); }
+    for (void *q : p) cudaFree(q);
+    if (s) cudaStreamDestroy(s);
+  }
+};
+}  // namespace
+
+extern "C" int qpalm_b200_dense_probe_gemm(c_int nb_, c_int M_, c_int N_, c_int K_, const c_int *Kz, const c_int *mask,
+                                           const c_float *A, c_int lda, c_int sA, const c_float *B, c_int ldb, c_int sB,
+                                           c_float *C, c_int ldc, c_int sC, c_float alpha, c_float beta, c_int lower_only,
+                                           c_int in_place, c_int *tile_rows) {
+  if (nb_ < 1 || M_ < 1 || N_ < 1 || K_ < 0 || M_ % 128 || N_ % 128 || K_ % 16 || M_ > (1 << 20) || N_ > (1 << 20) || K_ > (1 << 20)) return 1;
+  if (in_place) { A = C; lda = ldc; sA = sC; if (N_ != 128 || K_ > N_) return 1; }
+  if ((K_ > 0 && (!A || !B)) || !C || lda < M_ || ldb < N_ || ldc < M_ || (lda | ldb | ldc | sA | sB | sC) & 1) return 1;
+  if (nb_ > 1 && (sA < lda * K_ || sB < ldb * K_ || sC < ldc * N_)) return 1;
+  const int nb = (int)nb_, M = (int)M_, N = (int)N_, K = (int)K_;
+  std::vector<int> kz, mk;
+  DenseProbe d;
+  if (Kz) {
+    kz = d.flags(Kz, (size_t)nb);
+    for (int b = 0; b < nb; b++) if (kz[b] < 0 || kz[b] > K || kz[b] % 16) return 1;   // the kernel runs Kz / 16 k-tiles
+  }
+  if (mask) mk = d.flags(mask, (size_t)nb);
+  QB_CUDA_TRY(cudaStreamCreateWithFlags(&d.s, cudaStreamNonBlocking));
+  const size_t nA = (size_t)(nb - 1) * sA + (size_t)lda * K, nB = (size_t)(nb - 1) * sB + (size_t)ldb * K;
+  const size_t nC = (size_t)(nb - 1) * sC + (size_t)ldc * N;
+  double *dC = d.up(C, nC);
+  const double *dA = in_place ? dC : d.up(A, nA), *dB = d.up(B, nB);
+  const int *dKz = Kz ? d.up(kz.data(), (size_t)nb) : nullptr, *dmask = mask ? d.up(mk.data(), (size_t)nb) : nullptr;
+  if (d.failed) return 2;
+  if (int r = dgemm_nt_batched(d.s, nb, M, N, K, dKz, dA, (int)lda, sA, dB, (int)ldb, sB, dC, (int)ldc, sC, alpha, beta,
+                               lower_only != 0, dmask)) return r;
+  if (tile_rows) *tile_rows = dgemm_last_tile_rows();
+  QB_CUDA_TRY(cudaMemcpyAsync(C, dC, sizeof(double) * nC, cudaMemcpyDeviceToHost, d.s));
+  QB_CUDA_TRY(cudaStreamSynchronize(d.s));
+  return 0;
+}
+
+extern "C" int qpalm_b200_dense_probe_potrf(c_int nb_, c_int npad_, c_float *L, c_float *invdiag, const c_int *mask, c_int *info,
+                                            c_int mode) {
+  if (nb_ < 1 || npad_ < 128 || npad_ % 128 || npad_ > (1 << 16) || (mode != 0 && mode != 1) || !L || !invdiag || !info) return 1;
+  if (mode == 0 && (nb_ != 1 || mask)) return 1;
+  const int nb = (int)nb_, npad = (int)npad_;
+  const size_t sL = (size_t)npad * npad, sX = (size_t)npad * kPanel;
+  DenseProbe d;
+  std::vector<int> mk = mask ? d.flags(mask, (size_t)nb) : std::vector<int>((size_t)nb, 1), inf = d.flags(info, (size_t)nb);
+  QB_CUDA_TRY(cudaStreamCreateWithFlags(&d.s, cudaStreamNonBlocking));
+  double *dL = d.up(L, nb * sL), *dX = d.up(invdiag, nb * sX);
+  int *dinfo = d.up(inf.data(), (size_t)nb), *dmask = mode == 1 ? d.up(mk.data(), (size_t)nb) : nullptr;
+  if (d.failed) return 2;
+  // mode 0: the single-matrix entry (look-ahead for npad > 1024); mode 1: the batched schedule, never with look-ahead
+  if (int r = mode == 0 ? potrf_lower(d.s, npad, dL, npad, dX, dinfo)
+                        : potrf_lower_batched(d.s, nb, npad, dL, npad, (long long)sL, dX, (long long)sX, dinfo, dmask)) return r;
+  QB_CUDA_TRY(cudaMemcpyAsync(L, dL, sizeof(double) * nb * sL, cudaMemcpyDeviceToHost, d.s));
+  QB_CUDA_TRY(cudaMemcpyAsync(invdiag, dX, sizeof(double) * nb * sX, cudaMemcpyDeviceToHost, d.s));
+  QB_CUDA_TRY(cudaMemcpyAsync(inf.data(), dinfo, sizeof(int) * nb, cudaMemcpyDeviceToHost, d.s));
+  QB_CUDA_TRY(cudaStreamSynchronize(d.s));
+  for (int b = 0; b < nb; b++) info[b] = inf[b];
+  return 0;
+}
+
+extern "C" int qpalm_b200_dense_probe_trtri(c_int npad_, const c_float *L, c_float *invdiag) {
+  if (npad_ < 128 || npad_ % 128 || npad_ > (1 << 16) || !L || !invdiag) return 1;
+  const int npad = (int)npad_;
+  DenseProbe d;
+  QB_CUDA_TRY(cudaStreamCreateWithFlags(&d.s, cudaStreamNonBlocking));
+  const double *dL = d.up(L, (size_t)npad * npad);
+  double *dX = d.get<double>((size_t)npad * kPanel);
+  if (d.failed) return 2;
+  if (int r = trtri_diag_blocks(d.s, npad, dL, npad, dX)) return r;
+  QB_CUDA_TRY(cudaMemcpyAsync(invdiag, dX, sizeof(double) * npad * kPanel, cudaMemcpyDeviceToHost, d.s));
+  QB_CUDA_TRY(cudaStreamSynchronize(d.s));
+  return 0;
+}
+
+extern "C" int qpalm_b200_dense_probe_solve(c_int nb_, c_int npad_, const c_float *L, const c_float *invdiag, c_float *V, c_int rounds_,
+                                            const c_int *sizes, const c_int *mask, c_int mode, c_int *grid) {
+  if (nb_ < 1 || npad_ < 128 || npad_ % 128 || npad_ > (1 << 16) || rounds_ < 1 || (mode != 0 && mode != 1) || !L || !invdiag || !V) return 1;
+  if (mode == 0 && (nb_ != 1 || mask)) return 1;
+  const int nb = (int)nb_, npad = (int)npad_, rounds = (int)rounds_;
+  for (int r = 0; r < rounds && sizes; r++) if (sizes[r] < 128 || sizes[r] > npad || sizes[r] % 128) return 1;
+  const size_t sL = (size_t)npad * npad, sX = (size_t)npad * kPanel, sV = (size_t)rounds * npad;
+  DenseProbe d;
+  std::vector<int> mk = mask ? d.flags(mask, (size_t)nb) : std::vector<int>();
+  QB_CUDA_TRY(cudaStreamCreateWithFlags(&d.s, cudaStreamNonBlocking));
+  const double *dL = d.up(L, nb * sL), *dX = d.up(invdiag, nb * sX);
+  double *dV = d.up(V, nb * sV);
+  const int *dmask = mask ? d.up(mk.data(), (size_t)nb) : nullptr;
+  if (d.failed) return 2;
+  // round r: V[b, r, :size_r] <- (L L')^{-1} V[b, r, :size_r] with the leading size_r x size_r block of L (its own factor)
+  for (int r = 0; r < rounds; r++) {
+    const int n = sizes ? (int)sizes[r] : npad;
+    double *v = dV + (size_t)r * npad;
+    if (int e = mode == 0 ? chol_solve(d.s, n, dL, npad, dX, v)
+                          : chol_solve_batched(d.s, nb, n, dL, npad, (long long)sL, dX, (long long)sX, v, (long long)sV, dmask)) return e;
+    if (grid) grid[r] = mode == 0 ? chol_solve_last_grid() : 0;
+  }
+  QB_CUDA_TRY(cudaMemcpyAsync(V, dV, sizeof(double) * nb * sV, cudaMemcpyDeviceToHost, d.s));
+  QB_CUDA_TRY(cudaStreamSynchronize(d.s));
+  return 0;
+}
