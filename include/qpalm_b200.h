@@ -434,7 +434,17 @@ int qpalm_b200_batchp_probe_sort(c_int shape, c_int nb, c_int N, unsigned long l
  * solve: V[b][r] <- (L L')^{-1} V[b][r] for rounds r = 0 .. rounds - 1 in turn on one stream (V: nb x rounds x npad), with the
  *        leading sizes[r] x sizes[r] block of L (sizes NULL: npad; multiples of 128); entries beyond it untouched.  mode 0: the
  *        single-matrix solve (nb = 1, no mask), grid[r] = its cooperative grid, 0 for the per-block launches; mode 1: the batched
- *        per-block launches with the mask, grid[r] = 0.  grid may be NULL. */
+ *        per-block launches with the mask, grid[r] = 0.  grid may be NULL.
+ * updown: rank-k updates / downdates L L' <- L L' + W_r S_r W_r' for passes r = 0 .. passes - 1 in turn on ONE stream, on the
+ *        leading sizes[r] x sizes[r] block of L (npad x npad, lower triangle, leading dimension npad; sizes NULL: npad; multiples
+ *        of 128).  Pass r takes the next k[r] columns of W (npad rows each), S_r = diag(+1 x kpos[r], -1 x (k[r] - kpos[r])).
+ *        Before each pass the device info is reset; info[r] receives it afterwards (0, or 1 + 32 B for a failing 32-row block B
+ *        in mode 0, nonzero in mode 1).  mode 0: trtri_diag_blocks, then the generator-form pass (updown_gen.cu, k[r] <= 32);
+ *        grid_cap > 0 caps the CTAs per column group of its triangular solve for this call (block rows are dealt to fewer
+ *        CTAs; the result must not change); grid[2 r] receives the per-group grid that ran, grid[2 r + 1] the limit it ran
+ *        under.  mode 1: the per-panel sweep of dense.cu (k[r] <= 8, kpos[r] = 0 or k[r]), grid entries 0.  What, Z (npad x k)
+ *        and D (npad), mode 0 only, each may be NULL: the last pass's inv(L) W, its generators z_j (rows) and d_j, rows from
+ *        sizes[last] on untouched.  grid may be NULL.  Returns 3 when the generator form is unavailable on this device. */
 int qpalm_b200_dense_probe_gemm(c_int nb, c_int M, c_int N, c_int K, const c_int *Kz, const c_int *mask, const c_float *A, c_int lda,
         c_int sA, const c_float *B, c_int ldb, c_int sB, c_float *C, c_int ldc, c_int sC, c_float alpha, c_float beta,
         c_int lower_only, c_int in_place, c_int *tile_rows);
@@ -442,6 +452,8 @@ int qpalm_b200_dense_probe_potrf(c_int nb, c_int npad, c_float *L, c_float *invd
 int qpalm_b200_dense_probe_trtri(c_int npad, const c_float *L, c_float *invdiag);
 int qpalm_b200_dense_probe_solve(c_int nb, c_int npad, const c_float *L, const c_float *invdiag, c_float *V, c_int rounds,
         const c_int *sizes, const c_int *mask, c_int mode, c_int *grid);
+int qpalm_b200_dense_probe_updown(c_int npad, c_float *L, const c_float *W, c_int passes, const c_int *k, const c_int *kpos,
+        const c_int *sizes, c_int mode, c_int grid_cap, c_int *info, c_int *grid, c_float *What, c_float *Z, c_float *D);
 
 #ifdef __cplusplus
 }

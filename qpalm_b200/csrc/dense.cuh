@@ -56,6 +56,14 @@ int chol_updown_gen(cudaStream_t s, int npad, double *L, int ld, const double *i
                     int *info_dev);
 int chol_updown_gen_max_rank();
 void chol_updown_gen_release(cudaStream_t s);
+// test hooks.  last_grid: the per-group cooperative grid (blockIdx.x extent) of k_fwd_multi in this thread's last pass, 0 when
+// it launched none; *gmax (may be NULL) the limit it ran under (the resident CTAs / groups, or the cap).  set_grid_cap: caps
+// this thread's limit at cap CTAs per group (cap <= 0: no cap, the default) so that tests can deal block rows to fewer CTAs.
+// workspace: the device work space of stream s's last pass, What (npad x 32) | Z (npad x 32) | D (npad) with the column
+// stride npad of that pass, or NULL.
+int chol_updown_gen_last_grid(int *gmax);
+void chol_updown_gen_set_grid_cap(int cap);
+const double *chol_updown_gen_workspace(cudaStream_t s);
 
 // L(lower) <- H(lower) + diag_add * I on the leading n x n block; pad block <- identity.
 int copy_lower_add_diag(cudaStream_t s, int n, int npad, const double *H, double *L, int ld, double diag_add);

@@ -724,7 +724,7 @@ struct DenseProbe {   // stream and device buffers of one probe call, released o
     return t;
   }
   ~DenseProbe() {
-    if (s) { cudaStreamSynchronize(s); chol_solve_release(s); }
+    if (s) { cudaStreamSynchronize(s); chol_solve_release(s); chol_updown_gen_release(s); }
     for (void *q : p) cudaFree(q);
     if (s) cudaStreamDestroy(s);
   }
@@ -823,5 +823,69 @@ extern "C" int qpalm_b200_dense_probe_solve(c_int nb_, c_int npad_, const c_floa
   }
   QB_CUDA_TRY(cudaMemcpyAsync(V, dV, sizeof(double) * nb * sV, cudaMemcpyDeviceToHost, d.s));
   QB_CUDA_TRY(cudaStreamSynchronize(d.s));
+  return 0;
+}
+
+extern "C" int qpalm_b200_dense_probe_updown(c_int npad_, c_float *L, const c_float *W, c_int passes_, const c_int *k,
+                                             const c_int *kpos, const c_int *sizes, c_int mode, c_int grid_cap, c_int *info,
+                                             c_int *grid, c_float *What, c_float *Z, c_float *D) {
+  if (npad_ < 128 || npad_ % 128 || npad_ > (1 << 16) || passes_ < 1 || (mode != 0 && mode != 1) || !L || !W || !k || !kpos || !info) return 1;
+  const int npad = (int)npad_, passes = (int)passes_;
+  size_t kt = 0;
+  for (int r = 0; r < passes; r++) {
+    const c_int kmax = mode == 0 ? chol_updown_gen_max_rank() : 8;
+    if (k[r] < 1 || k[r] > kmax || kpos[r] < 0 || kpos[r] > k[r]) return 1;
+    if (mode == 1 && kpos[r] != 0 && kpos[r] != k[r]) return 1;                        // the per-panel sweep has one sign per call
+    if (sizes && (sizes[r] < 128 || sizes[r] > npad || sizes[r] % 128)) return 1;
+    kt += (size_t)k[r];
+  }
+  if ((What || Z || D) && mode != 0) return 1;
+  DenseProbe d;
+  QB_CUDA_TRY(cudaStreamCreateWithFlags(&d.s, cudaStreamNonBlocking));
+  double *dL = d.up(L, (size_t)npad * npad);
+  double *dW = d.up(W, (size_t)npad * kt);       // a copy: the per-panel sweep overwrites its W
+  double *dX = d.get<double>((size_t)npad * kPanel), *coef = d.get<double>(2 * 32 * 18 + 16);
+  int *dinfo = d.get<int>(1);
+  if (d.failed) return 2;
+  struct Cap {   // the grid cap holds for this call only, on every return path
+    explicit Cap(int c) { chol_updown_gen_set_grid_cap(c); }
+    ~Cap() { chol_updown_gen_set_grid_cap(0); }
+  } cap(mode == 0 ? (int)grid_cap : 0);
+  std::vector<int> inf((size_t)passes, 0);
+  size_t off = 0;
+  int n = npad, kk = 0;
+  for (int r = 0; r < passes; r++) {
+    n = sizes ? (int)sizes[r] : npad;
+    kk = (int)k[r];
+    double *w = dW + off * npad;
+    QB_CUDA_TRY(cudaMemsetAsync(dinfo, 0, sizeof(int), d.s));
+    if (mode == 0) {
+      if (int e = trtri_diag_blocks(d.s, n, dL, npad, dX)) return e;
+      const int e = chol_updown_gen(d.s, n, dL, npad, dX, w, npad, kk, (int)kpos[r], dinfo);
+      if (e == 1) return 3;
+      if (e) return e;
+    } else if (int e = chol_updown(d.s, n, dL, npad, w, npad, kk, kpos[r] ? +1 : -1, coef, dinfo)) {
+      return e;
+    }
+    if (grid) {
+      int gmax = 0;
+      grid[2 * r] = mode == 0 ? chol_updown_gen_last_grid(&gmax) : 0;
+      grid[2 * r + 1] = gmax;
+    }
+    QB_CUDA_TRY(cudaMemcpyAsync(&inf[r], dinfo, sizeof(int), cudaMemcpyDeviceToHost, d.s));
+    off += (size_t)kk;
+  }
+  if (What || Z || D) {   // the last pass's What | Z | D, column stride n in the work space, npad here (rows >= n untouched)
+    const double *ws = chol_updown_gen_workspace(d.s);
+    if (!ws) return 1;
+    const double *src[3] = {ws, ws + (size_t)n * 32, ws + (size_t)n * 64};
+    c_float *dst[3] = {What, Z, D};
+    for (int q = 0; q < 3; q++)
+      if (dst[q]) QB_CUDA_TRY(cudaMemcpy2DAsync(dst[q], sizeof(double) * npad, src[q], sizeof(double) * n, sizeof(double) * n,
+                                                q == 2 ? 1 : kk, cudaMemcpyDeviceToHost, d.s));
+  }
+  QB_CUDA_TRY(cudaMemcpyAsync(L, dL, sizeof(double) * npad * npad, cudaMemcpyDeviceToHost, d.s));
+  QB_CUDA_TRY(cudaStreamSynchronize(d.s));
+  for (int r = 0; r < passes; r++) info[r] = inf[r];
   return 0;
 }

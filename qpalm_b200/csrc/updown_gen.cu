@@ -374,6 +374,10 @@ struct State {
 };
 static std::mutex g_mu;
 static std::map<cudaStream_t, State> g_state;
+// test hooks (host only, no kernel reads them): the per-group grid of this thread's last k_fwd_multi launch and the limit it
+// was launched under, and a cap on that limit.  The cap applies to gmax, never to max_grid: a max_grid below NS would mark the
+// pass unavailable on the stream for good.  0: no cap (the default; only qpalm_b200_dense_probe_updown sets one).
+static thread_local int g_last_grid = 0, g_last_gmax = 0, g_grid_cap = 0;
 
 template <int KT, int KW>     // KT columns per pass, solved as KT / KW independent groups
 static int run(cudaStream_t s, State &st, int slot, int npad, double *L, int ld, const double *X, const double *W, int ldw, int k, int kpos,
@@ -393,7 +397,7 @@ static int run(cudaStream_t s, State &st, int slot, int npad, double *L, int ld,
   const int nblk = npad / NB, nblocks = npad / GB;
   double *What = st.buf, *Z = What + (size_t)npad * 32, *D = Z + (size_t)npad * 32, *G = D + npad;
   {
-    const int gmax = st.max_grid[slot] / NS;
+    const int gmax = (g_grid_cap > 0 && g_grid_cap < st.max_grid[slot] / NS) ? g_grid_cap : st.max_grid[slot] / NS;
     const int grid = nblk < gmax ? nblk : gmax;
     int ld_a = ld, ldw_a = ldw, k_a = k, npad_a = npad, nblk_a = nblk, epoch = st.epoch, kt = KT;
     uint4 *pk = st.packets;
@@ -405,6 +409,7 @@ static int run(cudaStream_t s, State &st, int slot, int npad, double *L, int ld,
     if (prof) prof_end(s);
     if (err != cudaSuccess) { (void)cudaGetLastError(); st.max_grid[slot] = -1; return 1; }
     ++g_kernel_launches;
+    g_last_grid = grid; g_last_gmax = gmax;
   }
   QB_LAUNCH(k_gen_gram<KT>, nblocks, 256, 0, s, What, npad, G);
   QB_LAUNCH(k_gen_scan<KT>, KT * KT / SCAN_E, SCAN_E * SCAN_C, 0, s, G, nblocks, k, kpos);
@@ -424,6 +429,7 @@ int chol_updown_gen_max_rank() { return 32; }
 int chol_updown_gen(cudaStream_t s, int npad, double *L, int ld, const double *invdiag, const double *W, int ldw, int k, int kpos,
                     int *info_dev) {
   using namespace udgen;
+  g_last_grid = g_last_gmax = 0;
   if (k <= 0) return 0;
   if (k > 32 || (npad % NB)) return 1;
   std::lock_guard<std::mutex> lk(g_mu);
@@ -454,6 +460,18 @@ int chol_updown_gen(cudaStream_t s, int npad, double *L, int ld, const double *i
   if (k <= 8) return run<8, 8>(s, st, 0, npad, L, ld, invdiag, W, ldw, k, kpos, info_dev);
   if (k <= 16) return run<16, 8>(s, st, 1, npad, L, ld, invdiag, W, ldw, k, kpos, info_dev);
   return run<32, 16>(s, st, 2, npad, L, ld, invdiag, W, ldw, k, kpos, info_dev);
+}
+
+int chol_updown_gen_last_grid(int *gmax) {
+  if (gmax) *gmax = udgen::g_last_gmax;
+  return udgen::g_last_grid;
+}
+void chol_updown_gen_set_grid_cap(int cap) { udgen::g_grid_cap = cap > 0 ? cap : 0; }
+
+const double *chol_updown_gen_workspace(cudaStream_t s) {
+  std::lock_guard<std::mutex> lk(udgen::g_mu);
+  auto it = udgen::g_state.find(s);
+  return it == udgen::g_state.end() ? nullptr : it->second.buf;
 }
 
 void chol_updown_gen_release(cudaStream_t s) {
